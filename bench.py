@@ -6,6 +6,7 @@ ms/frame at 4K, 1/2/4/8 B200, beside the reference's CPU path).
     python bench.py --impl reference --gpus N --steps K ...   # the reference's CPU algorithm
                                                               # (the oracle port; no Rust here)
     torchrun --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...     # N > 1
+    python bench.py ... --dump-outputs DIR                    # + the last timed frame as DIR/*.npy
 
 A step = one full frame of the workload (default C4 = BASELINE.json configs[3]: 3840x2160,
 10,000 mixed reflective/refractive spheres + ground plane, 3 lights, depth 8; synthetic,
@@ -29,6 +30,23 @@ import numpy as np  # noqa: E402
 
 METRIC = "Mrays/sec (all bounces) at 4K; ms/frame in ms_per_step"
 UNIT = "Mrays/s"
+# pixels of the frame --dump-outputs writes: 32 MiB of float32 RGBA + 16 MiB of float64 indices (a quarter of a 4K frame)
+DUMP_PIXELS = 1 << 21
+
+
+def dump_outputs(out_dir, frame, stats) -> None:
+    """--dump-outputs: what the device-resident arm's last timed step delivered, comparable between two builds.
+    frame_sample.npy is float32 RGBA (0..255) of a fixed, seeded sample of the frame's pixels, frame_sample_index.npy
+    their flat indices y * width + x; ray_counts.npy (one GPU) the frame's primary, shadow, reflection and
+    transmission rays."""
+    os.makedirs(out_dir, exist_ok=True)
+    h, w, _ = frame.shape
+    idx = np.sort(np.random.default_rng(0).choice(h * w, size=min(DUMP_PIXELS, h * w), replace=False))
+    np.save(os.path.join(out_dir, "frame_sample.npy"), frame.reshape(h * w, 4)[idx].astype(np.float32))
+    np.save(os.path.join(out_dir, "frame_sample_index.npy"), idx.astype(np.float64))
+    if stats is not None:
+        np.save(os.path.join(out_dir, "ray_counts.npy"), np.array(
+            [stats.rays_primary, stats.rays_shadow, stats.rays_reflection, stats.rays_transmission], np.float64))
 
 
 def flops_per_ray(data) -> float:
@@ -369,7 +387,12 @@ def main() -> int:
     ap.add_argument("--reference-budget", type=float, default=150.0, help="--impl reference: total seconds")
     ap.add_argument("--no-roofline", action="store_true")
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the last timed frame (a fixed, seeded sample of its pixels, float32) and its ray counts "
+                         "to DIR/*.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 0)
 
     rank = int(os.environ.get("RANK", "0"))
@@ -631,7 +654,11 @@ def main() -> int:
     # the frame of the device-resident arm, for the equality check of all arms below
     value_frame_sha = None
     if rank == 0:
-        value_frame_sha = sha((gathered["frame"] if world > 1 else staging.view(h, w, 4)).cpu().numpy())
+        value_frame = (gathered["frame"] if world > 1 else staging.view(h, w, 4)).cpu().numpy()
+        value_frame_sha = sha(value_frame)
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, value_frame, last_stats if world == 1 else None)
+        del value_frame
 
     # Steps in flight.  A step is upload -> render -> frame in host memory -> destroy, each a blocking call of the public
     # API; a host that renders a sequence of frames keeps the GPU busy during the host-side parts of a step (scene
