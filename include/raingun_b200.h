@@ -123,9 +123,11 @@ enum {
 };
 /* How `Scene::trace` is evaluated (results identical; see DESIGN.md). */
 enum {
-    RG_ACCEL_AUTO = 0,  /* grid when it pays, brute force otherwise */
+    RG_ACCEL_AUTO = 0,  /* grid when it pays (64 or more spheres, boxes and disks it can bin), brute force otherwise */
     RG_ACCEL_BRUTE = 1, /* the reference algorithm: every ray x every body */
-    RG_ACCEL_GRID = 2   /* exact culling through a uniform grid + brute-force rest */
+    RG_ACCEL_GRID = 2   /* exact culling through a uniform grid + brute-force rest: spheres, and boxes (lo <= hi) and
+                           disks (radius > 0) of finite geometry through enclosing spheres; planes and other
+                           bodies are tested per ray */
 };
 /* Option keys for rg_scene_set_option. */
 enum {
@@ -158,7 +160,8 @@ typedef struct rg_stats {
     uint64_t rays_reflection;
     uint64_t rays_transmission;
     uint64_t body_tests;           /* sum over rays of n_bodies (brute-force charge) */
-    uint64_t exact_tests;          /* FP64 intersect evaluations actually executed   */
+    uint64_t exact_tests;          /* FP64 intersect evaluations actually executed (the grid tracer
+                                      counts a box or disk it tests twice for one ray twice) */
     uint64_t cull_unsound;         /* RG_OPT_VERIFY_CULL: must be 0                   */
     /* conditions on which the reference would have panicked */
     uint64_t err_nan_distance;     /* scene.rs:38 partial_cmp().unwrap()             */

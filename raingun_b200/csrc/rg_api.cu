@@ -293,8 +293,41 @@ __global__ void __launch_bounds__(256) k_cull_records(const double4 *__restrict_
                 oz = __shfl_xor_sync(0xffffffffu, rec.z, 1), ow = __shfl_xor_sync(0xffffffffu, rec.w, 1);
     if (i >= n_padded) return;
     cull4[i] = rec;
+    if (!cull2) return;   // grid proxies (rg_scene.cuh): records for the grid only
     if ((i & 1u) == 0) cull2[i] = make_float4(rec.x, ox, rec.y, oy);
     else cull2[i] = make_float4(oz, rec.z, -ow, -rec.w);
+}
+
+// A box or disk the grid may bin through an enclosing sphere (DESIGN.md section 4.2): finite geometry, a disk of
+// positive radius, a box with lo <= hi on every axis.  Everything else (planes, inverted boxes, ...) is tested per ray.
+// The proxy is the box's centre and half-diagonal, the disk's origin and radius, with the radius inflated by
+// 1e-9 (|c|_inf + r): far more than the rounding of the centre and of the radius, and than the distance by which
+// the reference's FP64 tests can place a hit outside the body for origins within 1e6 (|c|_inf + r) of it.
+static bool grid_proxy(uint8_t kind, const double *g, double out[4]) {
+    double c[3], r;
+    if (kind == RG_BODY_DISK) {
+        for (int k = 0; k < 7; ++k)
+            if (!std::isfinite(g[k])) return false;
+        if (!(g[6] > 0.0)) return false;
+        c[0] = g[0]; c[1] = g[1]; c[2] = g[2];
+        r = g[6];
+    } else if (kind == RG_BODY_AABB) {
+        double h2 = 0.0;
+        for (int k = 0; k < 3; ++k) {
+            if (!std::isfinite(g[k]) || !std::isfinite(g[k + 3]) || !(g[k] <= g[k + 3])) return false;
+            c[k] = 0.5 * g[k] + 0.5 * g[k + 3];
+            const double e = 0.5 * g[k + 3] - 0.5 * g[k];
+            h2 += e * e;
+        }
+        r = std::sqrt(h2);
+    } else {
+        return false;
+    }
+    const double cmax = std::max(std::fabs(c[0]), std::max(std::fabs(c[1]), std::fabs(c[2])));
+    r = r + 1e-9 * (cmax + r);
+    if (!std::isfinite(r)) return false;
+    out[0] = c[0]; out[1] = c[1]; out[2] = c[2]; out[3] = r;
+    return true;
 }
 
 static int build_scene(rg_scene *sc, const rg_scene_desc *d) {
@@ -319,10 +352,13 @@ static int build_scene(rg_scene *sc, const rg_scene_desc *d) {
     // ---- everything the device needs from the host, laid out in ONE pinned staging buffer -> one async copy
     // (the sphere / non-sphere lists are laid out for the worst case, so that one pass over the bodies fills everything)
     auto align = [](size_t x) { return (x + 255) & ~(size_t)255; };
+    size_t n_boxes = 0;
+    for (uint32_t i = 0; i < n; ++i) n_boxes += d->body_kind[i] == RG_BODY_AABB;
     const size_t off_kind = 0, off_geom = align(off_kind + n), off_mat = align(off_geom + (size_t)n * 64),
                  off_sph = align(off_mat + (size_t)n * sizeof(BodyMat)), off_sphb = align(off_sph + (size_t)n * 32),
                  off_misc = align(off_sphb + (size_t)n * 4), off_bsph = align(off_misc + (size_t)n * 4),
-                 total = align(off_bsph + (size_t)n * 4);
+                 off_gmisc = align(off_bsph + (size_t)n * 4), off_face = align(off_gmisc + (size_t)n * 4),
+                 total = align(off_face + n_boxes * 6 * sizeof(FaceRef));
     if (sc->h_stage_cap < total) {
         if (sc->h_stage) cudaFreeHost(sc->h_stage);
         sc->h_stage = nullptr;
@@ -339,10 +375,25 @@ static int build_scene(rg_scene *sc, const rg_scene_desc *d) {
     BodyMat *mats = reinterpret_cast<BodyMat *>(hs + off_mat);
     double *sph = reinterpret_cast<double *>(hs + off_sph);
     uint32_t *sph_body = reinterpret_cast<uint32_t *>(hs + off_sphb), *misc_body = reinterpret_cast<uint32_t *>(hs + off_misc);
-    uint32_t *body_sph = reinterpret_cast<uint32_t *>(hs + off_bsph);
-    double lo[3] = {0, 0, 0}, hi[3] = {0, 0, 0};   // bounding box of the finite sphere centres
+    uint32_t *body_sph = reinterpret_cast<uint32_t *>(hs + off_bsph), *gmisc_body = reinterpret_cast<uint32_t *>(hs + off_gmisc);
+    double lo[3] = {0, 0, 0}, hi[3] = {0, 0, 0};   // bounding box of the finite sphere and proxy centres
     bool have = false;
-    uint32_t ns = 0, nm = 0;
+    auto extend = [&](const double *c) {
+        if (!(std::isfinite(c[0]) && std::isfinite(c[1]) && std::isfinite(c[2]))) return;
+        if (!have) {
+            for (int k = 0; k < 3; ++k) lo[k] = hi[k] = c[k];
+            have = true;
+        } else {   // plain comparisons: the operands are finite (fmin / fmax are library calls here)
+            for (int k = 0; k < 3; ++k) {
+                if (c[k] < lo[k]) lo[k] = c[k];
+                if (c[k] > hi[k]) hi[k] = c[k];
+            }
+        }
+    };
+    std::vector<double> prox;            // proxies (grid_proxy), appended to the sphere list below
+    std::vector<uint32_t> prox_body;
+    std::vector<FaceRef> faces[3];       // face planes of the binned boxes, per axis
+    uint32_t ns = 0, nm = 0, ngm = 0;
     for (uint32_t i = 0; i < n; ++i) {
         BodyMat m;
         m.color[0] = d->color[3 * (size_t)i]; m.color[1] = d->color[3 * (size_t)i + 1]; m.color[2] = d->color[3 * (size_t)i + 2];
@@ -362,26 +413,41 @@ static int build_scene(rg_scene *sc, const rg_scene_desc *d) {
             std::memcpy(sph + 4 * (size_t)ns, g, 32);
             body_sph[i] = ns;
             sph_body[ns++] = i;
-            if (std::isfinite(g[0]) && std::isfinite(g[1]) && std::isfinite(g[2])) {
-                if (!have) {
-                    for (int k = 0; k < 3; ++k) lo[k] = hi[k] = g[k];
-                    have = true;
-                } else {   // plain comparisons: the operands are finite (fmin / fmax are library calls here)
-                    for (int k = 0; k < 3; ++k) {
-                        if (g[k] < lo[k]) lo[k] = g[k];
-                        if (g[k] > hi[k]) hi[k] = g[k];
-                    }
-                }
-            }
+            extend(g);
         } else {
             body_sph[i] = 0xFFFFFFFFu;
             misc_body[nm++] = i;
+            double p[4];
+            if (grid_proxy(d->body_kind[i], g, p)) {
+                prox.insert(prox.end(), p, p + 4);
+                prox_body.push_back(i);
+                extend(p);
+                if (d->body_kind[i] == RG_BODY_AABB)
+                    for (int k = 0; k < 3; ++k) {
+                        faces[k].push_back(FaceRef{g[k], i, 0u});
+                        faces[k].push_back(FaceRef{g[k + 3], i, 0u});
+                    }
+            } else {
+                gmisc_body[ngm++] = i;
+            }
         }
+    }
+    const uint32_t np = (uint32_t)prox_body.size(), nsp = ns + np;
+    if (np) {   // the combined list: spheres, then proxies
+        std::memcpy(sph + 4 * (size_t)ns, prox.data(), prox.size() * sizeof(double));
+        std::memcpy(sph_body + ns, prox_body.data(), np * sizeof(uint32_t));
+    }
+    FaceRef *face = reinterpret_cast<FaceRef *>(hs + off_face);
+    const size_t n_faces = faces[0].size();
+    for (int k = 0; k < 3; ++k) {
+        std::sort(faces[k].begin(), faces[k].end(),
+                  [](const FaceRef &a, const FaceRef &b) { return a.c < b.c || (a.c == b.c && a.body < b.body); });
+        if (n_faces) std::memcpy(face + k * n_faces, faces[k].data(), n_faces * sizeof(FaceRef));
     }
     ds.n_spheres = ns;
     ds.n_misc = nm;
     const size_t cull_padded = ((size_t)ns + 3) / 4 * 4;
-    // P = centre of the bounding box of the sphere centres: reference point of the FP32 cull coordinates
+    // P = centre of the bounding box of the sphere and proxy centres: reference point of the FP32 cull coordinates
     for (int k = 0; k < 3; ++k) ds.cull_ref[k] = have ? 0.5 * (lo[k] + hi[k]) : 0.0;
 
     for (uint32_t l = 0; l < d->n_lights; ++l) {
@@ -402,30 +468,42 @@ static int build_scene(rg_scene *sc, const rg_scene_desc *d) {
 
     lap("host flatten");
     uint8_t *dev = static_cast<uint8_t *>(sc->arena.alloc(total));
-    float4 *cull4 = static_cast<float4 *>(sc->arena.alloc(std::max<size_t>(cull_padded, 1) * sizeof(float4)));
+    float4 *cull4 = static_cast<float4 *>(sc->arena.alloc(std::max<size_t>(std::max<size_t>(cull_padded, nsp), 1) * sizeof(float4)));
     float4 *cull2 = static_cast<float4 *>(sc->arena.alloc(std::max<size_t>(cull_padded, 1) * sizeof(float4)));
     if (!dev || !cull4 || !cull2) return RG_E_NOMEM;
     RG_CUDA(cudaMemcpyAsync(dev, hs, total, cudaMemcpyHostToDevice, sc->stream));
     ds.kind = n ? dev + off_kind : nullptr;
     ds.geom = n ? reinterpret_cast<const double *>(dev + off_geom) : nullptr;
     ds.mat = n ? reinterpret_cast<const BodyMat *>(dev + off_mat) : nullptr;
-    ds.sph = ns ? reinterpret_cast<const double4 *>(dev + off_sph) : nullptr;
-    ds.sph_body = ns ? reinterpret_cast<const uint32_t *>(dev + off_sphb) : nullptr;
+    ds.sph = nsp ? reinterpret_cast<const double4 *>(dev + off_sph) : nullptr;
+    ds.sph_body = nsp ? reinterpret_cast<const uint32_t *>(dev + off_sphb) : nullptr;
     ds.misc_body = nm ? reinterpret_cast<const uint32_t *>(dev + off_misc) : nullptr;
     ds.body_sph = n ? reinterpret_cast<const uint32_t *>(dev + off_bsph) : nullptr;
-    ds.cull4 = ns ? cull4 : nullptr;
+    ds.cull4 = nsp ? cull4 : nullptr;
     ds.cull2 = ns ? cull2 : nullptr;
     if (cull_padded) {
         k_cull_records<<<(unsigned)((cull_padded + 255) / 256), 256, 0, sc->stream>>>(ds.sph, ns, (uint32_t)cull_padded, ds.cull_ref[0],
                                                                                       ds.cull_ref[1], ds.cull_ref[2], cull4, cull2);
         RG_CUDA(cudaGetLastError());
     }
+    if (np) {   // (after the spheres' launch, whose padding records it overwrites)
+        k_cull_records<<<(np + 255) / 256, 256, 0, sc->stream>>>(ds.sph + ns, np, np, ds.cull_ref[0], ds.cull_ref[1], ds.cull_ref[2],
+                                                                 cull4 + ns, nullptr);
+        RG_CUDA(cudaGetLastError());
+    }
+    GridProxies &gp = sc->gp;
+    gp = GridProxies{};
+    gp.n_proxies = np;
+    gp.n_misc = ngm;
+    gp.misc_body = ngm ? reinterpret_cast<const uint32_t *>(dev + off_gmisc) : nullptr;
+    gp.n_faces = (uint32_t)n_faces;
+    gp.faces = n_faces ? reinterpret_cast<const FaceRef *>(dev + off_face) : nullptr;
     lap("enqueue upload");
     if (dbg_timing) { cudaStreamSynchronize(sc->stream); lap("(upload done)"); }
     int rc;
     if ((rc = create_textures(sc, d))) return rc;
     lap("textures");
-    if ((rc = grid_build(sc, sph, ns))) return rc;   // (synchronises the stream: the staging buffer is free again)
+    if ((rc = grid_build(sc, sph, nsp))) return rc;   // (synchronises the stream: the staging buffer is free again)
     lap("grid");
     RG_CUDA(cudaStreamSynchronize(sc->stream));
     return RG_OK;

@@ -21,7 +21,11 @@
 //     un-normalised plane normals — non-finite origins, origins farther than 1e9 cells) skip the
 //     grid and scan every sphere exactly; origins farther than 1024 cells are first moved along
 //     the ray, in FP64, to one cell before the grid box;
-//   * spheres too large for the grid ("loose") and all non-sphere bodies are tested per ray.
+//   * spheres too large for the grid ("loose") and the non-sphere bodies the grid does not hold are tested per ray;
+//   * boxes and disks with sound geometry are binned as enclosing spheres ("proxies", rg_scene.cuh): a line that
+//     misses the ball misses the body, and every point the body's test returns lies in the ball, except in one
+//     case of the box test (an origin exactly on a face plane of an axis whose 1.0 / d_k is infinite), which the
+//     ray set-up finds through the sorted face planes and tests exactly.
 //
 // Execution model.  Ray lengths differ wildly (a lit shadow ray crosses the whole grid, an
 // occluded one stops after a few cells) and the exact FP64 test is ~10x a cull test, so a
@@ -83,12 +87,22 @@ struct GridHit {
     }
 };
 
-template <bool ANY>
+// One item of the sphere list: a sphere, or (PROXY, index >= n_spheres) a box / disk binned through its enclosing
+// sphere, which runs the body's own test.
+template <bool ANY, bool PROXY>
 __device__ __forceinline__ void exact_sphere(const DScene &s, const Ray &ray, uint32_t sph, GridHit<ANY> &h,
                                              unsigned &n_exact, unsigned &nan_count) {
     const double4 sp = s.sph[sph];
     double t;
     ++n_exact;
+    if (PROXY && sph >= s.n_spheres) {
+        const uint32_t b = s.sph_body[sph];
+        if (misc_intersect(s, b, ray, t)) {
+            if (t != t) { ++nan_count; return; }
+            h.offer(t, b);
+        }
+        return;
+    }
     if (sphere_intersect(sp.x, sp.y, sp.z, sp.w, ray, t)) {
         if (t != t) { ++nan_count; return; }
         h.offer(t, s.sph_body[sph]);
@@ -97,8 +111,10 @@ __device__ __forceinline__ void exact_sphere(const DScene &s, const Ray &ray, ui
 
 // STATS = true: the instrumented build of the same kernel (RG_OPT_TRACE_STATS) that counts cells visited,
 // records fetched, cull tests, refills and lane use into DCounters::grid_*; results are unchanged.
-template <bool ANY, bool STATS = false>
-__global__ void __launch_bounds__(kGridTraceThreads, RG_GRID_MINB) k_trace_grid(const DScene s, const TraceArgs a) {
+// PROXY = true: the grid also holds boxes and disks (`gp`, rg_scene.cuh); false: spheres only, `gp` is not read.
+template <bool ANY, bool STATS = false, bool PROXY = false>
+__global__ void __launch_bounds__(kGridTraceThreads, RG_GRID_MINB) k_trace_grid(const DScene s, const TraceArgs a,
+                                                                                const GridProxies gp) {
     const GridDev &g = s.grid;
     const uint32_t lane = threadIdx.x & 31u;
     const uint32_t lanemask_lt = (1u << lane) - 1u;
@@ -180,6 +196,7 @@ __global__ void __launch_bounds__(kGridTraceThreads, RG_GRID_MINB) k_trace_grid(
                 h.best.init();
                 h.occluded = false;
                 h.tmax = ANY ? a.tmax[pi] : 0.0;
+                if (!PROXY) {   // (verbatim as before proxies: the sphere-only kernels compile to the same SASS)
                 for (uint32_t m = 0; m < s.n_misc; ++m) {          // planes, disks, boxes: exact, per ray
                     const uint32_t b = s.misc_body[m];
                     double t;
@@ -189,6 +206,40 @@ __global__ void __launch_bounds__(kGridTraceThreads, RG_GRID_MINB) k_trace_grid(
                     }
                 }
                 n_exact += s.n_misc;
+                } else {
+                    for (uint32_t m = 0; m < gp.n_misc; ++m) {     // non-sphere bodies kept out of the grid: exact, per ray
+                        const uint32_t b = gp.misc_body[m];
+                        double t;
+                        if (misc_intersect(s, b, ray, t)) {
+                            if (t != t) { ++nan_count; continue; }
+                            h.offer(t, b);
+                        }
+                    }
+                    n_exact += gp.n_misc;
+                    // The one case where the reference's box test can return a point outside the box: 1.0 / d_k is
+                    // infinite and o_k lies exactly on a face plane of axis k (0 * inf = NaN drops a slab check).
+                    // Such boxes are found through the sorted face planes and tested here, whatever else happens.
+                    const double od[3] = {ray.o.x, ray.o.y, ray.o.z}, dd[3] = {ray.d.x, ray.d.y, ray.d.z};
+#pragma unroll 1
+                    for (int k = 0; k < 3; ++k) {
+                        if (!isinf(1.0 / dd[k])) continue;
+                        const FaceRef *f = gp.faces + (size_t)k * gp.n_faces;
+                        uint32_t lo = 0, hi = gp.n_faces;
+                        while (lo < hi) {
+                            const uint32_t mid = (lo + hi) >> 1;
+                            if (f[mid].c < od[k]) lo = mid + 1; else hi = mid;
+                        }
+                        for (; lo < gp.n_faces && f[lo].c == od[k]; ++lo) {
+                            const uint32_t b = f[lo].body;
+                            double t;
+                            ++n_exact;
+                            if (aabb_intersect(s.geom + 8 * (size_t)b, ray, t)) {
+                                if (t != t) { ++nan_count; continue; }
+                                h.offer(t, b);
+                            }
+                        }
+                    }
+                }
                 if (ANY && skip == kHintOccluded) h.occluded = true;   // the sphere the ray starts on is in the way
                 if (!(ANY && h.occluded)) {
                 cr = make_cull_ray(s, ray, true);
@@ -239,13 +290,17 @@ __global__ void __launch_bounds__(kGridTraceThreads, RG_GRID_MINB) k_trace_grid(
                                       fabsf(ogy) <= kGridMaxCoord && fabsf(ogz) <= kGridMaxCoord));   // false on NaN
                 {
                     if (!walkable) {
-                        // outside the conservativeness argument: scan every sphere (cull + exact)
+                        // outside the conservativeness argument: scan every sphere (cull + exact) and every proxy's
+                        // body (exact: the cull's bound on a proxy assumes |d| = 1 within the walk's 1e-9, DESIGN 4.2)
                         for (uint32_t q = 0; q < s.n_spheres; ++q)
-                            if (q != skip && !cull_reject(cr, s.cull4[q])) exact_sphere<ANY>(s, ray, q, h, n_exact, nan_count);
+                            if (q != skip && !cull_reject(cr, s.cull4[q])) exact_sphere<ANY, PROXY>(s, ray, q, h, n_exact, nan_count);
+                        if (PROXY)
+                            for (uint32_t q = s.n_spheres; q < s.n_spheres + gp.n_proxies; ++q)
+                                exact_sphere<ANY, PROXY>(s, ray, q, h, n_exact, nan_count);
                     } else {
                         for (uint32_t q = 0; q < g.n_loose; ++q) {
                             const uint32_t sp = g.loose[q];
-                            if (sp != skip && !cull_reject(cr, s.cull4[sp])) exact_sphere<ANY>(s, ray, sp, h, n_exact, nan_count);
+                            if (sp != skip && !cull_reject(cr, s.cull4[sp])) exact_sphere<ANY, PROXY>(s, ray, sp, h, n_exact, nan_count);
                         }
                         // clip the ray to the grid box [0, dim]
                         const float ix = 1.0f / dgx, iy = 1.0f / dgy, iz = 1.0f / dgz;
@@ -379,8 +434,8 @@ __global__ void __launch_bounds__(kGridTraceThreads, RG_GRID_MINB) k_trace_grid(
                 const Ray ray = load_ray(a.q, pi);
                 const uint32_t first = pend0 != kNoSphere ? pend0 : pend1;
                 const uint32_t second = pend0 != kNoSphere ? pend1 : kNoSphere;
-                exact_sphere<ANY>(s, ray, first, h, n_exact, nan_count);
-                if (second != kNoSphere) exact_sphere<ANY>(s, ray, second, h, n_exact, nan_count);
+                exact_sphere<ANY, PROXY>(s, ray, first, h, n_exact, nan_count);
+                if (second != kNoSphere) exact_sphere<ANY, PROXY>(s, ray, second, h, n_exact, nan_count);
                 skip = second != kNoSphere ? second : first;   // re-listed in the cells that follow: same ray, same answer
                 pend0 = pend1 = kNoSphere;
                 boundf = h.bound() - t0f;

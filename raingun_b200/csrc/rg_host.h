@@ -87,6 +87,7 @@ struct rg_scene {
     rg::MultiState *multi = nullptr;       // set: this handle spans several GPUs (rg_multi.cu) and owns no device state itself
     std::atomic<bool> busy{false};         // a render call is running on this handle (second callers get RG_E_BUSY)
     rg::DScene ds{};                    // device pointers inside
+    rg::GridProxies gp{};               // boxes and disks binned into the grid (rg_scene.cuh)
     rg::SceneArena arena;               // scene arrays
     std::vector<cudaTextureObject_t> tex_objs;
     rg::DCounters *d_counters = nullptr;

@@ -7,7 +7,8 @@
 //     the "misc" list (planes, disks, boxes: few, tested one by one in f64).  The original
 //     index travels with every candidate because Scene::trace keeps the FIRST of equal
 //     minima (scene.rs:34-39);
-//   * cull4[n_spheres]: the FP32 conservative-cull record of each sphere (rg_trace.cuh);
+//   * cull4[n_spheres]: the FP32 conservative-cull record of each sphere (rg_trace.cuh), followed by those of
+//     the grid's box / disk proxies (GridProxies below);
 //   * the exact-culling grid (rg_grid.cuh);
 //   * lights by value inside the struct (<= RG_MAX_LIGHTS), textures as CUDA texture objects.
 #pragma once
@@ -68,8 +69,8 @@ struct DScene {
     const uint8_t *kind;
     const double *geom;           // [n_bodies][8]
     const BodyMat *mat;
-    const double4 *sph;           // [n_spheres] cx, cy, cz, r
-    const uint32_t *sph_body;     // [n_spheres] original body index
+    const double4 *sph;           // [n_spheres] cx, cy, cz, r (+ the grid's proxies behind them, GridProxies)
+    const uint32_t *sph_body;     // [n_spheres] original body index (+ the proxies')
     const uint32_t *body_sph;     // [n_bodies] the body's index in the sphere list (0xFFFFFFFF: not a sphere)
     const float4 *cull4;          // [n_spheres] c - P (f32), K - m_s       (rg_trace.cuh)
     const float4 *cull2;          // the same records pair-interleaved for FFMA2: (x0,x1,y0,y1)(z0,z1,-K0,-K1)
@@ -81,6 +82,23 @@ struct DScene {
     uint32_t max_depth;
     GridDev grid;
     DLight lights[RG_MAX_LIGHTS];
+};
+
+// Boxes and disks in the grid (rg_grid.cuh, DESIGN.md section 4.2).  A binnable box or disk enters the grid as
+// a sphere that encloses it (its "proxy"): DScene::sph[n_spheres, n_spheres + n_proxies), with its body index in
+// sph_body[] and its FP32 cull record in cull4[].  Only k_trace_grid reads this struct; it travels as a kernel
+// argument of its own, so that DScene — and every kernel that takes it — is what it is in a sphere-only scene.
+struct FaceRef {                  // one face plane of a binned box: the bound's coordinate and the box's body index
+    double c;
+    uint32_t body;
+    uint32_t pad;
+};
+struct GridProxies {
+    uint32_t n_proxies;
+    uint32_t n_misc;              // non-sphere bodies kept out of the grid (planes, inverted boxes, ...): tested per ray
+    const uint32_t *misc_body;    // [n_misc] original body index
+    uint32_t n_faces;             // = 2 x binned boxes
+    const FaceRef *faces;         // [3][n_faces]: per axis k, (lo_k, box) and (hi_k, box) of every binned box, sorted by c
 };
 
 // Per recursion level, for the host-free wavefront loop (rg_wavefront.cu): every launch of a

@@ -467,8 +467,13 @@ static int launch_trace(rg_scene *sc, const TraceArgs &ta, bool use_grid, cudaSt
             tuned.fetch = ANY ? &ta.ctr->fetch_shadow : &ta.ctr->fetch;   // the two kinds may run concurrently
             RG_CUDA(cudaMemsetAsync(tuned.fetch, 0, sizeof(unsigned int), stream));
         }
-        if (sc->trace_stats) k_trace_grid<ANY, true><<<blocks, kGridTraceThreads, 0, stream>>>(sc->ds, tuned);
-        else k_trace_grid<ANY, false><<<blocks, kGridTraceThreads, 0, stream>>>(sc->ds, tuned);
+        if (sc->gp.n_proxies) {   // boxes / disks in the grid
+            if (sc->trace_stats) k_trace_grid<ANY, true, true><<<blocks, kGridTraceThreads, 0, stream>>>(sc->ds, tuned, sc->gp);
+            else k_trace_grid<ANY, false, true><<<blocks, kGridTraceThreads, 0, stream>>>(sc->ds, tuned, sc->gp);
+        } else {
+            if (sc->trace_stats) k_trace_grid<ANY, true><<<blocks, kGridTraceThreads, 0, stream>>>(sc->ds, tuned, sc->gp);
+            else k_trace_grid<ANY, false><<<blocks, kGridTraceThreads, 0, stream>>>(sc->ds, tuned, sc->gp);
+        }
     } else if (brute_resident_fits(sc) && ta.n >= (uint32_t)sc->sm_count * 64u * 32u) {
         // the whole cull array fits in one SM's shared memory: one persistent CTA per SM, warps
         // pull ray tiles from a counter and never meet at a barrier again (rg_trace.cuh)
@@ -1022,7 +1027,7 @@ int wavefront_render(rg_scene *sc, uint32_t width, uint32_t height, uint32_t y0,
     const DScene &ds = sc->ds;
     bool use_grid = false;
     if (sc->accel == RG_ACCEL_GRID) use_grid = ds.grid.enabled != 0;
-    else if (sc->accel == RG_ACCEL_AUTO) use_grid = ds.grid.enabled != 0 && ds.n_spheres >= 64;
+    else if (sc->accel == RG_ACCEL_AUTO) use_grid = ds.grid.enabled != 0 && ds.n_spheres + sc->gp.n_proxies >= 64;
     st->accel_used = use_grid ? RG_ACCEL_GRID : RG_ACCEL_BRUTE;
 
     EventPool events(sc->wf.events);

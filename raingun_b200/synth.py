@@ -131,3 +131,64 @@ def make_scene(name: str, spheres: Optional[int] = None, depth: Optional[int] = 
     spec = SPECS[name]
     doc = make_scene_doc(spec, spheres, depth)
     return scene_from_dict(doc, texture_loader or default_texture_loader), spec
+
+
+# B4: the box-and-disk counterpart of C4, kept out of SPECS (the benchmark's configs).  Same volume, lights
+# and depth as C4 / C3; `spheres` counts its bodies and `radius` is the range of a box's half-extents.
+B4 = SynthSpec("B4", 3840, 2160, 1004, 10000, 24.0, (-1.5, 18.0), (-45.0, -4.0), (0.06, 0.3),
+               True, False, 3, 8)
+B4_DISK_RADIUS = (0.08, 0.35)
+
+
+def make_box_scene_doc(bodies: Optional[int] = None, depth: Optional[int] = None) -> Dict[str, Any]:
+    """The YAML document of B4: 3840x2160, depth 8, C3's three lights, a ground plane (body 0) and
+    10,000 boxes and disks in C4's volume.  SplitMix64 seed 1004, ``U`` as for C3-C5; per body the
+    draw order is x, y, z, a kind selector, then for a selector below 0.7 an AABB with half-extents
+    U(0.06, 0.3) drawn for x, y, z (bounds rounded to 6 decimals), else a Disk with radius
+    U(0.08, 0.35) and normal components U(-1, 1) drawn for x, y, z; then colour, albedo, surface
+    selector and surface parameters exactly as C4 draws them.  ``bodies`` / ``depth`` shrink the
+    scene for parity tests; the stream is the same, just cut short."""
+    spec = B4
+    n = spec.spheres if bodies is None else int(bodies)
+    rng = SplitMix64(spec.seed)
+    out: List[Dict[str, Any]] = [{"Plane": {
+        "origin": [0.0, -2.0, -5.0], "normal": [0.0, -1.0, 0.0],
+        "material": {"coloration": {"Color": "#808080"}, "albedo": 0.3, "surface": "Diffuse"}}}]
+    for _ in range(n):
+        x = rng.uniform(-spec.box_x, spec.box_x)
+        y = rng.uniform(*spec.box_y)
+        z = rng.uniform(*spec.box_z)
+        if rng.uniform(0.0, 1.0) < 0.7:
+            hx, hy, hz = (rng.uniform(*spec.radius) for _ in range(3))
+            lo = [round(x - hx, 6), round(y - hy, 6), round(z - hz, 6)]
+            hi = [round(x + hx, 6), round(y + hy, 6), round(z + hz, 6)]
+            kind, geom = "AABB", {"bounds": [lo, hi]}
+        else:
+            r = rng.uniform(*B4_DISK_RADIUS)
+            normal = [rng.uniform(-1.0, 1.0) for _ in range(3)]
+            kind, geom = "Disk", {"origin": [x, y, z], "normal": normal, "radius": r}
+        colour = "#%06x" % (rng.next_u64() & 0xFFFFFF)
+        albedo = rng.uniform(0.2, 0.9)
+        s = rng.uniform(0.0, 1.0)
+        surface: Any = "Diffuse"
+        if s < 0.4:
+            surface = {"Reflecting": {"reflectivity": rng.uniform(0.2, 0.9)}}
+        elif s < 0.8:
+            index = rng.uniform(1.1, 1.8)
+            surface = {"Refractive": {"index": index, "transparency": rng.uniform(0.7, 1.0)}}
+        geom["material"] = {"coloration": {"Color": colour}, "albedo": albedo, "surface": surface}
+        out.append({kind: geom})
+    return {"fov": 90.0, "defaultColor": "#667fff",
+            "maxRecursionDepth": spec.depth if depth is None else int(depth),
+            "lights": _lights(spec), "bodies": out}
+
+
+def make_box_scene(name: str = "B4", bodies: Optional[int] = None, depth: Optional[int] = None,
+                   texture_loader=None):
+    """SceneData of the box-and-disk scene ``B4`` (see make_box_scene_doc) and its spec."""
+    from .scene import default_texture_loader, scene_from_dict
+
+    if name != "B4":
+        raise KeyError(name)
+    doc = make_box_scene_doc(bodies, depth)
+    return scene_from_dict(doc, texture_loader or default_texture_loader), B4
