@@ -138,9 +138,9 @@ enum {
     RG_OPT_VERIFY_CULL = 5,  /* debug: count FP32-culled pairs the FP64 test hits  */
     RG_OPT_OVERLAP = 6,      /* shadow side of a level concurrent with the next level's path side:
                                 0 = automatic (on with the grid tracer), 1 = off, 2 = on */
-    RG_OPT_HOST_FREE = 7,    /* the level loop without host involvement (device-sized launches, one
-                                synchronisation per frame; render_image is one call, rendering.rs:24-38):
-                                0 = automatic (on), 1 = off (host reads every level's size), 2 = on */
+    RG_OPT_HOST_FREE = 7,    /* obsolete: every wavefront frame runs the host-free level loop (device-sized
+                                launches, one synchronisation per frame; render_image is one call,
+                                rendering.rs:24-38).  Values 0-2 are accepted and ignored */
     RG_OPT_GRAPH = 8,        /* replay the host-free frame as one CUDA graph: 0 = automatic, 1 = off, 2 = on */
     RG_OPT_TRACE_STATS = 9,  /* 1 = the grid tracer counts cells / fetches / cull tests / lane use
                                 (rg_stats.grid_*); an instrumented kernel, slower; results unchanged */
@@ -174,7 +174,8 @@ typedef struct rg_stats {
     uint32_t batches;              /* wavefront batches                              */
     uint32_t max_level;            /* deepest level that traced a ray                */
     uint32_t accel_used;           /* RG_ACCEL_BRUTE | RG_ACCEL_GRID                 */
-    uint32_t host_free;            /* 1 = the frame ran without host synchronisation (RG_OPT_HOST_FREE) */
+    uint32_t host_free;            /* 1 = the frame ran without host synchronisation (every wavefront frame;
+                                      0 for the megakernel) */
     uint32_t graph_replays;        /* batches replayed from a captured CUDA graph    */
     /* RG_OPT_TRACE_STATS (grid tracer only; zero otherwise) */
     uint64_t grid_cells;           /* grid cells visited by all rays                 */

@@ -39,7 +39,7 @@ pub const RG_OPT_MAX_DEPTH: i32 = 3; // src/main.rs:119-123
 pub const RG_OPT_BATCH_PIXELS: i32 = 4;
 pub const RG_OPT_VERIFY_CULL: i32 = 5;
 pub const RG_OPT_OVERLAP: i32 = 6;
-pub const RG_OPT_HOST_FREE: i32 = 7;
+pub const RG_OPT_HOST_FREE: i32 = 7; // obsolete: accepted (0-2) and ignored
 pub const RG_OPT_GRAPH: i32 = 8;
 pub const RG_OPT_TRACE_STATS: i32 = 9;
 pub const RG_OPT_SCHEDULE: i32 = 11;

@@ -78,8 +78,6 @@ void WavefrontScratch::release() {
     sync_events.clear();
     if (aux) cudaStreamDestroy(aux);
     aux = nullptr;
-    if (rb) cudaStreamDestroy(rb);
-    rb = nullptr;
 }
 
 void GraphCache::release() {
@@ -732,9 +730,8 @@ int rg_scene_set_option(rg_scene *sc, int32_t key, int64_t value) {
             if (value < 0 || value > 2) break;
             sc->overlap = (int)value;
             return RG_OK;
-        case RG_OPT_HOST_FREE:
+        case RG_OPT_HOST_FREE:   // obsolete: every wavefront frame runs the host-free loop; accepted and ignored
             if (value < 0 || value > 2) break;
-            sc->host_free = (int)value;
             return RG_OK;
         case RG_OPT_GRAPH:
             if (value < 0 || value > 2) break;

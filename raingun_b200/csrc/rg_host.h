@@ -57,12 +57,11 @@ struct WavefrontScratch {
     std::vector<DeviceBuffer> nodes;   // per level: NodeA float4 + NodeB uint4
     std::vector<cudaEvent_t> events;   // timing events of the trace launches, reused across frames
     cudaStream_t aux = nullptr;        // shadow-side stream (created on first use)
-    cudaStream_t rb = nullptr;         // counter read-back stream (lets the main stream run ahead of the host)
     std::vector<cudaEvent_t> sync_events;   // cross-stream dependencies (no timing), reused across frames
     void release();
 };
 
-// Captured host-free frames (rg_wavefront.cu): the launch sequence of a batch depends only on its
+// Captured wavefront frames (rg_wavefront.cu): the launch sequence of a batch depends only on its
 // key (batch geometry, output pointers, options, scratch addresses), so it is captured once into a
 // CUDA graph and replayed; a key must be seen twice before it is worth an instantiation.
 struct GraphEntry {
@@ -109,12 +108,12 @@ struct rg_scene {
     uint64_t batch_pixels = 0;
     int verify_cull = 0;
     int overlap = 0;                       // RG_OPT_OVERLAP: 0 auto (on with the grid tracer), 1 off, 2 on
-    int host_free = 0;                     // RG_OPT_HOST_FREE: 0 auto (on), 1 off (host-sized loop), 2 on
     int graph = 0;                         // RG_OPT_GRAPH: 0 auto, 1 off, 2 on
     bool trace_stats = false;              // RG_OPT_TRACE_STATS
     bool origin_hints = true;              // RG_OPT_ORIGIN_HINTS
     uint32_t depth_hint = 0;               // levels the ray tree of this scene has been seen to use (0 = unknown)
-    bool host_free_overflowed = false;     // a level once outgrew the default queue capacity: stay with the host-sized loop
+    uint32_t level_growth = 2;             // wavefront queue of level d holds min(2^d, level_growth) x the batch's pixels;
+                                           // doubled when a level outgrows its queue (the frame is then repeated)
     bool out_f32 = false;                  // this call delivers unquantised f32 colours, 3 per pixel (rg_render_rows_f32)
     bool scatter_out = false;              // this call stores rows at their place in a full frame (rg_render_rowlist_scatter)
     // derived

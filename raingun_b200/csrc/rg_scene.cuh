@@ -101,8 +101,8 @@ struct GridProxies {
     const FaceRef *faces;         // [3][n_faces]: per axis k, (lo_k, box) and (hi_k, box) of every binned box, sorted by c
 };
 
-// Per recursion level, for the host-free wavefront loop (rg_wavefront.cu): every launch of a
-// level reads its size from here instead of from the host.  Zeroed at the start of a batch.
+// Per recursion level of the wavefront loop (rg_wavefront.cu): every launch of a level reads its
+// size from here instead of from the host.  Zeroed at the start of a batch.
 struct DLevelCtr {
     unsigned int n;                    // path rays of this level (written by k_generate / the level above's k_shade)
     unsigned int n_lit;                // hits of this level that need shadow rays
@@ -116,11 +116,7 @@ struct DCounters {
     unsigned long long exact_tests;
     unsigned long long cull_unsound;
     unsigned long long err_nan, err_trans, err_aabb;
-    unsigned int q_next;               // wavefront: children emitted into the next level
-    unsigned int q_lit;                // wavefront: hits that need shadow rays
-    unsigned int fetch;                // persistent trace kernels: next unclaimed ray of the queue
-    unsigned int fetch_shadow;         // ... of the shadow queue (the two kinds of trace run concurrently)
-    // ---- host-free loop
+    // ---- wavefront loop
     unsigned int overflow;             // a level outgrew its queue capacity: the frame is void, the host re-renders
     unsigned int max_level;            // deepest level that held a ray
     unsigned int deeper;               // the last enqueued level emitted children (depth hint too small): frame void

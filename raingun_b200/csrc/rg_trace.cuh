@@ -52,17 +52,17 @@ constexpr uint32_t kHintOccluded = 0xFFFFFFFEu;
 struct TraceArgs {
     RayQueue q;
     const double *tmax;      // ANY: light.distance(hit_point) per ray
-    uint32_t n;
-    uint32_t seg_len, seg_stride;   // light-major shadow queues: ray i lives at (i / seg_len) * seg_stride + i % seg_len
-    const unsigned int *seg_len_dev;   // ... with seg_len (= lit hits of the level) read from device memory (host-free loop)
+    uint32_t n;              // capacity of the queue: an upper bound of the ray count
+    uint32_t seg_stride;     // light-major shadow queues: ray i lives at (i / seg_len) * seg_stride + i % seg_len
+    const unsigned int *seg_len_dev;   // ... with seg_len (= lit hits of the level) read from device memory; nullptr: dense
     double *out_t;           // nearest: distance (undefined when body == kNoBody)
     uint32_t *out_body;      // nearest: original body index or kNoBody
     uint8_t *out_lit;        // ANY: 1 = in light
     DCounters *ctr;
-    unsigned int *fetch;     // persistent kernels: the ray counter of THIS launch (ctr->fetch / ctr->fetch_shadow)
-    const unsigned int *n_dev;   // if set, the ray count is *n_dev * n_mul, read from device memory (a launch issued
-                                 // before the host knows it); `n` is then the capacity of the queue (an upper bound)
-    uint32_t n_mul;              // 0 means 1; shadow queues: lights per lit hit
+    unsigned int *fetch;     // persistent kernels: the ray counter of THIS launch (one per level and kind, zeroed per batch)
+    const unsigned int *n_dev;   // the ray count is *n_dev * n_mul, read from device memory (a launch issued
+                                 // before the host knows it)
+    uint32_t n_mul;              // path queues: 1; shadow queues: lights per lit hit
     const unsigned int *void_flag;   // if set and non-zero, the frame is void (a queue overflowed): trace nothing
     int verify;              // RG_OPT_VERIFY_CULL
     int g_refill, g_quorum, g_burst;   // persistent grid kernel tuning (rg_grid.cuh)
@@ -70,17 +70,16 @@ struct TraceArgs {
 
 // Number of rays this launch has to trace (see TraceArgs::n_dev).
 __device__ __forceinline__ uint32_t ray_count(const TraceArgs &a) {
-    if (!a.n_dev) return a.n;
     if (a.void_flag && *a.void_flag) return 0u;
-    const unsigned long long v = (unsigned long long)*a.n_dev * (a.n_mul ? a.n_mul : 1u);
+    const unsigned long long v = (unsigned long long)*a.n_dev * a.n_mul;
     return v < a.n ? (uint32_t)v : a.n;
 }
 
-// Path queues are dense (seg_len = 0).  Shadow queues hold one segment per light so that
+// Path queues are dense (seg_len = 0, no seg_len_dev).  Shadow queues hold one segment per light so that
 // neighbouring lanes trace neighbouring hits towards the SAME light (coherent origins AND directions:
 // measured -23 % on the all-diffuse C3 frame, -4 % on C4 against hit-major order).
 __device__ __forceinline__ uint32_t segment_length(const TraceArgs &a) {
-    if (!a.seg_len_dev) return a.seg_len;
+    if (!a.seg_len_dev) return 0u;
     const uint32_t v = *a.seg_len_dev;
     return v < a.seg_stride ? v : a.seg_stride;
 }

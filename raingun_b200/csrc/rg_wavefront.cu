@@ -45,27 +45,25 @@ struct LevelBuffers {
     float2 *s_ab;
     float4 *lit_bc;
     uint32_t *lit_node;
-    uint32_t n;            // rays of this level — or, with n_dev, the capacity of its queue
+    uint32_t cap;          // capacity of this level's queue
     uint32_t shadow_sl, shadow_sj;   // shadow ray of (lit hit j, light l) lives at l * shadow_sl + j * shadow_sj
     uint32_t can_spawn;    // depth + 1 < max_recursion_depth
-    // host-free loop: sizes live on the device
-    const unsigned int *n_dev;       // the level's ray count (nullptr: n is exact)
-    unsigned int *q_next, *q_lit;    // counters k_shade appends to: children (= next level's n), lit hits
+    // sizes live on the device
+    const unsigned int *n_dev;       // the level's ray count
+    unsigned int *q_next, *q_lit;    // counters k_shade appends to: children (= next level's n_dev), lit hits
     uint32_t cap_next;               // capacity of the next level's queue
     unsigned int *void_flag;         // set when a queue overflows; once set, every later launch does nothing
     uint32_t level;                  // recursion depth of this level
-    uint32_t count_on_device;        // shadow rays / deepest level are counted in DCounters (host-free loop)
     uint32_t last_enqueued;          // no launch follows for this level's children (depth hint): flag them
     uint32_t hints;                  // the tracer reads origin hints (rg_trace.cuh): 1 = compute them, 2 = write kHintNone
                                      // (RG_OPT_ORIGIN_HINTS = 0), 0 = the tracer ignores them (brute force): write nothing
 };
 
-// Size of a level as its kernels see it (host-sized, or read from the device and clamped to the capacity).
-__device__ __forceinline__ uint32_t level_size(uint32_t n, const unsigned int *n_dev, const unsigned int *void_flag) {
-    if (!n_dev) return n;
-    if (void_flag && *void_flag) return 0u;
+// Size of a level as its kernels see it: read from the device and clamped to the capacity (0 once the frame is void).
+__device__ __forceinline__ uint32_t level_size(uint32_t cap, const unsigned int *n_dev, const unsigned int *void_flag) {
+    if (*void_flag) return 0u;
     const uint32_t v = *n_dev;
-    return v < n ? v : n;
+    return v < cap ? v : cap;
 }
 
 // Order of the level-0 queue.  Rows of a batch are taken in strips of `strip` rows and a strip is
@@ -125,12 +123,12 @@ __device__ __forceinline__ uint32_t shadow_origin_hint(const double *og, uint32_
 #endif
 __global__ void __launch_bounds__(256, RG_SHADE_MINB) k_shade(const DScene s, const LevelBuffers lb, DCounters *ctr) {
     const uint32_t lane = threadIdx.x & 31u, lt = (1u << lane) - 1u;
-    const uint32_t n_level = level_size(lb.n, lb.n_dev, lb.void_flag);
-    if (lb.count_on_device && blockIdx.x == 0 && threadIdx.x == 0 && n_level) atomicMax(&ctr->max_level, lb.level);
+    const uint32_t n_level = level_size(lb.cap, lb.n_dev, lb.void_flag);
+    if (blockIdx.x == 0 && threadIdx.x == 0 && n_level) atomicMax(&ctr->max_level, lb.level);
     __shared__ uint32_t sh_cnt[3];     // lit, reflection, transmission entries of this block
     __shared__ uint32_t sh_base[2];    // block base in the lit / next-level queues
     __shared__ uint32_t sh_drop;       // the next level's queue is full: this block's children are dropped (frame void)
-    // grid-stride over the level: the launch is sized by the host (exact n) or by the queue's capacity
+    // grid-stride over the level: the launch is sized by the queue's capacity
     for (uint32_t base = blockIdx.x * blockDim.x; base < n_level; base += gridDim.x * blockDim.x) {
     const uint32_t i = base + threadIdx.x;
     const bool active = i < n_level;
@@ -199,14 +197,14 @@ __global__ void __launch_bounds__(256, RG_SHADE_MINB) k_shade(const DScene s, co
             if (n_next_b) ctr->deeper = 1u;   // the host repeats the frame with every level
         } else {
             sh_base[1] = n_next_b ? atomicAdd(lb.q_next, n_next_b) : 0u;
-            if (n_next_b && (uint64_t)sh_base[1] + n_next_b > lb.cap_next) {   // only possible with device-sized queues
+            if (n_next_b && (uint64_t)sh_base[1] + n_next_b > lb.cap_next) {   // the host repeats the frame with larger queues
                 sh_drop = 1u;
                 atomicExch(lb.void_flag, 1u);
             }
         }
         if (n_next_b - n_trans_b) atomicAdd(&ctr->rays[2], (unsigned long long)(n_next_b - n_trans_b));
         if (n_trans_b) atomicAdd(&ctr->rays[3], (unsigned long long)n_trans_b);
-        if (lb.count_on_device && n_lit_b) atomicAdd(&ctr->rays[1], (unsigned long long)n_lit_b * s.n_lights);
+        if (n_lit_b) atomicAdd(&ctr->rays[1], (unsigned long long)n_lit_b * s.n_lights);
     }
     __syncthreads();
     if (sh_drop) { want_refl = false; want_trans = false; }
@@ -264,10 +262,10 @@ __global__ void __launch_bounds__(256, RG_SHADE_MINB) k_shade(const DScene s, co
 // rendering.rs:140,157-171: final_color accumulates light by light, in scene order, then clamps.
 __global__ void __launch_bounds__(256) k_diffuse(const DScene s, const float4 *__restrict__ lit_bc,
                                                  const uint32_t *__restrict__ lit_node, const float2 *__restrict__ s_ab,
-                                                 const uint8_t *__restrict__ s_lit, float4 *node_a, uint32_t n_lit_host,
+                                                 const uint8_t *__restrict__ s_lit, float4 *node_a, uint32_t cap,
                                                  uint32_t shadow_sl, uint32_t shadow_sj, const unsigned int *n_lit_dev,
                                                  const unsigned int *void_flag) {
-    const uint32_t n_lit = level_size(n_lit_host, n_lit_dev, void_flag);
+    const uint32_t n_lit = level_size(cap, n_lit_dev, void_flag);
     for (uint32_t j = blockIdx.x * blockDim.x + threadIdx.x; j < n_lit; j += gridDim.x * blockDim.x) {
     const float4 b = lit_bc[j];
     const C3 bc = c3(b.x, b.y, b.z);
@@ -288,9 +286,9 @@ __global__ void __launch_bounds__(256) k_diffuse(const DScene s, const float4 *_
 // get_color's combination of child colours (rendering.rs:88-93, 112-116), one level at a time,
 // deepest level first.  `child_a` is the (already final) level below.
 __global__ void __launch_bounds__(256) k_combine(const DScene s, float4 *node_a, const uint4 *__restrict__ node_b,
-                                                 const float4 *__restrict__ child_a, uint32_t n_host,
+                                                 const float4 *__restrict__ child_a, uint32_t cap,
                                                  const unsigned int *n_dev, const unsigned int *void_flag) {
-    const uint32_t n = level_size(n_host, n_dev, void_flag);
+    const uint32_t n = level_size(cap, n_dev, void_flag);
     const C3 dflt = c3(s.default_color[0], s.default_color[1], s.default_color[2]);
     for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) {
     const uint4 b = node_b[i];
@@ -378,8 +376,8 @@ __global__ void __launch_bounds__(256) k_quantise_scatter(const float4 *__restri
 template <bool ANY>
 __global__ void __launch_bounds__(128) k_verify_trace(const DScene s, const TraceArgs a, int level) {
     const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= a.n) return;
-    const uint32_t pi = phys_index(a.seg_len, a.seg_stride, i);
+    if (i >= ray_count(a)) return;
+    const uint32_t pi = phys_index(segment_length(a), a.seg_stride, i);
     const Ray ray = load_ray(a.q, pi);
     const Nearest h = trace_exact_all(s, ray, a.ctr);
     bool bad;
@@ -454,7 +452,7 @@ template <bool ANY>
 static int launch_trace(rg_scene *sc, const TraceArgs &ta, bool use_grid, cudaStream_t stream) {
     if (ta.n == 0) return RG_OK;
     if (use_grid) {
-        // persistent warps: enough blocks to fill the chip, each pulling rays from ctr->fetch
+        // persistent warps: enough blocks to fill the chip, each pulling rays from ta.fetch
         const unsigned want = (ta.n + kGridTraceThreads - 1) / kGridTraceThreads;
         static const int bps = [] { const char *e = getenv("RG_GRID_BPS"); return e ? atoi(e) : RG_GRID_MINB; }();
         static const int t_refill = [] { const char *e = getenv("RG_GRID_REFILL"); return e ? atoi(e) : kGridRefill; }();
@@ -463,10 +461,6 @@ static int launch_trace(rg_scene *sc, const TraceArgs &ta, bool use_grid, cudaSt
         const unsigned blocks = std::min<unsigned>(want, (unsigned)(sc->sm_count * bps));
         TraceArgs tuned = ta;
         tuned.g_refill = t_refill; tuned.g_quorum = t_quorum; tuned.g_burst = t_burst;
-        if (!ta.fetch) {   // (the host-free loop brings a counter per level, zeroed once per batch)
-            tuned.fetch = ANY ? &ta.ctr->fetch_shadow : &ta.ctr->fetch;   // the two kinds may run concurrently
-            RG_CUDA(cudaMemsetAsync(tuned.fetch, 0, sizeof(unsigned int), stream));
-        }
         if (sc->gp.n_proxies) {   // boxes / disks in the grid
             if (sc->trace_stats) k_trace_grid<ANY, true, true><<<blocks, kGridTraceThreads, 0, stream>>>(sc->ds, tuned, sc->gp);
             else k_trace_grid<ANY, false, true><<<blocks, kGridTraceThreads, 0, stream>>>(sc->ds, tuned, sc->gp);
@@ -479,11 +473,6 @@ static int launch_trace(rg_scene *sc, const TraceArgs &ta, bool use_grid, cudaSt
         // pull ray tiles from a counter and never meet at a barrier again (rg_trace.cuh)
         static const int variant = [] { const char *e = getenv("RG_RESIDENT_VARIANT"); return e ? atoi(e) : 0; }();
         const uint32_t n_records = (uint32_t)(((size_t)sc->ds.n_spheres + 3) / 4 * 4);
-        TraceArgs tuned = ta;
-        if (!ta.fetch) {
-            tuned.fetch = ANY ? &ta.ctr->fetch_shadow : &ta.ctr->fetch;
-            RG_CUDA(cudaMemsetAsync(tuned.fetch, 0, sizeof(unsigned int), stream));
-        }
 #define RG_LAUNCH_RESIDENT(R_, U_, T_, PF_)                                                                                   \
     do {                                                                                                                      \
         static std::atomic<uint64_t> attr_set{0}; /* per device: the attribute belongs to the device's copy of the function */ \
@@ -495,7 +484,7 @@ static int launch_trace(rg_scene *sc, const TraceArgs &ta, bool use_grid, cudaSt
         }                                                                                                                     \
         const uint64_t tiles = ((uint64_t)ta.n + 32 * R_ - 1) / (32 * R_);                                                     \
         const unsigned blocks = (unsigned)std::min<uint64_t>((uint64_t)sc->sm_count, (tiles + (T_ / 32) - 1) / (T_ / 32));      \
-        k_trace_brute_resident<ANY, R_, U_, T_, PF_><<<blocks, T_, resident_smem_bytes(n_records, R_, T_ / 32), stream>>>(sc->ds, tuned, n_records); \
+        k_trace_brute_resident<ANY, R_, U_, T_, PF_><<<blocks, T_, resident_smem_bytes(n_records, R_, T_ / 32), stream>>>(sc->ds, ta, n_records); \
     } while (0)
         // Measured on C4 / C3 (ms per 4K brute-force frame) with the software-pipelined loop of round 2 (rg_trace.cuh):
         // R=4,U=2,512 thr 310.0 / 14.3;  R=3,U=2: 512 thr 313.4 / 17.6, 576 thr 322.1 / 9.1, 608 thr 322.1 / 10.1,
@@ -541,228 +530,20 @@ static int launch_trace(rg_scene *sc, const TraceArgs &ta, bool use_grid, cudaSt
     return RG_OK;
 }
 
-static int render_batch(rg_scene *sc, uint32_t width, uint32_t height, uint32_t y0, uint32_t y1,
-                        const uint32_t *d_rows, uchar4 *d_out, cudaStream_t stream, rg_stats *st, bool use_grid, EventPool &events,
-                        EventPool &sync_events, std::vector<std::pair<cudaEvent_t, cudaEvent_t>> &trace_spans) {
-    const uint64_t npix64 = (uint64_t)(y1 - y0) * width;
-    if (npix64 == 0) return RG_OK;
-    if (npix64 > 0x7FFFFFFFull) { set_error("batch of %llu pixels is too large", (unsigned long long)npix64); return RG_E_NOMEM; }
-    const uint32_t npix = (uint32_t)npix64;
-    const DScene &ds = sc->ds;
-    const uint32_t L = ds.n_lights;
-    WavefrontScratch &wf = sc->wf;
-    DCounters *dc = sc->d_counters, *hc = sc->h_counters;
-    int rc;
-    auto blocks = [](uint64_t n) { return (unsigned)((n + 255) / 256); };
-
-    // Two-stream schedule.  The shadow side of level d (any-hit trace + k_diffuse) depends only on
-    // k_shade(d); the path side of level d+1 (nearest trace + k_shade) depends only on k_shade(d)
-    // too.  With the grid tracer both are latency-bound persistent kernels with long tails, so the
-    // shadow side runs on an auxiliary stream, concurrently with the next level's path side; its
-    // buffers exist twice (level parity) and k_shade(d+2) waits for the shadow side of level d.
-    // The brute-force tracer fills the chip on its own and keeps the single-stream order (its
-    // per-kernel times are also what the roofline figure is computed from).
-    const bool overlap = L > 0 && (sc->overlap == 2 || (sc->overlap == 0 && use_grid));
-    cudaStream_t aux = stream;
-    if (overlap) {
-        if (!wf.aux) RG_CUDA(cudaStreamCreateWithFlags(&wf.aux, cudaStreamNonBlocking));
-        aux = wf.aux;
-    }
-    cudaEvent_t shadow_done[2] = {nullptr, nullptr};   // last shadow-side work that used the parity's buffers
-    // Run-ahead.  The host needs each level's counters (children, lit hits) to size the next
-    // launches, but the persistent grid tracer does not need a launch size: the nearest-hit trace
-    // of level d+1 is enqueued right behind k_shade(d) and reads its ray count from the device
-    // counter k_shade(d) leaves behind.  The counters travel to the host on a third stream, so the
-    // main stream never drains while the host catches up (one level of speculation; a level that
-    // turns out empty costs one no-op launch).
-    const bool run_ahead = overlap && use_grid && sc->verify_cull == 0;
-    if (run_ahead && !wf.rb) RG_CUDA(cudaStreamCreateWithFlags(&wf.rb, cudaStreamNonBlocking));
-    bool traced_ahead = false;   // the nearest trace of the current level is already in the stream
-
-    std::vector<uint32_t> level_n;
-    uint32_t n = npix, d = 0;
-    if ((rc = wf.ray[0].reserve((size_t)n * kRayBytes))) return rc;
-    RayQueue cur = make_queue(wf.ray[0], n);
-    const PixelOrder po = pixel_order(width, y1 - y0);
-    k_generate<<<blocks(n), 256, 0, stream>>>(ds, cur, width, height, y0, npix, d_rows, nullptr, po);
-    RG_CUDA(cudaGetLastError());
-    st->gpu_launches++;
-    st->rays_primary += npix;
-
-    while (n > 0) {
-        const bool can_spawn = d + 1 < ds.max_depth;
-        const uint64_t next_cap = can_spawn ? 2ull * n : 0ull;
-        const uint64_t shadow_cap = (uint64_t)n * L;
-        if (next_cap > 0x7FFFFFFFull || shadow_cap > 0x7FFFFFFFull) {
-            set_error("level %u would hold more than 2^31 rays; use a smaller batch", d);
-            return RG_E_NOMEM;
-        }
-        if (wf.nodes.size() <= d) wf.nodes.resize(d + 1);
-        if ((rc = wf.nodes[d].reserve((size_t)n * 32))) return rc;
-        if ((rc = wf.hit_t.reserve((size_t)n * 8))) return rc;
-        if ((rc = wf.hit_body.reserve((size_t)n * 4))) return rc;
-        DeviceBuffer &nextbuf = wf.ray[(d + 1) & 1];
-        if ((rc = nextbuf.reserve((size_t)std::max<uint64_t>(next_cap, 1) * kRayBytes))) return rc;
-        const int p = overlap ? (int)(d & 1u) : 0;   // parity of the shadow-side buffers
-        if ((rc = wf.sray[p].reserve((size_t)std::max<uint64_t>(shadow_cap, 1) * kRayBytes))) return rc;
-        if ((rc = wf.s_tmax[p].reserve((size_t)std::max<uint64_t>(shadow_cap, 1) * 8))) return rc;
-        if ((rc = wf.s_ab[p].reserve((size_t)std::max<uint64_t>(shadow_cap, 1) * 8))) return rc;
-        if ((rc = wf.s_lit[p].reserve((size_t)std::max<uint64_t>(shadow_cap, 1)))) return rc;
-        if ((rc = wf.lit_bc[p].reserve((size_t)n * 16))) return rc;
-        if ((rc = wf.lit_node[p].reserve((size_t)n * 4))) return rc;
-
-        // nearest hits of this level
-        TraceArgs ta{};
-        ta.q = cur;
-        ta.n = n;
-        ta.out_t = wf.hit_t.as<double>();
-        ta.out_body = wf.hit_body.as<uint32_t>();
-        ta.ctr = dc;
-        ta.verify = sc->verify_cull == 1;
-        if (!traced_ahead) {
-            cudaEvent_t e0 = events.get(), e1 = events.get();
-            RG_CUDA(cudaEventRecord(e0, stream));
-            if ((rc = launch_trace<false>(sc, ta, use_grid, stream))) return rc;
-            RG_CUDA(cudaEventRecord(e1, stream));
-            trace_spans.emplace_back(e0, e1);
-            st->gpu_launches++;
-            if (sc->verify_cull >= 2) k_verify_trace<false><<<(n + 127) / 128, 128, 0, stream>>>(ds, ta, (int)d);
-        }
-
-        LevelBuffers lb{};
-        lb.cur = cur;
-        lb.next = make_queue(nextbuf, (size_t)std::max<uint64_t>(next_cap, 1));
-        lb.shadow = make_queue(wf.sray[p], (size_t)std::max<uint64_t>(shadow_cap, 1));
-        lb.hit_t = wf.hit_t.as<double>();
-        lb.hit_body = wf.hit_body.as<uint32_t>();
-        lb.node_a = wf.nodes[d].as<float4>();
-        lb.node_b = reinterpret_cast<uint4 *>(wf.nodes[d].as<float4>() + n);
-        lb.s_tmax = wf.s_tmax[p].as<double>();
-        lb.s_ab = wf.s_ab[p].as<float2>();
-        lb.lit_bc = wf.lit_bc[p].as<float4>();
-        lb.lit_node = wf.lit_node[p].as<uint32_t>();
-        lb.n = n;
-        const bool light_major = shadow_light_major();
-        lb.shadow_sl = light_major ? n : 1u;
-        lb.shadow_sj = light_major ? 1u : L;
-        lb.can_spawn = can_spawn ? 1u : 0u;
-        lb.q_next = &dc->q_next;
-        lb.q_lit = &dc->q_lit;
-        lb.cap_next = 0xFFFFFFFFu;   // the next queue holds 2n rays: cannot overflow
-        lb.void_flag = &dc->overflow;
-        lb.level = d;
-        lb.hints = use_grid ? (sc->origin_hints ? 1u : 2u) : 0u;
-        RG_CUDA(cudaMemsetAsync(&dc->q_next, 0, 2 * sizeof(unsigned int), stream));
-        if (shadow_done[p]) RG_CUDA(cudaStreamWaitEvent(stream, shadow_done[p], 0));   // level d-2 still reads these buffers
-        k_shade<<<blocks(n), 256, 0, stream>>>(ds, lb, dc);
-        RG_CUDA(cudaGetLastError());
-        st->gpu_launches++;
-        traced_ahead = false;
-        cudaStream_t rbs = stream;
-        if (run_ahead) {
-            cudaEvent_t shaded = sync_events.get();
-            RG_CUDA(cudaEventRecord(shaded, stream));
-            if (can_spawn) {   // nearest trace of level d+1, sized on the device (q_next); hits for up to 2n rays
-                if ((rc = wf.hit_t.reserve((size_t)next_cap * 8))) return rc;
-                if ((rc = wf.hit_body.reserve((size_t)next_cap * 4))) return rc;
-                TraceArgs na{};
-                na.q = lb.next;
-                na.n = (uint32_t)next_cap;
-                na.n_dev = &dc->q_next;
-                na.out_t = wf.hit_t.as<double>();
-                na.out_body = wf.hit_body.as<uint32_t>();
-                na.ctr = dc;
-                cudaEvent_t e0 = events.get(), e1 = events.get();
-                RG_CUDA(cudaEventRecord(e0, stream));
-                if ((rc = launch_trace<false>(sc, na, use_grid, stream))) return rc;
-                RG_CUDA(cudaEventRecord(e1, stream));
-                trace_spans.emplace_back(e0, e1);
-                st->gpu_launches++;
-                traced_ahead = true;
-            }
-            rbs = wf.rb;
-            RG_CUDA(cudaStreamWaitEvent(rbs, shaded, 0));
-        }
-        RG_CUDA(cudaMemcpyAsync(&hc->q_next, &dc->q_next, 2 * sizeof(unsigned int), cudaMemcpyDeviceToHost, rbs));
-        RG_CUDA(cudaStreamSynchronize(rbs));
-        const uint32_t n_next = hc->q_next, n_lit = hc->q_lit;
-
-        // shadow side: on `aux` (== stream without overlap).  The host has just synchronised the
-        // main stream, so everything k_shade(d) wrote is visible to work submitted to aux now.
-        if (n_lit && L) {
-            TraceArgs sa{};
-            sa.q = lb.shadow;
-            sa.tmax = lb.s_tmax;
-            sa.n = n_lit * L;
-            sa.seg_len = light_major ? n_lit : 0u;
-            sa.seg_stride = n;
-            sa.out_lit = wf.s_lit[p].as<uint8_t>();
-            sa.ctr = dc;
-            sa.verify = sc->verify_cull == 1;
-            cudaEvent_t s0 = events.get(), s1 = events.get();
-            RG_CUDA(cudaEventRecord(s0, aux));
-            if ((rc = launch_trace<true>(sc, sa, use_grid, aux))) return rc;
-            RG_CUDA(cudaEventRecord(s1, aux));
-            trace_spans.emplace_back(s0, s1);
-            if (sc->verify_cull >= 2) k_verify_trace<true><<<(sa.n + 127) / 128, 128, 0, aux>>>(ds, sa, (int)d);
-            st->gpu_launches++;
-            st->rays_shadow += (uint64_t)n_lit * L;
-        }
-        if (n_lit) {
-            k_diffuse<<<blocks(n_lit), 256, 0, aux>>>(ds, lb.lit_bc, lb.lit_node, lb.s_ab, wf.s_lit[p].as<uint8_t>(),
-                                                      lb.node_a, n_lit, lb.shadow_sl, lb.shadow_sj, nullptr, nullptr);
-            RG_CUDA(cudaGetLastError());
-            st->gpu_launches++;
-            if (overlap) {
-                shadow_done[p] = sync_events.get();
-                RG_CUDA(cudaEventRecord(shadow_done[p], aux));
-            }
-        }
-        level_n.push_back(n);
-        cur = lb.next;
-        n = n_next;
-        ++d;
-    }
-    // bottom-up colour combination (after the shadow side has delivered every diffuse term), then
-    // quantise level 0
-    for (int q = 0; q < 2; ++q)
-        if (shadow_done[q]) RG_CUDA(cudaStreamWaitEvent(stream, shadow_done[q], 0));
-    for (int lvl = (int)level_n.size() - 1; lvl >= 0; --lvl) {
-        const uint32_t ln = level_n[lvl];
-        float4 *a = wf.nodes[lvl].as<float4>();
-        const uint4 *b = reinterpret_cast<const uint4 *>(a + ln);
-        const float4 *child = (size_t)lvl + 1 < level_n.size() ? wf.nodes[lvl + 1].as<float4>() : nullptr;
-        k_combine<<<blocks(ln), 256, 0, stream>>>(ds, a, b, child, ln, nullptr, nullptr);
-        RG_CUDA(cudaGetLastError());
-        st->gpu_launches++;
-    }
-    if (sc->out_f32)
-        k_export_f32<<<blocks(npix), 256, 0, stream>>>(wf.nodes[0].as<float4>(), reinterpret_cast<float *>(d_out), npix, po);
-    else if (sc->scatter_out)   // d_out is the base of the whole frame; this batch covers row-list entries [y0, y1)
-        k_quantise_scatter<<<blocks(((uint64_t)npix + 3) / 4), 256, 0, stream>>>(wf.nodes[0].as<float4>(), d_out, npix, d_rows, y0, po);
-    else
-        k_quantise<<<blocks(((uint64_t)npix + 3) / 4), 256, 0, stream>>>(wf.nodes[0].as<float4>(), d_out, npix, po);
-    RG_CUDA(cudaGetLastError());
-    st->gpu_launches++;
-    st->batches++;
-    if (level_n.size() > st->max_level + 1) st->max_level = (uint32_t)level_n.size() - 1;
-    return RG_OK;
-}
-
 // ---- the host-free level loop ------------------------------------------------------------------
 // render_image is one call with no per-depth host involvement (rendering.rs:24-38).  Here the
 // whole batch — every level's trace, shade, shadow trace, diffuse, then combine and quantise —
 // is ENQUEUED without a single host synchronisation: each launch reads its level's size from
 // DCounters::lvl[] (written by the level above) and is sized for the queue's CAPACITY; persistent
 // / grid-stride kernels make surplus blocks free.  Queue capacities are fixed up front:
-//     cap[0] = pixels,   cap[d] = min(2 cap[d-1], kLevelGrowth * pixels)
-// (a hit spawns <= 2 rays, so 2 cap[d-1] is exact; real scenes stay far below kLevelGrowth x).  A level
-// that would outgrow its queue sets DCounters::overflow, every later launch of the frame then does
-// nothing, and the host repeats the render with the exact, host-sized loop above (sticky per scene).
-// The launch sequence depends only on (pixels, depth, lights, buffers), so it can be captured
-// once into a CUDA graph and replayed per frame (RG_OPT_GRAPH).
-constexpr uint32_t kLevelGrowth = 2;
-
+//     cap[0] = pixels,   cap[d] = min(2 cap[d-1], rg_scene::level_growth * pixels)
+// (a hit spawns <= 2 rays, so 2 cap[d-1] is exact; real scenes stay far below the initial growth of 2x).
+// A level that would outgrow its queue sets DCounters::overflow, every later launch of the frame then
+// does nothing, and the host doubles the scene's level_growth and repeats the render (sticky per scene).
+// Once level_growth >= 2^(levels-1) the clamp is inactive and no level can overflow, so a scene repeats
+// at most levels - 2 frames over its lifetime.
+// The launch sequence depends only on (pixels, depth, lights, capacities, buffers), so it can be
+// captured once into a CUDA graph and replayed per frame (RG_OPT_GRAPH).
 struct DevPlan {
     uint32_t levels = 0;                    // levels 0 .. levels-1 are enqueued
     uint32_t cap[RG_MAX_DEPTH + 2] = {0};
@@ -780,7 +561,7 @@ static int plan_batch_dev(rg_scene *sc, uint32_t npix, DevPlan &plan, bool use_g
     if (sc->depth_hint && sc->depth_hint < plan.levels) plan.levels = sc->depth_hint;
     uint64_t cap_max[2] = {0, 0}, cap_all = 0;
     for (uint32_t d = 0; d < plan.levels; ++d) {
-        const uint64_t c = d == 0 ? npix : std::min<uint64_t>(2ull * plan.cap[d - 1], (uint64_t)kLevelGrowth * npix);
+        const uint64_t c = d == 0 ? npix : std::min<uint64_t>(2ull * plan.cap[d - 1], (uint64_t)sc->level_growth * npix);
         if (c > 0x7FFFFFFFull || c * std::max<uint32_t>(L, 1u) > 0x7FFFFFFFull) {
             set_error("level %u could hold more than 2^31 rays; use a smaller batch", d);
             return RG_E_NOMEM;
@@ -822,9 +603,15 @@ static int enqueue_batch_dev(rg_scene *sc, const DevPlan &plan, uint32_t width, 
     // enough blocks to fill the chip several times over; grid-stride loops do the rest
     const unsigned max_blocks = (unsigned)sc->sm_count * 16u;
     auto blocks = [&](uint64_t n) { return (unsigned)std::max<uint64_t>(1, std::min<uint64_t>((n + 255) / 256, max_blocks)); };
+    // Two-stream schedule.  The shadow side of level d (any-hit trace + k_diffuse) depends only on
+    // k_shade(d); the path side of level d+1 (nearest trace + k_shade) depends only on k_shade(d)
+    // too.  With the grid tracer both are latency-bound persistent kernels with long tails, so the
+    // shadow side runs on an auxiliary stream, concurrently with the next level's path side; its
+    // buffers exist twice (level parity) and k_shade(d+2) waits for the shadow side of level d.
+    // The brute-force tracer fills the chip on its own and keeps the single-stream order (its
+    // per-kernel times are also what the roofline figure is computed from).  (A second auxiliary stream
+    // for the odd levels, so that two shadow sides overlap as well, was measured: no gain at any batch size.)
     const bool overlap = L > 0 && (sc->overlap == 2 || (sc->overlap == 0 && use_grid));
-    // the shadow side of a level runs beside the path side of the next levels, on one auxiliary stream (a second
-    // one for the odd levels, so that two shadow sides overlap as well, was measured: no gain at any batch size)
     cudaStream_t aux = overlap ? wf.aux : stream;
     cudaEvent_t shadow_done[2] = {nullptr, nullptr};
 
@@ -856,6 +643,7 @@ static int enqueue_batch_dev(rg_scene *sc, const DevPlan &plan, uint32_t width, 
         if ((rc = launch_trace<false>(sc, ta, use_grid, stream))) return rc;
         if (events) { RG_CUDA(cudaEventRecord(e1, stream)); trace_spans->emplace_back(e0, e1); }
         st->gpu_launches++;
+        if (sc->verify_cull >= 2) k_verify_trace<false><<<(cap + 127) / 128, 128, 0, stream>>>(ds, ta, (int)d);
 
         LevelBuffers lb{};
         lb.cur = cur;
@@ -869,7 +657,7 @@ static int enqueue_batch_dev(rg_scene *sc, const DevPlan &plan, uint32_t width, 
         lb.s_ab = wf.s_ab[p].as<float2>();
         lb.lit_bc = wf.lit_bc[p].as<float4>();
         lb.lit_node = wf.lit_node[p].as<uint32_t>();
-        lb.n = cap;
+        lb.cap = cap;
         lb.n_dev = &dc->lvl[d].n;
         const bool light_major = shadow_light_major();
         lb.shadow_sl = light_major ? cap : 1u;   // one segment of `cap` slots per light, or the L rays of a hit adjacent
@@ -881,7 +669,6 @@ static int enqueue_batch_dev(rg_scene *sc, const DevPlan &plan, uint32_t width, 
         lb.void_flag = &dc->overflow;
         lb.level = d;
         lb.hints = use_grid ? (sc->origin_hints ? 1u : 2u) : 0u;
-        lb.count_on_device = 1u;
         lb.last_enqueued = (d + 1 == plan.levels && can_spawn) ? 1u : 0u;
         if (shadow_done[p]) RG_CUDA(cudaStreamWaitEvent(stream, shadow_done[p], 0));   // level d-2 still reads these buffers
         k_shade<<<blocks(cap), 256, 0, stream>>>(ds, lb, dc);
@@ -911,6 +698,7 @@ static int enqueue_batch_dev(rg_scene *sc, const DevPlan &plan, uint32_t width, 
             if ((rc = launch_trace<true>(sc, sa, use_grid, aux))) return rc;
             if (events) { RG_CUDA(cudaEventRecord(e1, aux)); trace_spans->emplace_back(e0, e1); }
             st->gpu_launches++;
+            if (sc->verify_cull >= 2) k_verify_trace<true><<<(sa.n + 127) / 128, 128, 0, aux>>>(ds, sa, (int)d);
         }
         k_diffuse<<<blocks(cap), 256, 0, aux>>>(ds, lb.lit_bc, lb.lit_node, lb.s_ab, wf.s_lit[p].as<uint8_t>(), lb.node_a, cap,
                                                 lb.shadow_sl, lb.shadow_sj, &dc->lvl[d].n_lit, &dc->overflow);
@@ -950,7 +738,8 @@ static std::vector<uint64_t> graph_key(const rg_scene *sc, const DevPlan &plan, 
     const WavefrontScratch &wf = sc->wf;
     std::vector<uint64_t> k = {width, height, y0, npix, (uint64_t)(uintptr_t)d_rows, (uint64_t)(uintptr_t)d_out,
                                (uint64_t)use_grid, (uint64_t)sc->scatter_out | ((uint64_t)sc->out_f32 << 1), (uint64_t)sc->ds.max_depth, (uint64_t)sc->overlap,
-                               (uint64_t)sc->verify_cull, (uint64_t)sc->trace_stats | ((uint64_t)sc->origin_hints << 1), (uint64_t)plan.levels};
+                               (uint64_t)sc->verify_cull, (uint64_t)sc->trace_stats | ((uint64_t)sc->origin_hints << 1), (uint64_t)plan.levels,
+                               (uint64_t)sc->level_growth};   // the capacities are baked into the captured launches
     auto add = [&](const DeviceBuffer &b) { k.push_back((uint64_t)(uintptr_t)b.ptr); };
     add(wf.ray[0]); add(wf.ray[1]); add(wf.hit_t); add(wf.hit_body);
     for (int p = 0; p < 2; ++p) { add(wf.sray[p]); add(wf.s_tmax[p]); add(wf.s_ab[p]); add(wf.s_lit[p]); add(wf.lit_bc[p]); add(wf.lit_node[p]); }
@@ -1038,9 +827,6 @@ int wavefront_render(rg_scene *sc, uint32_t width, uint32_t height, uint32_t y0,
     uint32_t batch_rows = (uint32_t)std::max<uint64_t>(1, std::min<uint64_t>(rows ? rows : 1, batch_pixels / width));
     const rg_stats st0 = *st;
     for (;;) {   // a ray tree larger than device memory restarts the render with half the rows per batch
-        // host-free loop (device-sized launches, no synchronisation inside the frame) unless switched off,
-        // or this scene once outgrew the default queue capacities, or a debug mode needs the host in the loop
-        const bool host_free = sc->host_free != 1 && !sc->host_free_overflowed && sc->verify_cull < 2;
         *st = st0;
         events.used = 0;
         sync_events.used = 0;
@@ -1048,7 +834,7 @@ int wavefront_render(rg_scene *sc, uint32_t width, uint32_t height, uint32_t y0,
         RG_CUDA(cudaMemsetAsync(sc->d_counters, 0, sizeof(DCounters), stream));
         RG_CUDA(cudaEventRecord(sc->ev[0], stream));
         int rc = RG_OK;
-        if (host_free && sc->ds.n_lights > 0 && (sc->overlap == 2 || (sc->overlap == 0 && use_grid))) {
+        if (sc->ds.n_lights > 0 && (sc->overlap == 2 || (sc->overlap == 0 && use_grid))) {
             if (!sc->wf.aux) RG_CUDA(cudaStreamCreateWithFlags(&sc->wf.aux, cudaStreamNonBlocking));
         }
         for (uint32_t y = y0; y < y1 && rc == RG_OK;) {
@@ -1056,27 +842,22 @@ int wavefront_render(rg_scene *sc, uint32_t width, uint32_t height, uint32_t y0,
             // RGBA8: 4 bytes per pixel; f32 colours (rg_render_rows_f32): 12
             uchar4 *out = sc->scatter_out ? d_out
                         : reinterpret_cast<uchar4 *>(reinterpret_cast<unsigned char *>(d_out) + (size_t)(y - y0) * width * (sc->out_f32 ? 12 : 4));
-            if (host_free) {
-                DevPlan plan;
-                const uint64_t npix64 = (uint64_t)(ye - y) * width;
-                if (npix64 > 0x7FFFFFFFull) { set_error("batch of %llu pixels is too large", (unsigned long long)npix64); rc = RG_E_NOMEM; }
-                else if (npix64 && (rc = plan_batch_dev(sc, (uint32_t)npix64, plan, use_grid)) == RG_OK) {
-                    bool done = false;
-                    if (sc->graph != 1 && sc->verify_cull == 0)
-                        rc = graph_batch(sc, plan, width, height, y, (uint32_t)npix64, d_rows, out, stream, st, use_grid, sync_events, &done);
-                    if (rc == RG_OK && !done)
-                        rc = enqueue_batch_dev(sc, plan, width, height, y, (uint32_t)npix64, d_rows, out, stream, st, use_grid, &events,
-                                               sync_events, &trace_spans);
-                }
-            } else {
-                rc = render_batch(sc, width, height, y, ye, d_rows, out, stream, st, use_grid, events, sync_events, trace_spans);
+            DevPlan plan;
+            const uint64_t npix64 = (uint64_t)(ye - y) * width;
+            if (npix64 > 0x7FFFFFFFull) { set_error("batch of %llu pixels is too large", (unsigned long long)npix64); rc = RG_E_NOMEM; }
+            else if (npix64 && (rc = plan_batch_dev(sc, (uint32_t)npix64, plan, use_grid)) == RG_OK) {
+                bool done = false;
+                if (sc->graph != 1 && sc->verify_cull == 0)
+                    rc = graph_batch(sc, plan, width, height, y, (uint32_t)npix64, d_rows, out, stream, st, use_grid, sync_events, &done);
+                if (rc == RG_OK && !done)
+                    rc = enqueue_batch_dev(sc, plan, width, height, y, (uint32_t)npix64, d_rows, out, stream, st, use_grid, &events,
+                                           sync_events, &trace_spans);
             }
             y = ye;
         }
         if (rc == RG_E_NOMEM && batch_rows > 1) {
             cudaStreamSynchronize(stream);
             if (sc->wf.aux) cudaStreamSynchronize(sc->wf.aux);
-            if (sc->wf.rb) cudaStreamSynchronize(sc->wf.rb);
             sc->wf.release();
             batch_rows = (batch_rows + 1) / 2;
             continue;
@@ -1085,11 +866,11 @@ int wavefront_render(rg_scene *sc, uint32_t width, uint32_t height, uint32_t y0,
         RG_CUDA(cudaEventRecord(sc->ev[1], stream));
         RG_CUDA(cudaMemcpyAsync(sc->h_counters, sc->d_counters, sizeof(DCounters), cudaMemcpyDeviceToHost, stream));
         RG_CUDA(cudaStreamSynchronize(stream));
-        if (host_free && sc->h_counters->overflow) {   // a level outgrew its queue: repeat with exact, host-sized queues
-            sc->host_free_overflowed = true;
+        if (sc->h_counters->overflow) {   // a level outgrew its queue: repeat with twice the growth per level
+            sc->level_growth *= 2;
             continue;
         }
-        if (host_free && sc->depth_hint && sc->depth_hint < std::max<uint32_t>(sc->ds.max_depth, 1u) &&
+        if (sc->depth_hint && sc->depth_hint < std::max<uint32_t>(sc->ds.max_depth, 1u) &&
             sc->h_counters->deeper) {   // the ray tree went deeper than the hint: repeat with every level
             sc->depth_hint = 0;
             continue;
@@ -1101,7 +882,7 @@ int wavefront_render(rg_scene *sc, uint32_t width, uint32_t height, uint32_t y0,
         const uint32_t used = std::max(st->max_level, sc->h_counters->max_level) + 1u;
         sc->depth_hint = std::max(sc->depth_hint, used);
     }
-    st->host_free = (sc->host_free != 1 && !sc->host_free_overflowed && sc->verify_cull < 2) ? 1u : 0u;
+    st->host_free = 1;
     float ms = 0.f;
     RG_CUDA(cudaEventElapsedTime(&ms, sc->ev[0], sc->ev[1]));
     st->ms_device = ms;
@@ -1112,7 +893,7 @@ int wavefront_render(rg_scene *sc, uint32_t width, uint32_t height, uint32_t y0,
     }
     st->ms_trace = tr;
     const DCounters &c = *sc->h_counters;
-    st->rays_shadow += c.rays[1];                        // host-free loop: counted on the device
+    st->rays_shadow += c.rays[1];                        // counted on the device
     if (c.max_level > st->max_level) st->max_level = c.max_level;
     st->grid_cells = c.grid_cells;
     st->grid_fetches = c.grid_fetches;

@@ -94,10 +94,11 @@ def test_small_batches_equal_one_batch():
     assert np.array_equal(tiled, full)
 
 
-def test_host_free_loop_graph_replay_and_host_sized_loop_agree(oracle):
-    """The level loop without host involvement (device-sized launches, RG_OPT_HOST_FREE), its CUDA-graph
-    replay (the third identical frame is a replay) and the host-sized loop produce the same bytes and ray
-    counts, on a grid scene and on a brute-force one, for a full frame, a row band and a scattered row list."""
+def test_host_free_loop_and_graph_replay_agree(oracle):
+    """The level loop without host involvement (device-sized launches) and its CUDA-graph replay (the second
+    identical frame is a replay) produce the oracle's bytes and ray counts, on a grid scene and on a brute-force
+    one, for a full frame, a row band and a scattered row list.  RG_OPT_HOST_FREE is obsolete: setting it
+    changes nothing."""
     import torch
 
     for name, data, w, h in (("C4-small", make_scene("C4", spheres=400, depth=8)[0], 256, 144),
@@ -124,15 +125,16 @@ def test_host_free_loop_graph_replay_and_host_sized_loop_agree(oracle):
             assert np.array_equal(img, ref)
             sc.set_option(rg._native.OPT_HOST_FREE, 1)
             img = sc.render_image(w, h)
-            _assert_same(img, ref, sc.last_stats, ost, f"{name}/host-sized")
-            assert sc.last_stats.host_free == 0
+            _assert_same(img, ref, sc.last_stats, ost, f"{name}/OPT_HOST_FREE=1")
+            assert sc.last_stats.host_free == 1
 
 
-def test_host_free_queue_overflow_falls_back_to_exact_queues(oracle):
-    """Device-sized queues hold at most 2x the pixels per level.  Nested glass spheres around the camera
+def test_host_free_queue_overflow_grows_the_queues(oracle):
+    """Device-sized queues start at 2x the pixels per level.  Nested glass spheres around the camera
     double the rays at every level (reflection stays inside, transmission meets the next shell), so
-    level 2 outgrows its queue: the device flags it, the library repeats the frame with host-sized
-    (exact) queues and stays there for this scene; the image must still be the oracle's."""
+    level 2 outgrows its queue: the device flags it, the library doubles the scene's queue growth and
+    repeats the frame until it fits, and keeps the larger queues for this scene.  The image must still be
+    the oracle's, every frame runs the host-free loop, and from the second frame on it is a graph replay."""
     from raingun_b200.scene import scene_from_dict
 
     glass = lambda r: {"Sphere": {"center": [0.0, 0.0, 0.0], "radius": r, "material": {
@@ -144,10 +146,13 @@ def test_host_free_queue_overflow_falls_back_to_exact_queues(oracle):
     ref, ost, _ = oracle.render(data, w, h)
     assert ost.rays_reflection + ost.rays_transmission > 6 * w * h   # the tree really doubles
     with rg.Scene(data) as sc:
-        for it in range(2):
+        sc.set_pipeline(rg.PIPELINE_WAVEFRONT)   # (the default would pick the megakernel for five bodies)
+        for it in range(3):
             img = sc.render_image(w, h)
             _assert_same(img, ref, sc.last_stats, ost, f"overflow frame {it}")
-            assert sc.last_stats.host_free == 0
+            assert sc.last_stats.host_free == 1
+            if it >= 1:
+                assert sc.last_stats.graph_replays == 1, (it, sc.last_stats.graph_replays)
 
 
 def test_multi_device_scene_renders_the_single_device_frame(oracle):
@@ -438,7 +443,7 @@ def test_origin_hints_change_no_pixel_and_spare_the_exact_tests():
             with rg.Scene(data) as sc:
                 sc.set_accel(rg.ACCEL_GRID)
                 sc.set_option(rg._native.OPT_ORIGIN_HINTS, hints)
-                sc.set_option(rg._native.OPT_VERIFY_CULL, 2)     # (host-sized loop + the verbatim re-trace)
+                sc.set_option(rg._native.OPT_VERIFY_CULL, 2)     # (eager host-free loop + the verbatim re-trace)
                 img = sc.render_image(w, h)
                 assert sc.last_stats.cull_unsound == 0, (name, hints)
                 sc.set_option(rg._native.OPT_VERIFY_CULL, 0)

@@ -1,4 +1,4 @@
-"""Host-free level loop vs host-sized loop vs CUDA-graph replay: device ms of the C4 frame, of 1/N of it
+"""Host-free level loop, eager vs CUDA-graph replay: device ms of the C4 frame, of 1/N of it
 (one interleaved row-list batch, the multi-GPU unit) and of the shipped examples at 800x600."""
 import sys, time
 sys.path.insert(0, ".")
@@ -9,7 +9,7 @@ from raingun_b200.synth import make_scene
 from raingun_b200.examples import example_scene
 from raingun_b200.dist import rows_of_tiles, n_tiles
 
-MODES = (("host-sized", 1, 1), ("host-free eager", 2, 1), ("host-free graph", 2, 2))
+MODES = (("host-free eager", 1), ("host-free graph", 2))
 
 
 def timed(fn, reps=6):
@@ -30,9 +30,8 @@ w, h = spec.width, spec.height
 out = torch.empty(h * w * 4, dtype=torch.uint8, device="cuda")
 nt = n_tiles(h, 8)
 stream = torch.cuda.current_stream().cuda_stream
-for label, hf, graph in MODES:
+for label, graph in MODES:
     sc = rg.Scene(sd)
-    sc.set_option(N.OPT_HOST_FREE, hf)
     sc.set_option(N.OPT_GRAPH, graph)
     for frac in (1, 2, 4, 8, 16, 32):
         rows = rows_of_tiles(list(range(0, nt, frac)), 8, h)
@@ -43,9 +42,8 @@ for label, hf, graph in MODES:
 
 for name in ("test1", "test2", "test3"):
     data = example_scene(name)
-    for label, hf, graph in MODES:
+    for label, graph in MODES:
         sc = rg.Scene(data)
-        sc.set_option(N.OPT_HOST_FREE, hf)
         sc.set_option(N.OPT_GRAPH, graph)
         for (ww, hh) in ((800, 600), (3840, 2160)):
             dev, wall, st = timed(lambda: sc.render_rows_device(ww, hh, 0, hh, out.data_ptr(), stream), reps=8)

@@ -1,4 +1,4 @@
-"""Per-launch times of one C4 frame (host-sized loop, events around every trace launch are not exported, so this
+"""Per-launch times of one C4 frame (events around every trace launch are not exported, so this
 uses the launch list under ncu instead) -- here: just total ms and trace-span sum for a few orderings."""
 import sys
 sys.path.insert(0, ".")
