@@ -184,28 +184,26 @@ class Scene:
         self.last_stats = st
         return st
 
+    def _render_rowlist(self, entry, width: int, height: int, rows, ptr: int, *stream) -> Stats:
+        rows = np.ascontiguousarray(rows, np.uint32)
+        st = Stats()
+        _native.check(entry(self._h, width, height, ctypes.c_void_p(rows.ctypes.data), int(rows.size), ctypes.c_void_p(ptr),
+                            *stream, ctypes.byref(st)))
+        self.last_stats = st
+        return st
+
     def render_rowlist_device(self, width: int, height: int, rows, device_ptr: int, cuda_stream: int = 0) -> Stats:
         """Row-tile sharding unit: renders the listed image rows, compacted in list order, into
         HBM at ``device_ptr`` (len(rows)*width*4 bytes)."""
-        rows = np.ascontiguousarray(rows, np.uint32)
-        st = Stats()
-        _native.check(_native.lib().rg_render_rowlist_device(
-            self._h, width, height, ctypes.c_void_p(rows.ctypes.data), int(rows.size), ctypes.c_void_p(device_ptr),
-            ctypes.c_void_p(cuda_stream), ctypes.byref(st)))
-        self.last_stats = st
-        return st
+        return self._render_rowlist(_native.lib().rg_render_rowlist_device, width, height, rows, device_ptr,
+                                    ctypes.c_void_p(cuda_stream))
 
     def render_rowlist_scatter(self, width: int, height: int, rows, frame_ptr: int, cuda_stream: int = 0) -> Stats:
         """As render_rowlist_device, but row ``rows[k]`` lands at its own place in the FULL frame at
         ``frame_ptr`` — which may be another GPU's memory (``SharedFrame``): the gather of a sharded
         frame fused into the last kernel."""
-        rows = np.ascontiguousarray(rows, np.uint32)
-        st = Stats()
-        _native.check(_native.lib().rg_render_rowlist_scatter(
-            self._h, width, height, ctypes.c_void_p(rows.ctypes.data), int(rows.size), ctypes.c_void_p(frame_ptr),
-            ctypes.c_void_p(cuda_stream), ctypes.byref(st)))
-        self.last_stats = st
-        return st
+        return self._render_rowlist(_native.lib().rg_render_rowlist_scatter, width, height, rows, frame_ptr,
+                                    ctypes.c_void_p(cuda_stream))
 
     def render_rows_f32(self, width: int, height: int, y0: int = 0, y1: Optional[int] = None) -> np.ndarray:
         """The unquantised f32 colours (``RenderedPixel.color``, rendering.rs:18-22): (rows, width, 3) float32."""
@@ -218,57 +216,35 @@ class Scene:
 
     def streaming_render_f32(self, width: int, height: int, on_rows: Callable[[int, np.ndarray], bool], band_rows: int = 0) -> bool:
         """``streaming_render`` with the colours as the reference's channel carries them: unquantised f32 RGB."""
-        failure = []
-
-        def trampoline(y0, rows, w, ptr, _user):
-            try:
-                arr = np.ctypeslib.as_array(ptr, shape=(rows, w, 3))
-                keep_going = on_rows(int(y0), arr)
-                return 0 if (keep_going is None or keep_going) else 1
-            except BaseException as e:  # never unwind through C
-                failure.append(e)
-                return 1
-
-        cb = _native.ROWS_F32_CB(trampoline)
-        st = Stats()
-        rc = _native.lib().rg_render_stream_f32(self._h, width, height, band_rows, cb, None, ctypes.byref(st))
-        self.last_stats = st
-        if failure:
-            raise failure[0]
-        if rc == _native.E_CANCELLED:
-            return False
-        _native.check(rc)
-        return True
+        return self._stream(_native.lib().rg_render_stream_f32, _native.ROWS_F32_CB, 3, width, height, on_rows, band_rows)
 
     def render_rowlist_host(self, width: int, height: int, rows, frame_ptr: int) -> Stats:
         """Renders the listed image rows and copies row ``rows[k]`` to ``frame_ptr + rows[k]*width*4`` in HOST
         memory (a full frame, ideally pinned / ``host_register``-ed; may be shared by one process per GPU)."""
-        rows = np.ascontiguousarray(rows, np.uint32)
-        st = Stats()
-        _native.check(_native.lib().rg_render_rowlist_host(
-            self._h, width, height, ctypes.c_void_p(rows.ctypes.data), int(rows.size), ctypes.c_void_p(frame_ptr), ctypes.byref(st)))
-        self.last_stats = st
-        return st
+        return self._render_rowlist(_native.lib().rg_render_rowlist_host, width, height, rows, frame_ptr)
 
     # -- Scene::streaming_render (scene.rs:45-51): finished row bands instead of single pixels
     def streaming_render(self, width: int, height: int, on_rows: Callable[[int, np.ndarray], bool],
                          band_rows: int = 0) -> bool:
         """Calls ``on_rows(y0, rgba_rows)`` per finished band; return False from it to cancel
         (the closed channel of rendering.rs:53-54,67).  Returns False if cancelled."""
+        return self._stream(_native.lib().rg_render_stream, _native.ROWS_CB, 4, width, height, on_rows, band_rows)
+
+    def _stream(self, entry, cb_type, channels: int, width: int, height: int, on_rows, band_rows: int) -> bool:
         failure = []
 
         def trampoline(y0, rows, w, ptr, _user):
             try:
-                arr = np.ctypeslib.as_array(ptr, shape=(rows, w, 4))
+                arr = np.ctypeslib.as_array(ptr, shape=(rows, w, channels))
                 keep_going = on_rows(int(y0), arr)
                 return 0 if (keep_going is None or keep_going) else 1
             except BaseException as e:  # never unwind through C
                 failure.append(e)
                 return 1
 
-        cb = _native.ROWS_CB(trampoline)
+        cb = cb_type(trampoline)
         st = Stats()
-        rc = _native.lib().rg_render_stream(self._h, width, height, band_rows, cb, None, ctypes.byref(st))
+        rc = entry(self._h, width, height, band_rows, cb, None, ctypes.byref(st))
         self.last_stats = st
         if failure:
             raise failure[0]

@@ -10,6 +10,7 @@
 #include <limits>
 #include <map>
 #include <mutex>
+#include <type_traits>
 
 #include "rg_cull.h"
 #include "rg_host.h"
@@ -87,39 +88,28 @@ void GraphCache::release() {
     seen.clear();
 }
 
-// Scratch arenas outlive a scene: destroying a scene parks its (possibly multi-GB) wavefront
-// buffers here and the next scene created on the same device adopts them, so a host that
-// re-uploads the scene every frame does not pay cudaMalloc/cudaFree for them each time.
-struct ParkedContext {
-    bool used = false;
-    WavefrontScratch wf;
-    DeviceBuffer frame, rowlist;
-    SceneArena arena;
-    DCounters *d_counters = nullptr, *h_counters = nullptr;
-    cudaStream_t stream = nullptr;
-    cudaEvent_t ev[4] = {nullptr, nullptr, nullptr, nullptr};
-    uint8_t *h_stage = nullptr;   // pinned staging of the scene upload
-    size_t h_stage_cap = 0;
-};
-static void free_parked(ParkedContext &p) {   // device of the context must be current
-    p.wf.release();
-    p.frame.release();
-    p.rowlist.release();
-    p.arena.release();
-    if (p.d_counters) cudaFree(p.d_counters);
-    if (p.h_counters) cudaFreeHost(p.h_counters);
-    if (p.h_stage) cudaFreeHost(p.h_stage);
-    for (auto &e : p.ev) if (e) cudaEventDestroy(e);
-    if (p.stream) cudaStreamDestroy(p.stream);
+void DeviceContext::release() {
+    wf.release();
+    frame.release();
+    rowlist.release();
+    arena.release();
+    if (d_counters) cudaFree(d_counters);
+    if (h_counters) cudaFreeHost(h_counters);
+    if (h_stage) cudaFreeHost(h_stage);
+    for (auto &e : ev) if (e) cudaEventDestroy(e);
+    if (stream) cudaStreamDestroy(stream);
+    *this = DeviceContext();
 }
+
+// Contexts of destroyed scenes, waiting for the next scene on their device.
 static std::mutex g_park_mutex;
 // a few per device: a multi-GPU host keeps several batches (scene handles) in flight per GPU
-static std::map<int, std::vector<ParkedContext>> g_parked;
+static std::map<int, std::vector<DeviceContext>> g_parked;
 constexpr size_t kMaxParkedPerDevice = 4;
 
 // frees every context parked on `device` (-1: on all devices); returns how many were freed
 static size_t trim_parked(int device) {
-    std::vector<std::pair<int, ParkedContext>> victims;
+    std::vector<std::pair<int, DeviceContext>> victims;
     {
         std::lock_guard<std::mutex> lock(g_park_mutex);
         for (auto &kv : g_parked) {
@@ -132,7 +122,7 @@ static size_t trim_parked(int device) {
     cudaGetDevice(&cur);
     for (auto &v : victims) {
         cudaSetDevice(v.first);
-        free_parked(v.second);
+        v.second.release();
     }
     cudaSetDevice(cur);
     return victims.size();
@@ -543,17 +533,6 @@ __global__ void __launch_bounds__(256) k_fma_peak(T *out, int iters, T a, T b, l
 using namespace rg;
 
 extern "C" {
-static int rg_render_rowlist_device_impl(rg_scene *sc, uint32_t w, uint32_t h, const uint32_t *rows, uint32_t n_rows, void *d_rgba_out,
-                                         void *cuda_stream, rg_stats *stats);
-}
-namespace rg {
-int rowlist_device_unguarded(rg_scene *sc, uint32_t w, uint32_t h, const uint32_t *rows, uint32_t n_rows, void *d_rgba_out,
-                             void *cuda_stream, rg_stats *stats) {
-    return rg_render_rowlist_device_impl(sc, w, h, rows, n_rows, d_rgba_out, cuda_stream, stats);
-}
-}  // namespace rg
-
-extern "C" {
 
 const char *rg_last_error(void) { return g_last_error.c_str(); }
 
@@ -569,41 +548,17 @@ void rg_scene_destroy(rg_scene *sc) {
     cudaSetDevice(sc->device);
     sc->graphs.release();
     for (auto o : sc->tex_objs) cudaDestroyTextureObject(o);
+    if (sc->h_frame) cudaFreeHost(sc->h_frame);
     {
         std::lock_guard<std::mutex> lock(g_park_mutex);
-        std::vector<ParkedContext> &parked = g_parked[sc->device];
-        // park the device-side context for the next scene on this device — only a COMPLETE one (a create() that
-        // failed half-way must not hand its holes to the next scene)
-        const bool complete = sc->stream && sc->d_counters && sc->h_counters && sc->ev[0] && sc->ev[1] && sc->ev[2] && sc->ev[3];
-        if (parked.size() < kMaxParkedPerDevice && complete) {
-            if (sc->h_frame) cudaFreeHost(sc->h_frame);
-            parked.emplace_back();
-            ParkedContext &slot = parked.back();
-            slot.used = true;
-            slot.wf = std::move(sc->wf);
-            slot.frame = sc->frame;
-            slot.rowlist = sc->rowlist;
-            slot.arena = std::move(sc->arena);
-            slot.d_counters = sc->d_counters;
-            slot.h_counters = sc->h_counters;
-            slot.stream = sc->stream;
-            slot.h_stage = sc->h_stage;
-            slot.h_stage_cap = sc->h_stage_cap;
-            for (int k = 0; k < 4; ++k) slot.ev[k] = sc->ev[k];
+        std::vector<DeviceContext> &parked = g_parked[sc->device];
+        if (parked.size() < kMaxParkedPerDevice && sc->complete()) {   // park it for the next scene on this device
+            parked.push_back(std::move(static_cast<DeviceContext &>(*sc)));
             delete sc;
             return;
         }
     }
-    sc->arena.release();
-    sc->wf.release();
-    sc->frame.release();
-    sc->rowlist.release();
-    if (sc->h_frame) cudaFreeHost(sc->h_frame);
-    if (sc->h_stage) cudaFreeHost(sc->h_stage);
-    if (sc->d_counters) cudaFree(sc->d_counters);
-    if (sc->h_counters) cudaFreeHost(sc->h_counters);
-    for (auto &e : sc->ev) if (e) cudaEventDestroy(e);
-    if (sc->stream) cudaStreamDestroy(sc->stream);
+    sc->release();
     delete sc;
 }
 
@@ -670,19 +625,9 @@ int rg_scene_create(const rg_scene_desc *desc, int32_t device, rg_scene **out) {
         std::lock_guard<std::mutex> lock(g_park_mutex);
         auto it = g_parked.find(device);
         if (it != g_parked.end() && !it->second.empty()) {   // adopt a context an earlier scene left behind
-            ParkedContext slot = std::move(it->second.back());
+            static_cast<DeviceContext &>(*sc) = std::move(it->second.back());
             it->second.pop_back();
-            sc->wf = std::move(slot.wf);
-            sc->frame = slot.frame;
-            sc->rowlist = slot.rowlist;
-            sc->arena = std::move(slot.arena);
             sc->arena.reset();
-            sc->d_counters = slot.d_counters;
-            sc->h_counters = slot.h_counters;
-            sc->stream = slot.stream;
-            sc->h_stage = slot.h_stage;
-            sc->h_stage_cap = slot.h_stage_cap;
-            for (int k = 0; k < 4; ++k) sc->ev[k] = slot.ev[k];
         }
     }
     if (!sc->stream) {
@@ -749,6 +694,10 @@ int rg_scene_set_option(rg_scene *sc, int32_t key, int64_t value) {
     return RG_E_INVALID;
 }
 
+}  // extern "C"
+
+namespace rg {
+
 static int check_dims(rg_scene *sc, uint32_t w, uint32_t h, uint32_t y0, uint32_t y1) {
     if (!sc) { set_error("scene is NULL"); return RG_E_INVALID; }
     if (w == 0 || h == 0) { set_error("empty image %ux%u", w, h); return RG_E_INVALID; }
@@ -759,13 +708,13 @@ static int check_dims(rg_scene *sc, uint32_t w, uint32_t h, uint32_t y0, uint32_
 }
 
 static int mega_render(rg_scene *sc, uint32_t w, uint32_t h, uint32_t y0, uint32_t y1, const uint32_t *d_rows,
-                       uchar4 *d_out, cudaStream_t stream, rg_stats *st) {
+                       OutKind kind, uchar4 *d_out, cudaStream_t stream, rg_stats *st) {
     const uint64_t npix = (uint64_t)(y1 - y0) * w;
     RG_CUDA(cudaMemsetAsync(sc->d_counters, 0, sizeof(DCounters), stream));
     RG_CUDA(cudaEventRecord(sc->ev[0], stream));
     if (npix) {
         const unsigned blocks = (unsigned)((npix + 127) / 128);
-        float *f32 = sc->out_f32 ? reinterpret_cast<float *>(d_out) : nullptr;
+        float *f32 = kind == OutKind::F32 ? reinterpret_cast<float *>(d_out) : nullptr;
         if (sc->ds.max_depth <= 12) k_render_mega<12><<<blocks, 128, 0, stream>>>(sc->ds, w, h, y0, y1, d_rows, d_out, f32, sc->d_counters);
         else k_render_mega<RG_MAX_DEPTH><<<blocks, 128, 0, stream>>>(sc->ds, w, h, y0, y1, d_rows, d_out, f32, sc->d_counters);
         RG_CUDA(cudaGetLastError());
@@ -796,7 +745,7 @@ static int mega_render(rg_scene *sc, uint32_t w, uint32_t h, uint32_t y0, uint32
 
 // Common tail of the device-output entry points: rows [y0, y1), or entries [0, n) of a row list.
 static int render_device(rg_scene *sc, uint32_t w, uint32_t h, uint32_t y0, uint32_t y1, const uint32_t *d_rows,
-                         void *d_rgba_out, cudaStream_t stream, rg_stats *stats) {
+                         OutKind kind, void *d_out, cudaStream_t stream, rg_stats *stats) {
     auto t0 = std::chrono::steady_clock::now();
     rg_stats local;
     std::memset(&local, 0, sizeof(local));
@@ -806,9 +755,9 @@ static int render_device(rg_scene *sc, uint32_t w, uint32_t h, uint32_t y0, uint
     // the crossover lies near kMegaAutoBodies bodies (RG_MEGA_AUTO_BODIES for tuning runs)
     static const uint32_t mega_auto_bodies = [] { const char *e = getenv("RG_MEGA_AUTO_BODIES"); return e ? (uint32_t)atoi(e) : kMegaAutoBodies; }();
     const bool mega = sc->pipeline == RG_PIPELINE_MEGAKERNEL ||
-                      (sc->pipeline == RG_PIPELINE_AUTO && !sc->scatter_out && sc->n_bodies <= mega_auto_bodies && sc->verify_cull == 0);
-    if (mega) rc = mega_render(sc, w, h, y0, y1, d_rows, (uchar4 *)d_rgba_out, stream, &local);
-    else rc = wavefront_render(sc, w, h, y0, y1, d_rows, (uchar4 *)d_rgba_out, stream, &local);
+                      (sc->pipeline == RG_PIPELINE_AUTO && kind != OutKind::Rgba8Scatter && sc->n_bodies <= mega_auto_bodies && sc->verify_cull == 0);
+    if (mega) rc = mega_render(sc, w, h, y0, y1, d_rows, kind, (uchar4 *)d_out, stream, &local);
+    else rc = wavefront_render(sc, w, h, y0, y1, d_rows, kind, (uchar4 *)d_out, stream, &local);
     local.pipeline_used = mega ? RG_PIPELINE_MEGAKERNEL : RG_PIPELINE_WAVEFRONT;
     local.devices_used = 1;
     local.ms_wall = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count();
@@ -821,43 +770,119 @@ static int single_device_only(const rg_scene *sc, const char *what) {
     return RG_OK;
 }
 
-static int rg_render_rows_device_impl(rg_scene *sc, uint32_t w, uint32_t h, uint32_t y0, uint32_t y1, void *d_rgba_out,
-                          void *cuda_stream, rg_stats *stats) {
-    int rc = check_dims(sc, w, h, y0, y1);
-    if (rc) return rc;
-    if ((rc = single_device_only(sc, "rg_render_rows_device"))) return rc;
-    if (!d_rgba_out && y1 > y0) { set_error("output pointer is NULL"); return RG_E_INVALID; }
-    RG_CUDA(cudaSetDevice(sc->device));
-    return render_device(sc, w, h, y0, y1, nullptr, d_rgba_out, reinterpret_cast<cudaStream_t>(cuda_stream), stats);
-}
-
-static int rg_render_rowlist_device_impl(rg_scene *sc, uint32_t w, uint32_t h, const uint32_t *rows, uint32_t n_rows,
-                             void *d_rgba_out, void *cuda_stream, rg_stats *stats) {
+int render_rowlist_device(rg_scene *sc, uint32_t w, uint32_t h, const uint32_t *rows, uint32_t n_rows, OutKind kind, void *d_out,
+                          cudaStream_t stream, rg_stats *stats) {
     int rc = check_dims(sc, w, h, 0, h);
     if (rc) return rc;
     if ((rc = single_device_only(sc, "rg_render_rowlist_device"))) return rc;
-    if (n_rows && (!rows || !d_rgba_out)) { set_error("rows / output pointer is NULL"); return RG_E_INVALID; }
+    if (n_rows && (!rows || !d_out)) { set_error("rows / output pointer is NULL"); return RG_E_INVALID; }
     for (uint32_t k = 0; k < n_rows; ++k)
         if (rows[k] >= h) { set_error("rows[%u] = %u is outside the image (height %u)", k, rows[k], h); return RG_E_INVALID; }
     RG_CUDA(cudaSetDevice(sc->device));
-    cudaStream_t stream = reinterpret_cast<cudaStream_t>(cuda_stream);
     if (n_rows) {
         if ((rc = sc->rowlist.reserve((size_t)n_rows * sizeof(uint32_t)))) return rc;
         RG_CUDA(cudaMemcpyAsync(sc->rowlist.ptr, rows, (size_t)n_rows * sizeof(uint32_t), cudaMemcpyHostToDevice, stream));
         RG_CUDA(cudaStreamSynchronize(stream));   // `rows` may be pageable and reused by the caller
     }
-    return render_device(sc, w, h, 0, n_rows, sc->rowlist.as<uint32_t>(), d_rgba_out, stream, stats);
+    return render_device(sc, w, h, 0, n_rows, sc->rowlist.as<uint32_t>(), kind, d_out, stream, stats);
 }
 
-static int rg_render_rowlist_scatter_impl(rg_scene *sc, uint32_t w, uint32_t h, const uint32_t *rows, uint32_t n_rows,
-                              void *d_frame, void *cuda_stream, rg_stats *stats) {
-    if (sc && sc->pipeline == RG_PIPELINE_MEGAKERNEL) { set_error("rg_render_rowlist_scatter needs the wavefront pipeline"); return RG_E_INVALID; }
-    if (!sc) { set_error("scene is NULL"); return RG_E_INVALID; }
-    sc->scatter_out = true;
-    const int rc = rg_render_rowlist_device_impl(sc, w, h, rows, n_rows, d_frame, cuda_stream, stats);
-    sc->scatter_out = false;
+void merge_stats(rg_stats &total, const rg_stats &part, bool concurrent) {
+    total.rays_primary += part.rays_primary;
+    total.rays_shadow += part.rays_shadow;
+    total.rays_reflection += part.rays_reflection;
+    total.rays_transmission += part.rays_transmission;
+    total.body_tests += part.body_tests;
+    total.exact_tests += part.exact_tests;
+    total.cull_unsound += part.cull_unsound;
+    total.err_nan_distance += part.err_nan_distance;
+    total.err_transmission_none += part.err_transmission_none;
+    total.err_aabb_normal += part.err_aabb_normal;
+    total.ms_device = concurrent ? std::max(total.ms_device, part.ms_device) : total.ms_device + part.ms_device;
+    total.ms_trace = concurrent ? std::max(total.ms_trace, part.ms_trace) : total.ms_trace + part.ms_trace;
+    total.gpu_launches += part.gpu_launches;
+    total.batches += part.batches;
+    total.graph_replays += part.graph_replays;
+    total.grid_cells += part.grid_cells;
+    total.grid_fetches += part.grid_fetches;
+    total.grid_culls += part.grid_culls;
+    total.grid_refills += part.grid_refills;
+    total.grid_lane_steps += part.grid_lane_steps;
+    total.grid_lane_slots += part.grid_lane_slots;
+    total.max_level = std::max(total.max_level, part.max_level);
+    if (part.batches) {
+        total.accel_used = part.accel_used;
+        total.host_free = part.host_free;
+        total.pipeline_used = part.pipeline_used;
+    }
+}
+
+// Rows [y0, y1) into host memory (kind Rgba8 or F32), through the staging buffer sc->frame.  ms_wall includes the
+// copy to the host.
+static int render_rows_host(rg_scene *sc, uint32_t w, uint32_t h, uint32_t y0, uint32_t y1, OutKind kind, void *host, rg_stats *stats) {
+    int rc = check_dims(sc, w, h, y0, y1);
+    if (rc) return rc;
+    if (kind == OutKind::F32 && (rc = single_device_only(sc, "rg_render_rows_f32"))) return rc;
+    if (!host && y1 > y0) { set_error("output pointer is NULL"); return RG_E_INVALID; }
+    if (sc->multi) return multi_render_rows(sc, w, h, y0, y1, static_cast<uint8_t *>(host), stats);   // every GPU of the scene takes its row tiles
+    auto t0 = std::chrono::steady_clock::now();
+    RG_CUDA(cudaSetDevice(sc->device));
+    const size_t bytes = (size_t)(y1 - y0) * w * bytes_per_pixel(kind);
+    if ((rc = sc->frame.reserve(bytes ? bytes : 4))) return rc;
+    rg_stats local;
+    if ((rc = render_device(sc, w, h, y0, y1, nullptr, kind, sc->frame.ptr, sc->stream, &local))) return rc;
+    if (bytes) {
+        RG_CUDA(cudaMemcpyAsync(host, sc->frame.ptr, bytes, cudaMemcpyDeviceToHost, sc->stream));
+        RG_CUDA(cudaStreamSynchronize(sc->stream));
+    }
+    local.ms_wall = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count();
+    if (stats) *stats = local;
+    return RG_OK;
+}
+
+// The whole image in bands of `band_rows` rows (0: about a megapixel each), each handed to `cb` once it is in host
+// memory.  Pixel is uint8_t (RGBA8, rg_render_stream) or float (f32 RGB, rg_render_stream_f32).
+template <typename Pixel>
+static int render_bands(rg_scene *sc, uint32_t w, uint32_t h, uint32_t band_rows,
+                        int (*cb)(uint32_t, uint32_t, uint32_t, const Pixel *, void *), void *user, rg_stats *stats) {
+    constexpr OutKind kind = std::is_same<Pixel, float>::value ? OutKind::F32 : OutKind::Rgba8;
+    int rc = check_dims(sc, w, h, 0, h);
+    if (rc) return rc;
+    if (!cb) { set_error("callback is NULL"); return RG_E_INVALID; }
+    if (kind == OutKind::F32 && (rc = single_device_only(sc, "rg_render_stream_f32"))) return rc;
+    auto t0 = std::chrono::steady_clock::now();
+    RG_CUDA(cudaSetDevice(sc->device));
+    if (band_rows == 0) band_rows = (uint32_t)std::max<uint64_t>(1, (1ull << 20) / w);
+    if (band_rows > h) band_rows = h;
+    const size_t band_bytes = (size_t)band_rows * w * bytes_per_pixel(kind);
+    if (sc->h_frame_cap < band_bytes) {
+        if (sc->h_frame) cudaFreeHost(sc->h_frame);
+        sc->h_frame = nullptr;
+        sc->h_frame_cap = 0;
+        RG_CUDA(cudaMallocHost(&sc->h_frame, band_bytes));
+        sc->h_frame_cap = band_bytes;
+    }
+    rg_stats total;
+    std::memset(&total, 0, sizeof(total));
+    for (uint32_t y0 = 0; y0 < h; y0 += band_rows) {
+        const uint32_t y1 = y0 + band_rows < h ? y0 + band_rows : h;
+        rg_stats s;
+        if ((rc = render_rows_host(sc, w, h, y0, y1, kind, sc->h_frame, &s))) return rc;
+        merge_stats(total, s, false);
+        if (cb(y0, y1 - y0, w, reinterpret_cast<const Pixel *>(sc->h_frame), user) != 0) {   // closed channel: rendering.rs:53-54,67
+            set_error("render cancelled by the row callback at row %u", y0);
+            rc = RG_E_CANCELLED;
+            break;
+        }
+    }
+    total.ms_wall = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count();
+    if (stats) *stats = total;
     return rc;
 }
+
+}  // namespace rg
+
+extern "C" {
 
 // ---- frames another process' GPU can write into (CUDA IPC; peer stores travel over NVLink) ----
 static_assert(sizeof(cudaIpcMemHandle_t) == RG_IPC_HANDLE_BYTES, "RG_IPC_HANDLE_BYTES");
@@ -894,99 +919,6 @@ int rg_shared_frame_close(int32_t device, void *d_ptr, int32_t is_owner) {
     return RG_OK;
 }
 
-static int rg_render_rows_impl(rg_scene *sc, uint32_t w, uint32_t h, uint32_t y0, uint32_t y1, uint8_t *rgba_out, rg_stats *stats) {
-    int rc = check_dims(sc, w, h, y0, y1);
-    if (rc) return rc;
-    if (!rgba_out && y1 > y0) { set_error("output pointer is NULL"); return RG_E_INVALID; }
-    if (sc->multi) return multi_render_rows(sc, w, h, y0, y1, rgba_out, stats);   // every GPU of the scene takes its row tiles
-    auto t0 = std::chrono::steady_clock::now();
-    RG_CUDA(cudaSetDevice(sc->device));
-    const size_t bytes = (size_t)(y1 - y0) * w * 4;
-    if ((rc = sc->frame.reserve(bytes ? bytes : 4))) return rc;
-    rg_stats local;
-    std::memset(&local, 0, sizeof(local));
-    rc = rg_render_rows_device_impl(sc, w, h, y0, y1, sc->frame.ptr, sc->stream, &local);
-    if (rc) return rc;
-    if (bytes) {
-        RG_CUDA(cudaMemcpyAsync(rgba_out, sc->frame.ptr, bytes, cudaMemcpyDeviceToHost, sc->stream));
-        RG_CUDA(cudaStreamSynchronize(sc->stream));
-    }
-    local.ms_wall = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count();
-    if (stats) *stats = local;
-    return RG_OK;
-}
-
-static int rg_render_impl(rg_scene *sc, uint32_t w, uint32_t h, uint8_t *rgba_out, rg_stats *stats) {
-    return rg_render_rows_impl(sc, w, h, 0, h, rgba_out, stats);
-}
-
-static void accumulate(rg_stats *total, const rg_stats &s) {
-    total->rays_primary += s.rays_primary;
-    total->rays_shadow += s.rays_shadow;
-    total->rays_reflection += s.rays_reflection;
-    total->rays_transmission += s.rays_transmission;
-    total->body_tests += s.body_tests;
-    total->exact_tests += s.exact_tests;
-    total->cull_unsound += s.cull_unsound;
-    total->err_nan_distance += s.err_nan_distance;
-    total->err_transmission_none += s.err_transmission_none;
-    total->err_aabb_normal += s.err_aabb_normal;
-    total->ms_device += s.ms_device;
-    total->ms_trace += s.ms_trace;
-    total->gpu_launches += s.gpu_launches;
-    total->batches += s.batches;
-    total->graph_replays += s.graph_replays;
-    total->host_free = s.host_free;
-    total->pipeline_used = s.pipeline_used;
-    total->grid_cells += s.grid_cells;
-    total->grid_fetches += s.grid_fetches;
-    total->grid_culls += s.grid_culls;
-    total->grid_refills += s.grid_refills;
-    total->grid_lane_steps += s.grid_lane_steps;
-    total->grid_lane_slots += s.grid_lane_slots;
-    if (s.max_level > total->max_level) total->max_level = s.max_level;
-    total->accel_used = s.accel_used;
-}
-
-static int rg_render_stream_impl(rg_scene *sc, uint32_t w, uint32_t h, uint32_t band_rows, rg_rows_cb cb, void *user, rg_stats *stats) {
-    int rc = check_dims(sc, w, h, 0, h);
-    if (rc) return rc;
-    if (!cb) { set_error("callback is NULL"); return RG_E_INVALID; }
-    auto t0 = std::chrono::steady_clock::now();
-    RG_CUDA(cudaSetDevice(sc->device));
-    if (band_rows == 0) {
-        uint64_t rows = (1ull << 20) / w;   // ~1 Mpixel per band
-        band_rows = (uint32_t)(rows < 1 ? 1 : rows);
-    }
-    if (band_rows > h) band_rows = h;
-    const size_t band_bytes = (size_t)band_rows * w * 4;
-    if (sc->h_frame_cap < band_bytes) {
-        if (sc->h_frame) cudaFreeHost(sc->h_frame);
-        sc->h_frame = nullptr;
-        sc->h_frame_cap = 0;
-        RG_CUDA(cudaMallocHost(&sc->h_frame, band_bytes));
-        sc->h_frame_cap = band_bytes;
-    }
-    rg_stats total;
-    std::memset(&total, 0, sizeof(total));
-    for (uint32_t y0 = 0; y0 < h; y0 += band_rows) {
-        uint32_t y1 = y0 + band_rows < h ? y0 + band_rows : h;
-        rg_stats s;
-        rc = rg_render_rows_impl(sc, w, h, y0, y1, sc->h_frame, &s);
-        if (rc) return rc;
-        accumulate(&total, s);
-        if (cb(y0, y1 - y0, w, sc->h_frame, user) != 0) {   // closed channel: rendering.rs:53-54,67
-            set_error("render cancelled by the row callback at row %u", y0);
-            total.ms_wall = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count();
-            if (stats) *stats = total;
-            return RG_E_CANCELLED;
-        }
-    }
-    total.ms_wall = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count();
-    if (stats) *stats = total;
-    return RG_OK;
-}
-
 // ---- public render entry points: one call at a time per handle ---------------------------------------
 // The reference's &Scene is Sync; a device-side scene is not (its scratch queues belong to the handle), so a
 // second render on a handle that is already rendering is refused with RG_E_BUSY instead of corrupting both.
@@ -1005,88 +937,43 @@ struct BusyGuard {
 
 int rg_render_rows_device(rg_scene *sc, uint32_t w, uint32_t h, uint32_t y0, uint32_t y1, void *d_rgba_out, void *cuda_stream, rg_stats *stats) {
     RG_ENTER(sc);
-    return rg_render_rows_device_impl(sc, w, h, y0, y1, d_rgba_out, cuda_stream, stats);
+    int rc = check_dims(sc, w, h, y0, y1);
+    if (rc) return rc;
+    if ((rc = single_device_only(sc, "rg_render_rows_device"))) return rc;
+    if (!d_rgba_out && y1 > y0) { set_error("output pointer is NULL"); return RG_E_INVALID; }
+    RG_CUDA(cudaSetDevice(sc->device));
+    return render_device(sc, w, h, y0, y1, nullptr, OutKind::Rgba8, d_rgba_out, reinterpret_cast<cudaStream_t>(cuda_stream), stats);
 }
 int rg_render_rowlist_device(rg_scene *sc, uint32_t w, uint32_t h, const uint32_t *rows, uint32_t n_rows, void *d_rgba_out, void *cuda_stream, rg_stats *stats) {
     RG_ENTER(sc);
-    return rg_render_rowlist_device_impl(sc, w, h, rows, n_rows, d_rgba_out, cuda_stream, stats);
+    return render_rowlist_device(sc, w, h, rows, n_rows, OutKind::Rgba8, d_rgba_out, reinterpret_cast<cudaStream_t>(cuda_stream), stats);
 }
 int rg_render_rowlist_scatter(rg_scene *sc, uint32_t w, uint32_t h, const uint32_t *rows, uint32_t n_rows, void *d_frame, void *cuda_stream, rg_stats *stats) {
     RG_ENTER(sc);
-    return rg_render_rowlist_scatter_impl(sc, w, h, rows, n_rows, d_frame, cuda_stream, stats);
+    if (sc && sc->pipeline == RG_PIPELINE_MEGAKERNEL) { set_error("rg_render_rowlist_scatter needs the wavefront pipeline"); return RG_E_INVALID; }
+    return render_rowlist_device(sc, w, h, rows, n_rows, OutKind::Rgba8Scatter, d_frame, reinterpret_cast<cudaStream_t>(cuda_stream), stats);
 }
 int rg_render_rows(rg_scene *sc, uint32_t w, uint32_t h, uint32_t y0, uint32_t y1, uint8_t *rgba_out, rg_stats *stats) {
     RG_ENTER(sc);
-    return rg_render_rows_impl(sc, w, h, y0, y1, rgba_out, stats);
+    return render_rows_host(sc, w, h, y0, y1, OutKind::Rgba8, rgba_out, stats);
 }
 int rg_render(rg_scene *sc, uint32_t w, uint32_t h, uint8_t *rgba_out, rg_stats *stats) {
     RG_ENTER(sc);
-    return rg_render_impl(sc, w, h, rgba_out, stats);
+    return render_rows_host(sc, w, h, 0, h, OutKind::Rgba8, rgba_out, stats);
 }
 int rg_render_stream(rg_scene *sc, uint32_t w, uint32_t h, uint32_t band_rows, rg_rows_cb cb, void *user, rg_stats *stats) {
     RG_ENTER(sc);
-    return rg_render_stream_impl(sc, w, h, band_rows, cb, user, stats);
+    return render_bands(sc, w, h, band_rows, cb, user, stats);
 }
 
 // ---- unquantised colours: RenderedPixel.color is an f32 Color (rendering.rs:18-22), quantised only by the consumer
-static int render_rows_f32_impl(rg_scene *sc, uint32_t w, uint32_t h, uint32_t y0, uint32_t y1, float *rgb_out, rg_stats *stats) {
-    int rc = check_dims(sc, w, h, y0, y1);
-    if (rc) return rc;
-    if ((rc = single_device_only(sc, "rg_render_rows_f32"))) return rc;
-    if (!rgb_out && y1 > y0) { set_error("output pointer is NULL"); return RG_E_INVALID; }
-    RG_CUDA(cudaSetDevice(sc->device));
-    const size_t bytes = (size_t)(y1 - y0) * w * 12;
-    if ((rc = sc->frame.reserve(bytes ? bytes : 4))) return rc;
-    sc->out_f32 = true;
-    rc = render_device(sc, w, h, y0, y1, nullptr, sc->frame.ptr, sc->stream, stats);
-    sc->out_f32 = false;
-    if (rc) return rc;
-    if (bytes) {
-        RG_CUDA(cudaMemcpyAsync(rgb_out, sc->frame.ptr, bytes, cudaMemcpyDeviceToHost, sc->stream));
-        RG_CUDA(cudaStreamSynchronize(sc->stream));
-    }
-    return RG_OK;
-}
-
 int rg_render_rows_f32(rg_scene *sc, uint32_t w, uint32_t h, uint32_t y0, uint32_t y1, float *rgb_out, rg_stats *stats) {
     RG_ENTER(sc);
-    return render_rows_f32_impl(sc, w, h, y0, y1, rgb_out, stats);
+    return render_rows_host(sc, w, h, y0, y1, OutKind::F32, rgb_out, stats);
 }
-
 int rg_render_stream_f32(rg_scene *sc, uint32_t w, uint32_t h, uint32_t band_rows, rg_rows_f32_cb cb, void *user, rg_stats *stats) {
     RG_ENTER(sc);
-    int rc = check_dims(sc, w, h, 0, h);
-    if (rc) return rc;
-    if (!cb) { set_error("callback is NULL"); return RG_E_INVALID; }
-    if ((rc = single_device_only(sc, "rg_render_stream_f32"))) return rc;
-    RG_CUDA(cudaSetDevice(sc->device));
-    if (band_rows == 0) band_rows = (uint32_t)std::max<uint64_t>(1, (1ull << 20) / w);
-    if (band_rows > h) band_rows = h;
-    const size_t band_bytes = (size_t)band_rows * w * 12;
-    if (sc->h_frame_cap < band_bytes) {
-        if (sc->h_frame) cudaFreeHost(sc->h_frame);
-        sc->h_frame = nullptr;
-        sc->h_frame_cap = 0;
-        RG_CUDA(cudaMallocHost(&sc->h_frame, band_bytes));
-        sc->h_frame_cap = band_bytes;
-    }
-    rg_stats total;
-    std::memset(&total, 0, sizeof(total));
-    for (uint32_t y0 = 0; y0 < h; y0 += band_rows) {
-        const uint32_t y1 = y0 + band_rows < h ? y0 + band_rows : h;
-        rg_stats s;
-        std::memset(&s, 0, sizeof s);
-        rc = render_rows_f32_impl(sc, w, h, y0, y1, reinterpret_cast<float *>(sc->h_frame), &s);
-        if (rc) return rc;
-        accumulate(&total, s);
-        if (cb(y0, y1 - y0, w, reinterpret_cast<const float *>(sc->h_frame), user) != 0) {   // closed channel: rendering.rs:53-54,67
-            set_error("render cancelled by the row callback at row %u", y0);
-            if (stats) *stats = total;
-            return RG_E_CANCELLED;
-        }
-    }
-    if (stats) *stats = total;
-    return RG_OK;
+    return render_bands(sc, w, h, band_rows, cb, user, stats);
 }
 
 int rg_render_rowlist_host(rg_scene *sc, uint32_t w, uint32_t h, const uint32_t *rows, uint32_t n_rows, uint8_t *frame, rg_stats *stats) {

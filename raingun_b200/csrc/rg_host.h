@@ -32,8 +32,8 @@ struct DeviceBuffer {
 };
 
 // Scene arrays are carved out of a few large blocks instead of one cudaMalloc each, and the
-// blocks survive the scene (see ParkedContext in rg_api.cu): re-uploading a scene every frame
-// then costs H2D copies only.
+// blocks survive the scene (see DeviceContext): re-uploading a scene every frame then costs
+// H2D copies only.
 struct SceneArena {
     std::vector<DeviceBuffer> blocks;
     size_t cur = 0, off = 0;
@@ -77,29 +77,46 @@ struct GraphCache {
     void release();
 };
 
+// The device-side state of a scene that does not depend on the scene's content.  Destroying a scene
+// parks it (rg_api.cu) and the next scene created on the same device adopts it, so a host that
+// re-uploads the scene every frame does not pay cudaMalloc / cudaFree for its (possibly multi-GB)
+// scratch each time.
+struct DeviceContext {
+    WavefrontScratch wf;
+    DeviceBuffer frame;                // staging of host-buffer renders
+    DeviceBuffer rowlist;              // device copy of a caller's row list
+    SceneArena arena;                  // scene arrays
+    DCounters *d_counters = nullptr;
+    DCounters *h_counters = nullptr;   // pinned
+    cudaStream_t stream = nullptr;     // library-owned stream for host-buffer renders
+    cudaEvent_t ev[4] = {nullptr, nullptr, nullptr, nullptr};
+    uint8_t *h_stage = nullptr;        // pinned staging of the scene upload (one H2D copy per scene)
+    size_t h_stage_cap = 0;
+    // every handle exists: a create() that failed half-way must not hand its holes to the next scene
+    bool complete() const { return stream && d_counters && h_counters && ev[0] && ev[1] && ev[2] && ev[3]; }
+    void release();                    // frees everything; the context's device must be current
+};
+
+// What a render call delivers: RGBA8 rows in order, RGBA8 rows stored at their place in a full frame
+// (rg_render_rowlist_scatter), or unquantised f32 RGB (rg_render_rows_f32).
+enum class OutKind { Rgba8, Rgba8Scatter, F32 };
+constexpr size_t bytes_per_pixel(OutKind k) { return k == OutKind::F32 ? 12 : 4; }
+
 }  // namespace rg
 
 namespace rg { struct MultiState; }
 
-struct rg_scene {
+// Parking moves the DeviceContext base out (its DeviceBuffers are plain pointer pairs, so they are
+// copied) and deletes the scene without releasing anything: rg_scene must not free in a destructor.
+struct rg_scene : rg::DeviceContext {
     int device = 0;
     rg::MultiState *multi = nullptr;       // set: this handle spans several GPUs (rg_multi.cu) and owns no device state itself
     std::atomic<bool> busy{false};         // a render call is running on this handle (second callers get RG_E_BUSY)
     rg::DScene ds{};                    // device pointers inside
     rg::GridProxies gp{};               // boxes and disks binned into the grid (rg_scene.cuh)
-    rg::SceneArena arena;               // scene arrays
     std::vector<cudaTextureObject_t> tex_objs;
-    rg::DCounters *d_counters = nullptr;
-    rg::DCounters *h_counters = nullptr;   // pinned
-    cudaStream_t stream = nullptr;         // library-owned stream for host-buffer renders
-    cudaEvent_t ev[4] = {nullptr, nullptr, nullptr, nullptr};
-    rg::DeviceBuffer frame;                // RGBA8 staging for host-buffer renders
-    rg::DeviceBuffer rowlist;              // device copy of a caller's row list
-    uint8_t *h_stage = nullptr;            // pinned staging of the scene upload (one H2D copy per scene)
-    size_t h_stage_cap = 0;
-    uint8_t *h_frame = nullptr;            // pinned staging
+    uint8_t *h_frame = nullptr;            // pinned staging of the streaming renders (not parked; a multi-GPU handle has one too)
     size_t h_frame_cap = 0;
-    rg::WavefrontScratch wf;
     rg::GraphCache graphs;                 // dies with the scene (kernel parameters hold scene pointers by value)
     // options
     int pipeline = RG_PIPELINE_AUTO;
@@ -114,8 +131,6 @@ struct rg_scene {
     uint32_t depth_hint = 0;               // levels the ray tree of this scene has been seen to use (0 = unknown)
     uint32_t level_growth = 2;             // wavefront queue of level d holds min(2^d, level_growth) x the batch's pixels;
                                            // doubled when a level outgrows its queue (the frame is then repeated)
-    bool out_f32 = false;                  // this call delivers unquantised f32 colours, 3 per pixel (rg_render_rows_f32)
-    bool scatter_out = false;              // this call stores rows at their place in a full frame (rg_render_rowlist_scatter)
     // derived
     uint32_t n_bodies = 0;
     int sm_count = 0;
@@ -125,10 +140,15 @@ namespace rg {
 // rg_wavefront.cu
 // rows [y0, y1) of the image, or — when d_rows is given — entries [y0, y1) of that row list
 int wavefront_render(rg_scene *sc, uint32_t width, uint32_t height, uint32_t y0, uint32_t y1,
-                     const uint32_t *d_rows, uchar4 *d_out, cudaStream_t stream, rg_stats *st);
-// rg_api.cu: rg_render_rowlist_device without the one-render-at-a-time guard (for callers that hold it)
-int rowlist_device_unguarded(rg_scene *sc, uint32_t w, uint32_t h, const uint32_t *rows, uint32_t n_rows, void *d_rgba_out,
-                             void *cuda_stream, rg_stats *stats);
+                     const uint32_t *d_rows, OutKind kind, uchar4 *d_out, cudaStream_t stream, rg_stats *st);
+// rg_api.cu
+// rg_render_rowlist_device (kind Rgba8) and rg_render_rowlist_scatter (Rgba8Scatter) without the one-render-at-a-time
+// guard (for callers that hold it)
+int render_rowlist_device(rg_scene *sc, uint32_t w, uint32_t h, const uint32_t *rows, uint32_t n_rows, OutKind kind, void *d_out,
+                          cudaStream_t stream, rg_stats *stats);
+// adds the stats of one part of a call to `total`; device times add up for parts that ran one after another and
+// overlap for `concurrent` ones (the slowest counts)
+void merge_stats(rg_stats &total, const rg_stats &part, bool concurrent);
 // rg_multi.cu
 int render_rowlist_to_host(rg_scene *sc, uint32_t w, uint32_t h, const uint32_t *rows, uint32_t n_rows, uint8_t *frame, rg_stats *st);
 int multi_create(const rg_scene_desc *desc, const int32_t *devices, uint32_t n_devices, rg_scene **out);

@@ -104,7 +104,7 @@ int render_rowlist_to_host(rg_scene *sc, uint32_t w, uint32_t h, const uint32_t 
     if (rc) return rc;
     rg_stats local;
     std::memset(&local, 0, sizeof local);
-    rc = rowlist_device_unguarded(sc, w, h, rows, n_rows, sc->frame.ptr, sc->stream, &local);
+    rc = render_rowlist_device(sc, w, h, rows, n_rows, OutKind::Rgba8, sc->frame.ptr, sc->stream, &local);
     if (rc) return rc;
     if ((rc = copy_rows_to_host(static_cast<const uint8_t *>(sc->frame.ptr), rows, n_rows, frame, row_bytes, sc->stream))) return rc;
     RG_CUDA(cudaStreamSynchronize(sc->stream));
@@ -121,16 +121,7 @@ static int render_tiles_to_host(rg_scene *sc, const MultiJob &j, const std::vect
     // j.out holds rows [y0, y1): address of image row 0 = out - y0 rows
     const int rc = render_rowlist_to_host(sc, j.w, j.h, rows.data(), (uint32_t)rows.size(), j.out - (size_t)j.y0 * j.w * 4, &local);
     if (rc) return rc;
-    // accumulate
-    st->rays_primary += local.rays_primary; st->rays_shadow += local.rays_shadow;
-    st->rays_reflection += local.rays_reflection; st->rays_transmission += local.rays_transmission;
-    st->body_tests += local.body_tests; st->exact_tests += local.exact_tests; st->cull_unsound += local.cull_unsound;
-    st->err_nan_distance += local.err_nan_distance; st->err_transmission_none += local.err_transmission_none;
-    st->err_aabb_normal += local.err_aabb_normal;
-    st->ms_device += local.ms_device; st->ms_trace += local.ms_trace;
-    st->gpu_launches += local.gpu_launches; st->batches += local.batches; st->graph_replays += local.graph_replays;
-    st->max_level = std::max(st->max_level, local.max_level);
-    st->accel_used = local.accel_used; st->host_free = local.host_free; st->pipeline_used = local.pipeline_used;
+    merge_stats(*st, local, false);
     return RG_OK;
 }
 
@@ -282,17 +273,7 @@ int multi_render_rows(rg_scene *sc, uint32_t w, uint32_t h, uint32_t y0, uint32_
             rc = ms->rc[k];
             set_error("device %d: %s", ms->dev[k]->device, ms->err[k].c_str());
         }
-        const rg_stats &s = ms->stats[k];
-        total.rays_primary += s.rays_primary; total.rays_shadow += s.rays_shadow;
-        total.rays_reflection += s.rays_reflection; total.rays_transmission += s.rays_transmission;
-        total.body_tests += s.body_tests; total.exact_tests += s.exact_tests; total.cull_unsound += s.cull_unsound;
-        total.err_nan_distance += s.err_nan_distance; total.err_transmission_none += s.err_transmission_none;
-        total.err_aabb_normal += s.err_aabb_normal;
-        total.ms_device = std::max(total.ms_device, s.ms_device);   // the devices run concurrently
-        total.ms_trace = std::max(total.ms_trace, s.ms_trace);
-        total.gpu_launches += s.gpu_launches; total.batches += s.batches; total.graph_replays += s.graph_replays;
-        total.max_level = std::max(total.max_level, s.max_level);
-        if (s.batches) { total.accel_used = s.accel_used; total.host_free = s.host_free; total.pipeline_used = s.pipeline_used; }
+        merge_stats(total, ms->stats[k], true);   // the devices run concurrently
         if (ms->claims[k]) total.devices_used++;
     }
     total.ms_wall = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count();

@@ -592,7 +592,7 @@ static int plan_batch_dev(rg_scene *sc, uint32_t npix, DevPlan &plan, bool use_g
 // Enqueues one batch.  No allocation, no synchronisation, no host read: legal inside a stream capture.
 // `timed` = record CUDA events around the trace launches (not possible while capturing).
 static int enqueue_batch_dev(rg_scene *sc, const DevPlan &plan, uint32_t width, uint32_t height, uint32_t y0, uint32_t npix,
-                             const uint32_t *d_rows, uchar4 *d_out, cudaStream_t stream, rg_stats *st, bool use_grid,
+                             const uint32_t *d_rows, OutKind kind, uchar4 *d_out, cudaStream_t stream, rg_stats *st, bool use_grid,
                              EventPool *events, EventPool &sync_events,
                              std::vector<std::pair<cudaEvent_t, cudaEvent_t>> *trace_spans) {
     const DScene &ds = sc->ds;
@@ -720,9 +720,9 @@ static int enqueue_batch_dev(rg_scene *sc, const DevPlan &plan, uint32_t width, 
         RG_CUDA(cudaGetLastError());
         st->gpu_launches++;
     }
-    if (sc->out_f32)
+    if (kind == OutKind::F32)
         k_export_f32<<<(npix + 255) / 256, 256, 0, stream>>>(wf.nodes[0].as<float4>(), reinterpret_cast<float *>(d_out), npix, po);
-    else if (sc->scatter_out)
+    else if (kind == OutKind::Rgba8Scatter)
         k_quantise_scatter<<<(unsigned)((((uint64_t)npix + 3) / 4 + 255) / 256), 256, 0, stream>>>(wf.nodes[0].as<float4>(), d_out, npix, d_rows, y0, po);
     else
         k_quantise<<<(unsigned)((((uint64_t)npix + 3) / 4 + 255) / 256), 256, 0, stream>>>(wf.nodes[0].as<float4>(), d_out, npix, po);
@@ -734,10 +734,10 @@ static int enqueue_batch_dev(rg_scene *sc, const DevPlan &plan, uint32_t width, 
 
 // ---- one CUDA graph per batch shape --------------------------------------------------------------
 static std::vector<uint64_t> graph_key(const rg_scene *sc, const DevPlan &plan, uint32_t width, uint32_t height, uint32_t y0,
-                                       uint32_t npix, const uint32_t *d_rows, const uchar4 *d_out, bool use_grid) {
+                                       uint32_t npix, const uint32_t *d_rows, OutKind kind, const uchar4 *d_out, bool use_grid) {
     const WavefrontScratch &wf = sc->wf;
     std::vector<uint64_t> k = {width, height, y0, npix, (uint64_t)(uintptr_t)d_rows, (uint64_t)(uintptr_t)d_out,
-                               (uint64_t)use_grid, (uint64_t)sc->scatter_out | ((uint64_t)sc->out_f32 << 1), (uint64_t)sc->ds.max_depth, (uint64_t)sc->overlap,
+                               (uint64_t)use_grid, (uint64_t)kind, (uint64_t)sc->ds.max_depth, (uint64_t)sc->overlap,
                                (uint64_t)sc->verify_cull, (uint64_t)sc->trace_stats | ((uint64_t)sc->origin_hints << 1), (uint64_t)plan.levels,
                                (uint64_t)sc->level_growth};   // the capacities are baked into the captured launches
     auto add = [&](const DeviceBuffer &b) { k.push_back((uint64_t)(uintptr_t)b.ptr); };
@@ -750,11 +750,11 @@ static std::vector<uint64_t> graph_key(const rg_scene *sc, const DevPlan &plan, 
 // Replays the batch from a captured graph; captures it when its key is seen for the second time.
 // Returns RG_OK with *done = false when the batch should be enqueued the ordinary way.
 static int graph_batch(rg_scene *sc, const DevPlan &plan, uint32_t width, uint32_t height, uint32_t y0, uint32_t npix,
-                       const uint32_t *d_rows, uchar4 *d_out, cudaStream_t stream, rg_stats *st, bool use_grid,
+                       const uint32_t *d_rows, OutKind kind, uchar4 *d_out, cudaStream_t stream, rg_stats *st, bool use_grid,
                        EventPool &sync_events, bool *done) {
     *done = false;
     GraphCache &gc = sc->graphs;
-    const std::vector<uint64_t> key = graph_key(sc, plan, width, height, y0, npix, d_rows, d_out, use_grid);
+    const std::vector<uint64_t> key = graph_key(sc, plan, width, height, y0, npix, d_rows, kind, d_out, use_grid);
     GraphEntry *hit = nullptr;
     for (auto &e : gc.entries)
         if (e.key == key) { hit = &e; break; }
@@ -772,7 +772,7 @@ static int graph_batch(rg_scene *sc, const DevPlan &plan, uint32_t width, uint32
         rg_stats tmp{};
         const size_t sync_used = sync_events.used;
         RG_CUDA(cudaStreamBeginCapture(cs, cudaStreamCaptureModeThreadLocal));
-        const int rc = enqueue_batch_dev(sc, plan, width, height, y0, npix, d_rows, d_out, cs, &tmp, use_grid, nullptr, sync_events, nullptr);
+        const int rc = enqueue_batch_dev(sc, plan, width, height, y0, npix, d_rows, kind, d_out, cs, &tmp, use_grid, nullptr, sync_events, nullptr);
         cudaGraph_t graph = nullptr;
         const cudaError_t ce = cudaStreamEndCapture(cs, &graph);
         sync_events.used = sync_used;
@@ -812,7 +812,7 @@ static int graph_batch(rg_scene *sc, const DevPlan &plan, uint32_t width, uint32
 }
 
 int wavefront_render(rg_scene *sc, uint32_t width, uint32_t height, uint32_t y0, uint32_t y1,
-                     const uint32_t *d_rows, uchar4 *d_out, cudaStream_t stream, rg_stats *st) {
+                     const uint32_t *d_rows, OutKind kind, uchar4 *d_out, cudaStream_t stream, rg_stats *st) {
     const DScene &ds = sc->ds;
     bool use_grid = false;
     if (sc->accel == RG_ACCEL_GRID) use_grid = ds.grid.enabled != 0;
@@ -839,18 +839,17 @@ int wavefront_render(rg_scene *sc, uint32_t width, uint32_t height, uint32_t y0,
         }
         for (uint32_t y = y0; y < y1 && rc == RG_OK;) {
             const uint32_t ye = (uint32_t)std::min<uint64_t>((uint64_t)y + batch_rows, y1);
-            // RGBA8: 4 bytes per pixel; f32 colours (rg_render_rows_f32): 12
-            uchar4 *out = sc->scatter_out ? d_out
-                        : reinterpret_cast<uchar4 *>(reinterpret_cast<unsigned char *>(d_out) + (size_t)(y - y0) * width * (sc->out_f32 ? 12 : 4));
+            uchar4 *out = kind == OutKind::Rgba8Scatter ? d_out
+                        : reinterpret_cast<uchar4 *>(reinterpret_cast<unsigned char *>(d_out) + (size_t)(y - y0) * width * bytes_per_pixel(kind));
             DevPlan plan;
             const uint64_t npix64 = (uint64_t)(ye - y) * width;
             if (npix64 > 0x7FFFFFFFull) { set_error("batch of %llu pixels is too large", (unsigned long long)npix64); rc = RG_E_NOMEM; }
             else if (npix64 && (rc = plan_batch_dev(sc, (uint32_t)npix64, plan, use_grid)) == RG_OK) {
                 bool done = false;
                 if (sc->graph != 1 && sc->verify_cull == 0)
-                    rc = graph_batch(sc, plan, width, height, y, (uint32_t)npix64, d_rows, out, stream, st, use_grid, sync_events, &done);
+                    rc = graph_batch(sc, plan, width, height, y, (uint32_t)npix64, d_rows, kind, out, stream, st, use_grid, sync_events, &done);
                 if (rc == RG_OK && !done)
-                    rc = enqueue_batch_dev(sc, plan, width, height, y, (uint32_t)npix64, d_rows, out, stream, st, use_grid, &events,
+                    rc = enqueue_batch_dev(sc, plan, width, height, y, (uint32_t)npix64, d_rows, kind, out, stream, st, use_grid, &events,
                                            sync_events, &trace_spans);
             }
             y = ye;
