@@ -35,7 +35,9 @@ extern "C" {
 /* Largest scene.max_recursion_depth the device path accepts (the reference's
  * default is 10, scene.rs:26; `--draft` lowers it to 4, src/main.rs:74-75). */
 #define RG_MAX_DEPTH 64u
-/* Largest light count (shadow results are kept in a 32-bit mask per hit). */
+/* Obsolete: scenes may have any number of lights.  Kept so that existing hosts compile.  It is
+ * still the size of one light chunk: the device shades a scene's lights RG_MAX_LIGHTS at a time,
+ * so a scene with at most this many lights takes exactly the path it always took. */
 #define RG_MAX_LIGHTS 32u
 
 /* ---- error codes (0 = ok, negative = failure; never unwinds across the ABI) */
@@ -48,7 +50,7 @@ enum {
     RG_E_CUDA = -5,       /* CUDA runtime failure / no usable device            */
     RG_E_NOMEM = -6,      /* device or host allocation failed                   */
     RG_E_CANCELLED = -7,  /* streaming callback asked to stop (rendering.rs:53-54,67) */
-    RG_E_LIGHTS = -8,     /* more than RG_MAX_LIGHTS lights                     */
+    RG_E_LIGHTS = -8,     /* obsolete: no longer returned (any light count is accepted) */
     RG_E_BUSY = -9        /* the handle is already rendering on another thread (the reference's &Scene
                              is Sync; a device scene owns its scratch: one render at a time per handle) */
 };

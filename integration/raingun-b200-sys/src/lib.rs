@@ -6,7 +6,7 @@ use std::os::raw::{c_char, c_int, c_void};
 
 pub const RG_ABI_VERSION: u32 = 2;
 pub const RG_MAX_DEPTH: u32 = 64;
-pub const RG_MAX_LIGHTS: u32 = 32;
+pub const RG_MAX_LIGHTS: u32 = 32; // obsolete: any light count is accepted (the size of one light chunk)
 pub const RG_IPC_HANDLE_BYTES: usize = 64;
 
 pub const RG_OK: c_int = 0;
@@ -17,7 +17,7 @@ pub const RG_E_DEPTH: c_int = -4;
 pub const RG_E_CUDA: c_int = -5;
 pub const RG_E_NOMEM: c_int = -6;
 pub const RG_E_CANCELLED: c_int = -7; // closed channel, rendering.rs:53-54,67
-pub const RG_E_LIGHTS: c_int = -8;
+pub const RG_E_LIGHTS: c_int = -8; // obsolete: no longer returned
 pub const RG_E_BUSY: c_int = -9;
 pub const RG_DEVICE_ALL: i32 = -1;
 

@@ -18,6 +18,7 @@ LIB_PATH = os.environ.get("RAINGUN_B200_LIB") or os.path.join(_HERE, "libraingun
 RG_OK = 0
 ERRORS = {0: "RG_OK", -1: "RG_E_INVALID", -2: "RG_E_PORTRAIT", -3: "RG_E_TOO_LARGE", -4: "RG_E_DEPTH",
           -5: "RG_E_CUDA", -6: "RG_E_NOMEM", -7: "RG_E_CANCELLED", -8: "RG_E_LIGHTS", -9: "RG_E_BUSY"}
+# E_LIGHTS is obsolete: scenes may have any number of lights, and the library no longer returns it
 E_INVALID, E_PORTRAIT, E_TOO_LARGE, E_DEPTH, E_CUDA, E_NOMEM, E_CANCELLED, E_LIGHTS, E_BUSY = -1, -2, -3, -4, -5, -6, -7, -8, -9
 DEVICE_ALL = -1
 

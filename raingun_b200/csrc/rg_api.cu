@@ -70,6 +70,7 @@ void WavefrontScratch::release() {
     ray[0].release(); ray[1].release(); hit_t.release(); hit_body.release();
     for (int p = 0; p < 2; ++p) {
         sray[p].release(); s_tmax[p].release(); s_ab[p].release(); s_lit[p].release(); lit_bc[p].release(); lit_node[p].release();
+        lit_geo[p].release(); lit_acc[p].release();
     }
     for (auto &b : nodes) b.release();
     nodes.clear();
@@ -166,7 +167,6 @@ static int validate(const rg_scene_desc *d) {
     if (!d) { set_error("scene desc is NULL"); return RG_E_INVALID; }
     if (d->abi_version != RG_ABI_VERSION) { set_error("abi_version %u != %u", d->abi_version, RG_ABI_VERSION); return RG_E_INVALID; }
     if (d->max_recursion_depth > RG_MAX_DEPTH) { set_error("max_recursion_depth %u > %u", d->max_recursion_depth, RG_MAX_DEPTH); return RG_E_DEPTH; }
-    if (d->n_lights > RG_MAX_LIGHTS) { set_error("%u lights > %u", d->n_lights, RG_MAX_LIGHTS); return RG_E_LIGHTS; }
     if (d->n_bodies && (!d->body_kind || !d->body_geom || !d->coloration_kind || !d->color || !d->texture_id ||
                         !d->texture_offset || !d->albedo || !d->surface_kind || !d->surface_param)) {
         set_error("a per-body array is NULL");
@@ -346,7 +346,8 @@ static int build_scene(rg_scene *sc, const rg_scene_desc *d) {
                  off_sph = align(off_mat + (size_t)n * sizeof(BodyMat)), off_sphb = align(off_sph + (size_t)n * 32),
                  off_misc = align(off_sphb + (size_t)n * 4), off_bsph = align(off_misc + (size_t)n * 4),
                  off_gmisc = align(off_bsph + (size_t)n * 4), off_face = align(off_gmisc + (size_t)n * 4),
-                 total = align(off_face + n_boxes * 6 * sizeof(FaceRef));
+                 off_light = align(off_face + n_boxes * 6 * sizeof(FaceRef)),
+                 total = align(off_light + (size_t)d->n_lights * sizeof(DLight));
     if (sc->h_stage_cap < total) {
         if (sc->h_stage) cudaFreeHost(sc->h_stage);
         sc->h_stage = nullptr;
@@ -438,8 +439,10 @@ static int build_scene(rg_scene *sc, const rg_scene_desc *d) {
     // P = centre of the bounding box of the sphere and proxy centres: reference point of the FP32 cull coordinates
     for (int k = 0; k < 3; ++k) ds.cull_ref[k] = have ? 0.5 * (lo[k] + hi[k]) : 0.0;
 
+    // every light goes to the arena (light_all); the first RG_MAX_LIGHTS also ride in the struct (rg_scene.cuh)
+    sc->lights.assign(d->n_lights, DLight{});
     for (uint32_t l = 0; l < d->n_lights; ++l) {
-        DLight &L = ds.lights[l];
+        DLight &L = sc->lights[l];
         L.kind = d->light_kind[l];
         const double *v = d->light_vec + 3 * (size_t)l;
         if (L.kind == RG_LIGHT_DIRECTIONAL) {
@@ -452,7 +455,9 @@ static int build_scene(rg_scene *sc, const rg_scene_desc *d) {
         }
         for (int k = 0; k < 3; ++k) L.color[k] = d->light_color[3 * (size_t)l + k];
         L.intensity = d->light_intensity[l];
+        if (l < RG_MAX_LIGHTS) ds.lights[l] = L;
     }
+    if (d->n_lights) std::memcpy(hs + off_light, sc->lights.data(), (size_t)d->n_lights * sizeof(DLight));
 
     lap("host flatten");
     uint8_t *dev = static_cast<uint8_t *>(sc->arena.alloc(total));
@@ -469,6 +474,7 @@ static int build_scene(rg_scene *sc, const rg_scene_desc *d) {
     ds.body_sph = n ? reinterpret_cast<const uint32_t *>(dev + off_bsph) : nullptr;
     ds.cull4 = nsp ? cull4 : nullptr;
     ds.cull2 = ns ? cull2 : nullptr;
+    ds.light_all = d->n_lights ? reinterpret_cast<const DLight *>(dev + off_light) : nullptr;
     if (cull_padded) {
         k_cull_records<<<(unsigned)((cull_padded + 255) / 256), 256, 0, sc->stream>>>(ds.sph, ns, (uint32_t)cull_padded, ds.cull_ref[0],
                                                                                       ds.cull_ref[1], ds.cull_ref[2], cull4, cull2);
@@ -715,8 +721,9 @@ static int mega_render(rg_scene *sc, uint32_t w, uint32_t h, uint32_t y0, uint32
     if (npix) {
         const unsigned blocks = (unsigned)((npix + 127) / 128);
         float *f32 = kind == OutKind::F32 ? reinterpret_cast<float *>(d_out) : nullptr;
-        if (sc->ds.max_depth <= 12) k_render_mega<12><<<blocks, 128, 0, stream>>>(sc->ds, w, h, y0, y1, d_rows, d_out, f32, sc->d_counters);
-        else k_render_mega<RG_MAX_DEPTH><<<blocks, 128, 0, stream>>>(sc->ds, w, h, y0, y1, d_rows, d_out, f32, sc->d_counters);
+        auto kernel = sc->ds.max_depth <= 12 ? k_render_mega<12, false> : k_render_mega<RG_MAX_DEPTH, false>;
+        if (sc->ds.n_lights > RG_MAX_LIGHTS) kernel = sc->ds.max_depth <= 12 ? k_render_mega<12, true> : k_render_mega<RG_MAX_DEPTH, true>;
+        kernel<<<blocks, 128, 0, stream>>>(sc->ds, w, h, y0, y1, d_rows, d_out, f32, sc->d_counters);
         RG_CUDA(cudaGetLastError());
     }
     RG_CUDA(cudaEventRecord(sc->ev[1], stream));

@@ -54,6 +54,9 @@ struct WavefrontScratch {
     DeviceBuffer s_lit[2];      // in_light byte per shadow ray
     DeviceBuffer lit_bc[2];     // float4 (body colour, albedo) per lit hit
     DeviceBuffer lit_node[2];   // node index per lit hit
+    // Scenes with more than RG_MAX_LIGHTS lights only (light chunks after the first, rg_wavefront.cu):
+    DeviceBuffer lit_geo[2];    // per lit hit: hit point and normal (f64, a RayQueue with o = point, d = normal) + body
+    DeviceBuffer lit_acc[2];    // per lit hit: float4 RGB sum of the chunks so far
     std::vector<DeviceBuffer> nodes;   // per level: NodeA float4 + NodeB uint4
     std::vector<cudaEvent_t> events;   // timing events of the trace launches, reused across frames
     cudaStream_t aux = nullptr;        // shadow-side stream (created on first use)
@@ -114,6 +117,8 @@ struct rg_scene : rg::DeviceContext {
     std::atomic<bool> busy{false};         // a render call is running on this handle (second callers get RG_E_BUSY)
     rg::DScene ds{};                    // device pointers inside
     rg::GridProxies gp{};               // boxes and disks binned into the grid (rg_scene.cuh)
+    std::vector<rg::DLight> lights;        // every light, as uploaded (light_all): the host builds each light chunk's
+                                           // DScene from these without reading the device
     std::vector<cudaTextureObject_t> tex_objs;
     uint8_t *h_frame = nullptr;            // pinned staging of the streaming renders (not parked; a multi-GPU handle has one too)
     size_t h_frame_cap = 0;

@@ -16,14 +16,18 @@ struct MegaFrame {
     uint8_t stage;    // Refractive: 0 = refraction in flight, 1 = reflection in flight
 };
 
-// rendering.rs:132-172 with a full nearest-hit trace per light, exactly as written there.
+// rendering.rs:132-172 with a full nearest-hit trace per light, exactly as written there.  MANY_LIGHTS (a scene with
+// more than RG_MAX_LIGHTS lights): the lights come from the arena copy (DScene::light_all) instead of the constant
+// bank.  (One kernel for both costs the common case 14 registers: lights read from global memory stay in registers
+// across the trace, where constant-bank ones are read again.)
+template <bool MANY_LIGHTS>
 __device__ __forceinline__ C3 mega_shade_diffuse(const DScene &s, uint32_t body, D3 hp, D3 n,
                                                  DCounters *ctr, unsigned long long &n_shadow) {
     C3 bc = body_color_at(s, body, hp);
     float albedo = s.mat[body].albedo;
     C3 fin = c3(0.0f, 0.0f, 0.0f);
     for (uint32_t l = 0; l < s.n_lights; ++l) {
-        const DLight &L = s.lights[l];
+        const DLight &L = MANY_LIGHTS ? s.light_all[l] : s.lights[l];
         D3 dir = light_direction_from(L, hp);
         Ray shadow;
         shadow.o = hp + n * kShadowBias;
@@ -37,7 +41,7 @@ __device__ __forceinline__ C3 mega_shade_diffuse(const DScene &s, uint32_t body,
     return clamp01(fin);
 }
 
-template <int STACK>
+template <int STACK, bool MANY_LIGHTS>
 __global__ void __launch_bounds__(128)
 k_render_mega(DScene s, uint32_t width, uint32_t height, uint32_t y0, uint32_t y1, const uint32_t *__restrict__ rows,
               uchar4 *__restrict__ out, float *__restrict__ out_f32, DCounters *ctr) {
@@ -67,13 +71,13 @@ k_render_mega(DScene s, uint32_t width, uint32_t height, uint32_t y0, uint32_t y
                 D3 n = surface_normal(s, h.body, hp, ctr);
                 const BodyMat &m = s.mat[h.body];
                 if (m.surface == RG_SURFACE_DIFFUSE) {
-                    ret = mega_shade_diffuse(s, h.body, hp, n, ctr, cnt[1]);
+                    ret = mega_shade_diffuse<MANY_LIGHTS>(s, h.body, hp, n, ctr, cnt[1]);
                     calling = false;
                 } else if (m.surface == RG_SURFACE_REFLECTING) {
                     MegaFrame &f = stack[sp++];
                     f.kind = RG_SURFACE_REFLECTING;
                     f.p0 = m.p0;
-                    f.a = mega_shade_diffuse(s, h.body, hp, n, ctr, cnt[1]);
+                    f.a = mega_shade_diffuse<MANY_LIGHTS>(s, h.body, hp, n, ctr, cnt[1]);
                     ray = create_reflection(n, ray.d, hp);
                     ray_kind = 2;
                 } else {

@@ -10,7 +10,11 @@
 //   * cull4[n_spheres]: the FP32 conservative-cull record of each sphere (rg_trace.cuh), followed by those of
 //     the grid's box / disk proxies (GridProxies below);
 //   * the exact-culling grid (rg_grid.cuh);
-//   * lights by value inside the struct (<= RG_MAX_LIGHTS), textures as CUDA texture objects.
+//   * lights: the first min(L, RG_MAX_LIGHTS) by value inside the struct (kernels read them from the
+//     constant bank), all L in the arena behind light_all; textures as CUDA texture objects.
+//     A scene with more than RG_MAX_LIGHTS lights is shaded in chunks of RG_MAX_LIGHTS lights
+//     (rg_wavefront.cu): each chunk's launches get a copy of this struct whose lights[] / n_lights
+//     hold that chunk only.
 #pragma once
 #include <cuda_runtime.h>
 #include <stdint.h>
@@ -81,7 +85,9 @@ struct DScene {
     float default_color[3];
     uint32_t max_depth;
     GridDev grid;
-    DLight lights[RG_MAX_LIGHTS];
+    DLight lights[RG_MAX_LIGHTS];   // lights [0, min(n_lights, RG_MAX_LIGHTS)), or one chunk of them (see above)
+    const DLight *light_all;      // [n_lights of the scene] every light, in scene order (after lights[]: the
+                                  // offsets of the fields above stay what they were)
 };
 
 // Boxes and disks in the grid (rg_grid.cuh, DESIGN.md section 4.2).  A binnable box or disk enters the grid as

@@ -9,6 +9,8 @@
 //                                                         get_color, fresnel, Ray::create_*
 //     k_trace_*  (ANY) the shadow rays                    shade_diffuse           rendering.rs:150-155
 //     k_diffuse  the per-light sum, in light order        shade_diffuse           rendering.rs:157-171
+// (a scene with more than RG_MAX_LIGHTS lights runs the last two per chunk of RG_MAX_LIGHTS lights,
+// k_shadow_rays setting up every chunk after the first: see enqueue_batch_dev)
 // and after the deepest level, bottom-up:
 //     k_combine  parent colour from its children's        get_color               rendering.rs:88-116
 //     k_quantise Color::rgba                                                      color.rs:32-37
@@ -57,7 +59,14 @@ struct LevelBuffers {
     uint32_t last_enqueued;          // no launch follows for this level's children (depth hint): flag them
     uint32_t hints;                  // the tracer reads origin hints (rg_trace.cuh): 1 = compute them, 2 = write kHintNone
                                      // (RG_OPT_ORIGIN_HINTS = 0), 0 = the tracer ignores them (brute force): write nothing
+    uint32_t n_lights;               // lights of the scene: shadow rays per lit hit, all chunks together
+    RayQueue lit_geo;                // light chunks after the first follow (k_shadow_rays): per lit hit, hit point (o),
+                                     // normal (d) and body (hint); a == nullptr: not kept
 };
+
+// Lights are shaded in chunks of this many (a scene with at most this many lights has exactly one).  It bounds the
+// shadow queues at cap x kLightChunk rays per level parity whatever the scene's light count.
+constexpr uint32_t kLightChunk = RG_MAX_LIGHTS;
 
 // Size of a level as its kernels see it: read from the device and clamped to the capacity (0 once the frame is void).
 __device__ __forceinline__ uint32_t level_size(uint32_t cap, const unsigned int *n_dev, const unsigned int *void_flag) {
@@ -116,6 +125,22 @@ __device__ __forceinline__ uint32_t shadow_origin_hint(const double *og, uint32_
     if (!sphere_intersect(og[0], og[1], og[2], og[3], r, t)) return own;
     if (t <= tmax) return kHintOccluded;   // rendering.rs:150-155: nearest.distance <= light distance for some body
     return t == t ? own : kHintNone;       // beyond the light: contributes nothing; NaN: the tracer counts it (scene.rs:38)
+}
+
+// shade_diffuse's per-(hit, light) setup (rendering.rs:141-149,163): the shadow ray from hit_point + n * SHADOW_BIAS
+// towards the light, stored at slot k with the light's distance (the trace's tmax), the ray's origin hint and the
+// light-dependent scalars (max(n.L, 0), intensity) that k_diffuse needs.  k_shade runs it for the first light chunk,
+// k_shadow_rays for the later ones: the arithmetic exists once.
+__device__ __forceinline__ void shadow_ray_setup(const LevelBuffers &lb, uint32_t k, const DLight &L, D3 hp, D3 n,
+                                                 const double *og, uint32_t own) {
+    Ray sh;
+    sh.o = hp + n * kShadowBias;
+    sh.d = light_direction_from(L, hp);
+    store_ray(lb.shadow, k, sh);
+    const double tmax = light_distance(L, hp);
+    lb.s_tmax[k] = tmax;
+    if (lb.hints) lb.shadow.hint[k] = shadow_origin_hint(og, own, sh, tmax);
+    lb.s_ab[k] = make_float2(fmaxf((float)dot(n, sh.d), 0.0f), light_intensity(L, hp));
 }
 
 #ifndef RG_SHADE_MINB
@@ -204,7 +229,7 @@ __global__ void __launch_bounds__(256, RG_SHADE_MINB) k_shade(const DScene s, co
         }
         if (n_next_b - n_trans_b) atomicAdd(&ctr->rays[2], (unsigned long long)(n_next_b - n_trans_b));
         if (n_trans_b) atomicAdd(&ctr->rays[3], (unsigned long long)n_trans_b);
-        if (n_lit_b) atomicAdd(&ctr->rays[1], (unsigned long long)n_lit_b * s.n_lights);
+        if (n_lit_b) atomicAdd(&ctr->rays[1], (unsigned long long)n_lit_b * lb.n_lights);
     }
     __syncthreads();
     if (sh_drop) { want_refl = false; want_trans = false; }
@@ -230,27 +255,21 @@ __global__ void __launch_bounds__(256, RG_SHADE_MINB) k_shade(const DScene s, co
         if (lb.hints) lb.next.hint[child_trans] = path_origin_hint(og, own, trans);
     }
     if (want_lit) {
-        // shade_diffuse's per-light setup (rendering.rs:141-149,163): shadow ray from
-        // hit_point + n * SHADOW_BIAS towards the light; the light-dependent scalars are kept
-        // for k_diffuse.  (Doing this warp-cooperatively — one (hit, light) pair per lane instead of a
+        // shade_diffuse's per-light setup of the lights in `s` (all of them, or the first chunk).  (Doing this warp-cooperatively — one (hit, light) pair per lane instead of a
         // per-light loop in the ~third of the lanes that are lit — was measured: no gain once the kernel
         // runs at 64 registers; it waits on gathers, not on issue slots.  Likewise partitioning a block's rays
         // into misses / refractive hits / lit hits so that every warp runs one path: 18.83 vs 18.93 ms.)
         const uint32_t j = base_lit + __popc(m_lit & lt);
         lb.lit_node[j] = i;
         lb.lit_bc[j] = make_float4(bc.r, bc.g, bc.b, s.mat[body].albedo);
-        Ray sh;
-        sh.o = hp + n * kShadowBias;
-        for (uint32_t l = 0; l < s.n_lights; ++l) {
-            const DLight &L = s.lights[l];
-            sh.d = light_direction_from(L, hp);
-            const uint32_t k = l * lb.shadow_sl + j * lb.shadow_sj;
-            store_ray(lb.shadow, k, sh);
-            const double tmax = light_distance(L, hp);
-            lb.s_tmax[k] = tmax;
-            if (lb.hints) lb.shadow.hint[k] = shadow_origin_hint(og, own, sh, tmax);
-            lb.s_ab[k] = make_float2(fmaxf((float)dot(n, sh.d), 0.0f), light_intensity(L, hp));
+        if (lb.lit_geo.a) {   // more light chunks follow: keep what k_shadow_rays needs (the path side reuses hit_t / hit_body)
+            Ray g;
+            g.o = hp;
+            g.d = n;
+            store_ray(lb.lit_geo, j, g);
+            lb.lit_geo.hint[j] = body;
         }
+        for (uint32_t l = 0; l < s.n_lights; ++l) shadow_ray_setup(lb, l * lb.shadow_sl + j * lb.shadow_sj, s.lights[l], hp, n, og, own);
     }
     if (active) {
         lb.node_a[i] = na;
@@ -259,22 +278,49 @@ __global__ void __launch_bounds__(256, RG_SHADE_MINB) k_shade(const DScene s, co
     }   // grid-stride loop
 }
 
-// rendering.rs:140,157-171: final_color accumulates light by light, in scene order, then clamps.
+// Shadow rays of a light chunk after the first (scenes with more than kLightChunk lights), from the lit-hit geometry
+// k_shade kept: one thread per (light of the chunk, lit hit), light-major like the queue, so that neighbouring threads
+// store neighbouring slots of one light's segment.  `s` holds the chunk's lights.  Block 0 rearms the level's
+// shadow-trace counter for this chunk's trace: the previous chunk's trace, earlier on the same stream, used it up.
+__global__ void __launch_bounds__(256) k_shadow_rays(const DScene s, const LevelBuffers lb, unsigned int *fetch_shadow) {
+    if (blockIdx.x == 0 && threadIdx.x == 0) *fetch_shadow = 0u;
+    const uint32_t n_lit = level_size(lb.cap, lb.q_lit, lb.void_flag);
+    const uint32_t n = n_lit * s.n_lights;   // <= cap x kLightChunk < 2^31 (plan_batch_dev)
+    for (uint32_t t = blockIdx.x * blockDim.x + threadIdx.x; t < n; t += gridDim.x * blockDim.x) {
+        const uint32_t l = t / n_lit, j = t - l * n_lit;
+        const Ray g = load_ray(lb.lit_geo, j);   // o = hit point, d = normal
+        const uint32_t body = lb.lit_geo.hint[j];
+        const double *og = nullptr;
+        uint32_t own = kHintNone;
+        if (lb.hints == 1u && s.kind[body] == RG_BODY_SPHERE) {   // as in k_shade
+            own = s.body_sph[body];
+            og = s.geom + 8 * (size_t)body;
+        }
+        shadow_ray_setup(lb, l * lb.shadow_sl + j * lb.shadow_sj, s.lights[l], g.o, g.d, og, own);
+    }
+}
+
+// rendering.rs:140,157-171: final_color accumulates light by light, in scene order, then clamps.  With several light
+// chunks (`s` holds one), `acc_in` (nullptr: the first chunk, start from 0) is the sum of the chunks before, and
+// `acc_out` (nullptr: the last chunk, clamp and write the node) receives the sum so far.  An f32 stored and loaded
+// keeps its bits and the chunks run in light order, so the sum is ((0 + t0) + t1) + ..., the reference's.
 __global__ void __launch_bounds__(256) k_diffuse(const DScene s, const float4 *__restrict__ lit_bc,
                                                  const uint32_t *__restrict__ lit_node, const float2 *__restrict__ s_ab,
                                                  const uint8_t *__restrict__ s_lit, float4 *node_a, uint32_t cap,
                                                  uint32_t shadow_sl, uint32_t shadow_sj, const unsigned int *n_lit_dev,
-                                                 const unsigned int *void_flag) {
+                                                 const unsigned int *void_flag, const float4 *acc_in, float4 *acc_out) {
     const uint32_t n_lit = level_size(cap, n_lit_dev, void_flag);
     for (uint32_t j = blockIdx.x * blockDim.x + threadIdx.x; j < n_lit; j += gridDim.x * blockDim.x) {
     const float4 b = lit_bc[j];
     const C3 bc = c3(b.x, b.y, b.z);
     C3 fin = c3(0.0f, 0.0f, 0.0f);
+    if (acc_in) { const float4 c = acc_in[j]; fin = c3(c.x, c.y, c.z); }
     for (uint32_t l = 0; l < s.n_lights; ++l) {
         const uint32_t k = l * shadow_sl + j * shadow_sj;
         const float2 ab = s_ab[k];
         fin = fin + light_term(bc, s.lights[l], b.w, ab.x, ab.y, s_lit[k] != 0);
     }
+    if (acc_out) { acc_out[j] = make_float4(fin.r, fin.g, fin.b, 0.0f); continue; }
     fin = clamp01(fin);
     const uint32_t node = lit_node[j];
     float4 a = node_a[node];
@@ -559,10 +605,11 @@ static int plan_batch_dev(rg_scene *sc, uint32_t npix, DevPlan &plan, bool use_g
     // emitted children (wavefront_render), else it is repeated with every level.
     plan.levels = std::max<uint32_t>(ds.max_depth, 1u);
     if (sc->depth_hint && sc->depth_hint < plan.levels) plan.levels = sc->depth_hint;
+    const uint32_t C = std::min(L, kLightChunk);   // lights per chunk: the shadow queues hold one chunk at a time
     uint64_t cap_max[2] = {0, 0}, cap_all = 0;
     for (uint32_t d = 0; d < plan.levels; ++d) {
         const uint64_t c = d == 0 ? npix : std::min<uint64_t>(2ull * plan.cap[d - 1], (uint64_t)sc->level_growth * npix);
-        if (c > 0x7FFFFFFFull || c * std::max<uint32_t>(L, 1u) > 0x7FFFFFFFull) {
+        if (c > 0x7FFFFFFFull || c * std::max<uint32_t>(C, 1u) > 0x7FFFFFFFull) {
             set_error("level %u could hold more than 2^31 rays; use a smaller batch", d);
             return RG_E_NOMEM;
         }
@@ -577,7 +624,7 @@ static int plan_batch_dev(rg_scene *sc, uint32_t npix, DevPlan &plan, bool use_g
     if ((rc = wf.hit_t.reserve((size_t)cap_all * 8))) return rc;
     if ((rc = wf.hit_body.reserve((size_t)cap_all * 4))) return rc;
     for (int p = 0; p < 2; ++p) {
-        const uint64_t c = std::max<uint64_t>(cap_max[p], 1), sc_ = std::max<uint64_t>(c * L, 1);
+        const uint64_t c = std::max<uint64_t>(cap_max[p], 1), sc_ = std::max<uint64_t>(c * C, 1);
         if ((rc = wf.ray[p].reserve((size_t)c * kRayBytes))) return rc;
         if ((rc = wf.sray[p].reserve((size_t)sc_ * kRayBytes))) return rc;
         if ((rc = wf.s_tmax[p].reserve((size_t)sc_ * 8))) return rc;
@@ -585,8 +632,21 @@ static int plan_batch_dev(rg_scene *sc, uint32_t npix, DevPlan &plan, bool use_g
         if ((rc = wf.s_lit[p].reserve((size_t)sc_))) return rc;
         if ((rc = wf.lit_bc[p].reserve((size_t)c * 16))) return rc;
         if ((rc = wf.lit_node[p].reserve((size_t)c * 4))) return rc;
+        if (L > kLightChunk) {   // the lit hits' geometry and partial sums outlive k_shade by the later chunks
+            if ((rc = wf.lit_geo[p].reserve((size_t)c * kRayBytes))) return rc;
+            if ((rc = wf.lit_acc[p].reserve((size_t)c * 16))) return rc;
+        }
     }
     return RG_OK;
+}
+
+// The DScene of light chunk c: lights [c * kLightChunk, ...) inline, the rest of the struct as the scene's.
+static DScene chunk_scene(const rg_scene *sc, uint32_t c) {
+    DScene cs = sc->ds;
+    const uint32_t first = c * kLightChunk;
+    cs.n_lights = std::min<uint32_t>(kLightChunk, (uint32_t)sc->lights.size() - first);
+    std::copy(sc->lights.begin() + first, sc->lights.begin() + first + cs.n_lights, cs.lights);
+    return cs;
 }
 
 // Enqueues one batch.  No allocation, no synchronisation, no host read: legal inside a stream capture.
@@ -614,6 +674,16 @@ static int enqueue_batch_dev(rg_scene *sc, const DevPlan &plan, uint32_t width, 
     const bool overlap = L > 0 && (sc->overlap == 2 || (sc->overlap == 0 && use_grid));
     cudaStream_t aux = overlap ? wf.aux : stream;
     cudaEvent_t shadow_done[2] = {nullptr, nullptr};
+    // Light chunks.  A scene with more than kLightChunk lights shades them kLightChunk at a time: k_shade sets up the
+    // first chunk's shadow rays and keeps each lit hit's geometry; every later chunk gets its rays from k_shadow_rays.
+    // Each chunk is traced and summed by k_diffuse into a per-hit f32 accumulator; the last chunk clamps.  Each chunk's
+    // launches take a DScene holding that chunk's lights, so the kernels read them from the constant bank as always.
+    const bool chunked = L > kLightChunk;
+    const uint32_t n_chunks = chunked ? (L + kLightChunk - 1) / kLightChunk : 1u;
+    const uint32_t C = std::min(L, kLightChunk);
+    std::vector<DScene> chunks;
+    if (chunked)
+        for (uint32_t c = 0; c < n_chunks; ++c) chunks.push_back(chunk_scene(sc, c));
 
     RG_CUDA(cudaMemsetAsync(dc->lvl, 0, sizeof(dc->lvl), stream));
     RayQueue cur = make_queue(wf.ray[0], plan.cap[0]);
@@ -648,7 +718,7 @@ static int enqueue_batch_dev(rg_scene *sc, const DevPlan &plan, uint32_t width, 
         LevelBuffers lb{};
         lb.cur = cur;
         lb.next = make_queue(wf.ray[(d + 1) & 1], std::max<uint32_t>(cap_next, 1u));
-        lb.shadow = make_queue(wf.sray[p], (size_t)std::max<uint64_t>((uint64_t)cap * L, 1));
+        lb.shadow = make_queue(wf.sray[p], (size_t)std::max<uint64_t>((uint64_t)cap * C, 1));
         lb.hit_t = wf.hit_t.as<double>();
         lb.hit_body = wf.hit_body.as<uint32_t>();
         lb.node_a = wf.nodes[d].as<float4>();
@@ -661,7 +731,7 @@ static int enqueue_batch_dev(rg_scene *sc, const DevPlan &plan, uint32_t width, 
         lb.n_dev = &dc->lvl[d].n;
         const bool light_major = shadow_light_major();
         lb.shadow_sl = light_major ? cap : 1u;   // one segment of `cap` slots per light, or the L rays of a hit adjacent
-        lb.shadow_sj = light_major ? 1u : L;
+        lb.shadow_sj = light_major ? 1u : C;
         lb.can_spawn = can_spawn ? 1u : 0u;
         lb.q_next = &dc->lvl[d + 1].n;
         lb.q_lit = &dc->lvl[d].n_lit;
@@ -670,40 +740,55 @@ static int enqueue_batch_dev(rg_scene *sc, const DevPlan &plan, uint32_t width, 
         lb.level = d;
         lb.hints = use_grid ? (sc->origin_hints ? 1u : 2u) : 0u;
         lb.last_enqueued = (d + 1 == plan.levels && can_spawn) ? 1u : 0u;
+        lb.n_lights = L;
+        if (chunked) lb.lit_geo = make_queue(wf.lit_geo[p], cap);
         if (shadow_done[p]) RG_CUDA(cudaStreamWaitEvent(stream, shadow_done[p], 0));   // level d-2 still reads these buffers
-        k_shade<<<blocks(cap), 256, 0, stream>>>(ds, lb, dc);
+        k_shade<<<blocks(cap), 256, 0, stream>>>(chunked ? chunks[0] : ds, lb, dc);
         RG_CUDA(cudaGetLastError());
         st->gpu_launches++;
 
-        if (L) {   // shadow side, concurrent with the next level's path side
-            if (overlap) {
-                cudaEvent_t shaded = sync_events.get();
-                RG_CUDA(cudaEventRecord(shaded, stream));
-                RG_CUDA(cudaStreamWaitEvent(aux, shaded, 0));
-            }
-            TraceArgs sa{};
-            sa.q = lb.shadow;
-            sa.tmax = lb.s_tmax;
-            sa.n = cap * L;
-            sa.n_dev = &dc->lvl[d].n_lit;
-            sa.n_mul = L;
-            sa.seg_len_dev = light_major ? &dc->lvl[d].n_lit : nullptr;
-            sa.seg_stride = cap;
-            sa.void_flag = &dc->overflow;
-            sa.fetch = &dc->lvl[d].fetch_shadow;
-            sa.out_lit = wf.s_lit[p].as<uint8_t>();
-            sa.ctr = dc;
-            sa.verify = sc->verify_cull == 1;
-            if (events) { e0 = events->get(); e1 = events->get(); RG_CUDA(cudaEventRecord(e0, aux)); }
-            if ((rc = launch_trace<true>(sc, sa, use_grid, aux))) return rc;
-            if (events) { RG_CUDA(cudaEventRecord(e1, aux)); trace_spans->emplace_back(e0, e1); }
-            st->gpu_launches++;
-            if (sc->verify_cull >= 2) k_verify_trace<true><<<(sa.n + 127) / 128, 128, 0, aux>>>(ds, sa, (int)d);
+        if (L && overlap) {   // shadow side, concurrent with the next level's path side
+            cudaEvent_t shaded = sync_events.get();
+            RG_CUDA(cudaEventRecord(shaded, stream));
+            RG_CUDA(cudaStreamWaitEvent(aux, shaded, 0));
         }
-        k_diffuse<<<blocks(cap), 256, 0, aux>>>(ds, lb.lit_bc, lb.lit_node, lb.s_ab, wf.s_lit[p].as<uint8_t>(), lb.node_a, cap,
-                                                lb.shadow_sl, lb.shadow_sj, &dc->lvl[d].n_lit, &dc->overflow);
-        RG_CUDA(cudaGetLastError());
-        st->gpu_launches++;
+        float4 *acc = chunked ? wf.lit_acc[p].as<float4>() : nullptr;
+        for (uint32_t c = 0; c < n_chunks; ++c) {   // (one pass, c = 0, unless the scene has more than kLightChunk lights)
+            const DScene &cs = chunked ? chunks[c] : ds;
+            const uint32_t Lc = cs.n_lights;
+            LevelBuffers lc = lb;
+            lc.shadow_sj = light_major ? 1u : Lc;
+            if (c > 0) {
+                k_shadow_rays<<<blocks((uint64_t)cap * Lc), 256, 0, aux>>>(cs, lc, &dc->lvl[d].fetch_shadow);
+                RG_CUDA(cudaGetLastError());
+                st->gpu_launches++;
+            }
+            if (Lc) {
+                TraceArgs sa{};
+                sa.q = lc.shadow;
+                sa.tmax = lc.s_tmax;
+                sa.n = cap * Lc;
+                sa.n_dev = &dc->lvl[d].n_lit;
+                sa.n_mul = Lc;
+                sa.seg_len_dev = light_major ? &dc->lvl[d].n_lit : nullptr;
+                sa.seg_stride = cap;
+                sa.void_flag = &dc->overflow;
+                sa.fetch = &dc->lvl[d].fetch_shadow;
+                sa.out_lit = wf.s_lit[p].as<uint8_t>();
+                sa.ctr = dc;
+                sa.verify = sc->verify_cull == 1;
+                if (events) { e0 = events->get(); e1 = events->get(); RG_CUDA(cudaEventRecord(e0, aux)); }
+                if ((rc = launch_trace<true>(sc, sa, use_grid, aux))) return rc;
+                if (events) { RG_CUDA(cudaEventRecord(e1, aux)); trace_spans->emplace_back(e0, e1); }
+                st->gpu_launches++;
+                if (sc->verify_cull >= 2) k_verify_trace<true><<<(sa.n + 127) / 128, 128, 0, aux>>>(cs, sa, (int)d);
+            }
+            k_diffuse<<<blocks(cap), 256, 0, aux>>>(cs, lc.lit_bc, lc.lit_node, lc.s_ab, wf.s_lit[p].as<uint8_t>(), lc.node_a, cap,
+                                                    lc.shadow_sl, lc.shadow_sj, &dc->lvl[d].n_lit, &dc->overflow,
+                                                    c > 0 ? acc : nullptr, c + 1 < n_chunks ? acc : nullptr);
+            RG_CUDA(cudaGetLastError());
+            st->gpu_launches++;
+        }
         if (overlap) {
             shadow_done[p] = sync_events.get();
             RG_CUDA(cudaEventRecord(shadow_done[p], aux));
@@ -744,6 +829,9 @@ static std::vector<uint64_t> graph_key(const rg_scene *sc, const DevPlan &plan, 
     add(wf.ray[0]); add(wf.ray[1]); add(wf.hit_t); add(wf.hit_body);
     for (int p = 0; p < 2; ++p) { add(wf.sray[p]); add(wf.s_tmax[p]); add(wf.s_ab[p]); add(wf.s_lit[p]); add(wf.lit_bc[p]); add(wf.lit_node[p]); }
     for (uint32_t d = 0; d < plan.levels; ++d) add(wf.nodes[d]);
+    // The light-chunk count needs no entry: it is fixed by the handle's scene, and a graph dies with its scene.
+    if (sc->ds.n_lights > kLightChunk)
+        for (int p = 0; p < 2; ++p) { add(wf.lit_geo[p]); add(wf.lit_acc[p]); }
     return k;
 }
 

@@ -192,3 +192,55 @@ def make_box_scene(name: str = "B4", bodies: Optional[int] = None, depth: Option
         raise KeyError(name)
     doc = make_box_scene_doc(bodies, depth)
     return scene_from_dict(doc, texture_loader or default_texture_loader), B4
+
+
+# L<n>: C4's bodies (its stream, cut short by `spheres`) lit by n lights, kept out of SPECS as B4 is.  The lights
+# come from a stream of their own, so the bodies of every light count are the same.
+LIGHTS_SEED = 1005
+
+
+def make_light_scene_doc(lights: int, spheres: Optional[int] = None, depth: Optional[int] = None
+                         ) -> Dict[str, Any]:
+    """The YAML document of a many-light scene: C4's ground plane and mixed reflecting / refractive /
+    diffuse spheres (``spheres`` of them, default C4's 10,000; depth 8 unless ``depth``), lit by
+    ``lights`` lights that alternate directional (even indices) and spherical (odd indices).  SplitMix64
+    seed 1005, ``U`` as for C3-C5; per light the draw order is the colour (``next_u64 & 0xFFFFFF``),
+    then for a directional light x, y, z of the direction from U(-1, 1), U(-1, -0.2), U(-1, 1) and the
+    intensity from U(1, 7), for a spherical light x, y, z of the position from U(-20, 20), U(4, 20),
+    U(-50, 0) and the intensity from U(4000, 12000); intensities are scaled by 3 / lights so that the
+    image does not saturate.  Three lights are then placed by hand: light 1 sits at the centre of the
+    first sphere (inside a body), light 3 behind the camera at (0, 2, 6), and light 2 has intensity 0."""
+    doc = make_scene_doc(SPECS["C4"], spheres, depth)
+    rng = SplitMix64(LIGHTS_SEED)
+    scale = 3.0 / max(int(lights), 1)
+    first_sphere = next((b["Sphere"]["center"] for b in doc["bodies"] if "Sphere" in b), [0.0, 4.0, -20.0])
+    out: List[Dict[str, Any]] = []
+    for i in range(int(lights)):
+        colour = "#%06x" % (rng.next_u64() & 0xFFFFFF)
+        if i % 2 == 0:
+            direction = {"x": rng.uniform(-1.0, 1.0), "y": rng.uniform(-1.0, -0.2), "z": rng.uniform(-1.0, 1.0)}
+            intensity = round(rng.uniform(1.0, 7.0) * scale, 6)
+            if i == 2:
+                intensity = 0.0
+            out.append({"Directional": {"direction": direction, "color": colour, "intensity": intensity}})
+        else:
+            position = [rng.uniform(-20.0, 20.0), rng.uniform(4.0, 20.0), rng.uniform(-50.0, 0.0)]
+            intensity = round(rng.uniform(4000.0, 12000.0) * scale, 6)
+            if i == 1:
+                position = list(first_sphere)
+            elif i == 3:
+                position = [0.0, 2.0, 6.0]
+            out.append({"Spherical": {"position": position, "color": colour, "intensity": intensity}})
+    doc["lights"] = out
+    return doc
+
+
+def make_light_scene(lights: int, spheres: Optional[int] = None, depth: Optional[int] = None,
+                     texture_loader=None):
+    """SceneData of the many-light scene with ``lights`` lights (see make_light_scene_doc) and its spec."""
+    from .scene import default_texture_loader, scene_from_dict
+
+    doc = make_light_scene_doc(lights, spheres, depth)
+    spec = SynthSpec("L%d" % int(lights), 3840, 2160, LIGHTS_SEED, len(doc["bodies"]) - 1, 24.0, (-1.5, 18.0),
+                     (-45.0, -4.0), (0.08, 0.35), True, False, int(lights), doc["maxRecursionDepth"])
+    return scene_from_dict(doc, texture_loader or default_texture_loader), spec
