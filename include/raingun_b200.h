@@ -136,7 +136,8 @@ enum {
     RG_OPT_PIPELINE = 1,
     RG_OPT_ACCEL = 2,
     RG_OPT_MAX_DEPTH = 3,    /* like main.rs:119-123: lowers max_recursion_depth  */
-    RG_OPT_BATCH_PIXELS = 4, /* pixels per wavefront batch (0 = automatic)         */
+    RG_OPT_BATCH_PIXELS = 4, /* pixels per wavefront batch (0 = automatic); with RG_OPT_SUPERSAMPLE > 1, samples per
+                                batch, and per band of the megakernel's sample scratch */
     RG_OPT_VERIFY_CULL = 5,  /* debug: count FP32-culled pairs the FP64 test hits  */
     RG_OPT_OVERLAP = 6,      /* shadow side of a level concurrent with the next level's path side:
                                 0 = automatic (on with the grid tracer), 1 = off, 2 = on */
@@ -149,9 +150,16 @@ enum {
     RG_OPT_SCHEDULE = 11,    /* multi-GPU scenes: 0 = automatic, 1 = static (tile t on device t mod N),
                                 2 = static share + a stealable tail handed out by an atomic tile counter */
     RG_OPT_TILE_ROWS = 12,   /* multi-GPU scenes: rows per tile (default 8) */
-    RG_OPT_ORIGIN_HINTS = 13 /* 1 (default) = every secondary ray carries the outcome of the reference's test against the
+    RG_OPT_ORIGIN_HINTS = 13, /* 1 (default) = every secondary ray carries the outcome of the reference's test against the
                                 sphere it starts on, and the grid tracer skips that test; 0 = off.  Results unchanged
                                 (Scene::trace is a minimum: a body proven to return None may be left out, scene.rs:34-39) */
+    RG_OPT_SUPERSAMPLE = 14  /* n x n primary rays per pixel, box-filtered on the device; 1 (default) ... 8, anything else
+                                is RG_E_INVALID.  A (w x h) frame is the reference's render at (n*w x n*h) reduced n x n:
+                                sample (X, Y) is the f32 Color of create_prime(X, Y, n*w, n*h) (ray.rs:37-54), and per
+                                channel, in f32, s = 0; for j in 0..n, for i in 0..n: s = s + sample(n*x + i, n*y + j);
+                                avg = s / (n*n), rounded to nearest.  The RGBA8 entry points store Color::rgba(avg)
+                                (color.rs:32-37), the f32 ones avg.  Output buffers keep their sizes; the ray and error
+                                counters count every sample's rays.  (n*w)*(n*h) must fit in u32, else RG_E_TOO_LARGE. */
 };
 
 /* Counters and timings of one render call.  A "ray" is one `Scene::trace`

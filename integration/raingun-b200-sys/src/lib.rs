@@ -45,6 +45,7 @@ pub const RG_OPT_TRACE_STATS: i32 = 9;
 pub const RG_OPT_SCHEDULE: i32 = 11;
 pub const RG_OPT_TILE_ROWS: i32 = 12;
 pub const RG_OPT_ORIGIN_HINTS: i32 = 13;
+pub const RG_OPT_SUPERSAMPLE: i32 = 14; // n x n primary rays per pixel (1-8), box-filtered on the device
 
 #[repr(C)]
 pub struct rg_texture_desc {

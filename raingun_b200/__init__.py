@@ -152,6 +152,12 @@ class Scene:
     def set_max_depth_limit(self, limit: int) -> None:
         self.set_option(_native.OPT_MAX_DEPTH, limit)
 
+    def set_supersample(self, n: int) -> None:
+        """Anti-aliasing (RG_OPT_SUPERSAMPLE, 1 <= n <= 8): every render then delivers the reference's frame at
+        n x width by n x height, averaged n x n per pixel in f32 on the GPU, in arrays of unchanged shape.  1 (the
+        default) is the reference's own frame."""
+        self.set_option(_native.OPT_SUPERSAMPLE, n)
+
     # -- Scene::render_image (scene.rs:41-43)
     def render_image(self, width: int, height: int, out: Optional[np.ndarray] = None) -> np.ndarray:
         return self.render_rows(width, height, 0, height, out)

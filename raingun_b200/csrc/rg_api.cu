@@ -93,6 +93,7 @@ void DeviceContext::release() {
     wf.release();
     frame.release();
     rowlist.release();
+    samples.release();
     arena.release();
     if (d_counters) cudaFree(d_counters);
     if (h_counters) cudaFreeHost(h_counters);
@@ -694,6 +695,10 @@ int rg_scene_set_option(rg_scene *sc, int32_t key, int64_t value) {
         case RG_OPT_ORIGIN_HINTS:
             sc->origin_hints = value != 0;
             return RG_OK;
+        case RG_OPT_SUPERSAMPLE:
+            if (value < 1 || value > 8) break;
+            sc->supersample = (uint32_t)value;
+            return RG_OK;
         default: break;
     }
     set_error("bad option key %d / value %lld", key, (long long)value);
@@ -710,21 +715,52 @@ static int check_dims(rg_scene *sc, uint32_t w, uint32_t h, uint32_t y0, uint32_
     if (w < h) { set_error("width %u < height %u: portrait images are not supported (ray.rs:42)", w, h); return RG_E_PORTRAIT; }
     if ((uint64_t)w * h > 0xFFFFFFFFull) { set_error("width*height overflows u32 (rendering.rs:27)"); return RG_E_TOO_LARGE; }
     if (y0 > y1 || y1 > h) { set_error("bad row range [%u, %u) of %u", y0, y1, h); return RG_E_INVALID; }
+    const uint64_t n = sc->supersample;
+    if (n * w * (n * h) > 0xFFFFFFFFull) {
+        set_error("(%llu*width)*(%llu*height) samples overflow u32 (rendering.rs:27, RG_OPT_SUPERSAMPLE)", (unsigned long long)n,
+                  (unsigned long long)n);
+        return RG_E_TOO_LARGE;
+    }
     return RG_OK;
 }
 
 static int mega_render(rg_scene *sc, uint32_t w, uint32_t h, uint32_t y0, uint32_t y1, const uint32_t *d_rows,
                        OutKind kind, uchar4 *d_out, cudaStream_t stream, rg_stats *st) {
     const uint64_t npix = (uint64_t)(y1 - y0) * w;
+    const uint32_t n = sc->supersample;
+    uint32_t launches = 0;
+    int rc;
     RG_CUDA(cudaMemsetAsync(sc->d_counters, 0, sizeof(DCounters), stream));
     RG_CUDA(cudaEventRecord(sc->ev[0], stream));
     if (npix) {
-        const unsigned blocks = (unsigned)((npix + 127) / 128);
-        float *f32 = kind == OutKind::F32 ? reinterpret_cast<float *>(d_out) : nullptr;
         auto kernel = sc->ds.max_depth <= 12 ? k_render_mega<12, false> : k_render_mega<RG_MAX_DEPTH, false>;
         if (sc->ds.n_lights > RG_MAX_LIGHTS) kernel = sc->ds.max_depth <= 12 ? k_render_mega<12, true> : k_render_mega<RG_MAX_DEPTH, true>;
-        kernel<<<blocks, 128, 0, stream>>>(sc->ds, w, h, y0, y1, d_rows, d_out, f32, sc->d_counters);
-        RG_CUDA(cudaGetLastError());
+        if (n == 1) {
+            const unsigned blocks = (unsigned)((npix + 127) / 128);
+            float *f32 = kind == OutKind::F32 ? reinterpret_cast<float *>(d_out) : nullptr;
+            kernel<<<blocks, 128, 0, stream>>>(sc->ds, w, h, y0, y1, d_rows, d_out, f32, sc->d_counters);
+            RG_CUDA(cudaGetLastError());
+            launches = 1;
+        } else {
+            // RG_OPT_SUPERSAMPLE: the kernel renders the (n w x n h) sample image's f32 colours (rows [n y0, n y1), or
+            // entries of the expanded row list) row-major into sc->samples, and launch_resolve averages them.  Bands of
+            // whole output rows keep that scratch within RG_OPT_BATCH_PIXELS samples (default 16M, 192 MB).
+            const uint64_t band_samples = sc->batch_pixels ? sc->batch_pixels : (16ull << 20);
+            const uint64_t row_samples = (uint64_t)n * n * w;   // samples per output row
+            const uint32_t band = (uint32_t)std::max<uint64_t>(1, std::min<uint64_t>(y1 - y0, band_samples / row_samples));
+            if ((rc = sc->samples.reserve((size_t)band * row_samples * 12))) return rc;
+            float *samples = sc->samples.as<float>();
+            for (uint32_t y = y0; y < y1; y += band) {
+                const uint32_t ye = std::min(y + band, y1);
+                const unsigned blocks = (unsigned)(((uint64_t)(ye - y) * row_samples + 127) / 128);
+                kernel<<<blocks, 128, 0, stream>>>(sc->ds, n * w, n * h, n * y, n * ye, d_rows, nullptr, samples, sc->d_counters);
+                RG_CUDA(cudaGetLastError());
+                uint8_t *out = kind == OutKind::Rgba8Scatter ? reinterpret_cast<uint8_t *>(d_out)
+                                                             : reinterpret_cast<uint8_t *>(d_out) + (size_t)(y - y0) * w * bytes_per_pixel(kind);
+                if ((rc = launch_resolve(kind, samples, 3, 1, n, w, ye - y, d_rows, n * y, out, stream))) return rc;
+                launches += 2;
+            }
+        }
     }
     RG_CUDA(cudaEventRecord(sc->ev[1], stream));
     RG_CUDA(cudaMemcpyAsync(sc->h_counters, sc->d_counters, sizeof(DCounters), cudaMemcpyDeviceToHost, stream));
@@ -741,7 +777,7 @@ static int mega_render(rg_scene *sc, uint32_t w, uint32_t h, uint32_t y0, uint32
     st->err_aabb_normal = c.err_aabb;
     st->ms_device = ms;
     st->ms_trace = ms;
-    st->gpu_launches = npix ? 1 : 0;
+    st->gpu_launches = launches;
     st->batches = 1;
     st->accel_used = RG_ACCEL_BRUTE;
     uint64_t rays = c.rays[0] + c.rays[1] + c.rays[2] + c.rays[3];
@@ -786,9 +822,18 @@ int render_rowlist_device(rg_scene *sc, uint32_t w, uint32_t h, const uint32_t *
     for (uint32_t k = 0; k < n_rows; ++k)
         if (rows[k] >= h) { set_error("rows[%u] = %u is outside the image (height %u)", k, rows[k], h); return RG_E_INVALID; }
     RG_CUDA(cudaSetDevice(sc->device));
+    std::vector<uint32_t> sample_rows;   // RG_OPT_SUPERSAMPLE = n > 1: listed row r is sample rows n r, ..., n r + n - 1
+    const uint32_t n = sc->supersample;
+    if (n > 1) {
+        sample_rows.reserve((size_t)n_rows * n);
+        for (uint32_t k = 0; k < n_rows; ++k)
+            for (uint32_t j = 0; j < n; ++j) sample_rows.push_back(n * rows[k] + j);
+        rows = sample_rows.data();
+    }
     if (n_rows) {
-        if ((rc = sc->rowlist.reserve((size_t)n_rows * sizeof(uint32_t)))) return rc;
-        RG_CUDA(cudaMemcpyAsync(sc->rowlist.ptr, rows, (size_t)n_rows * sizeof(uint32_t), cudaMemcpyHostToDevice, stream));
+        const size_t bytes = (size_t)n_rows * n * sizeof(uint32_t);
+        if ((rc = sc->rowlist.reserve(bytes))) return rc;
+        RG_CUDA(cudaMemcpyAsync(sc->rowlist.ptr, rows, bytes, cudaMemcpyHostToDevice, stream));
         RG_CUDA(cudaStreamSynchronize(stream));   // `rows` may be pageable and reused by the caller
     }
     return render_device(sc, w, h, 0, n_rows, sc->rowlist.as<uint32_t>(), kind, d_out, stream, stats);

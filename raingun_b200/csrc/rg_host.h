@@ -88,6 +88,7 @@ struct DeviceContext {
     WavefrontScratch wf;
     DeviceBuffer frame;                // staging of host-buffer renders
     DeviceBuffer rowlist;              // device copy of a caller's row list
+    DeviceBuffer samples;              // megakernel with RG_OPT_SUPERSAMPLE > 1: f32 RGB of a band of samples
     SceneArena arena;                  // scene arrays
     DCounters *d_counters = nullptr;
     DCounters *h_counters = nullptr;   // pinned
@@ -133,6 +134,8 @@ struct rg_scene : rg::DeviceContext {
     int graph = 0;                         // RG_OPT_GRAPH: 0 auto, 1 off, 2 on
     bool trace_stats = false;              // RG_OPT_TRACE_STATS
     bool origin_hints = true;              // RG_OPT_ORIGIN_HINTS
+    uint32_t supersample = 1;              // RG_OPT_SUPERSAMPLE: n x n samples per pixel (a multi-GPU handle keeps a copy
+                                           // for its size checks)
     uint32_t depth_hint = 0;               // levels the ray tree of this scene has been seen to use (0 = unknown)
     uint32_t level_growth = 2;             // wavefront queue of level d holds min(2^d, level_growth) x the batch's pixels;
                                            // doubled when a level outgrows its queue (the frame is then repeated)
@@ -143,9 +146,15 @@ struct rg_scene : rg::DeviceContext {
 
 namespace rg {
 // rg_wavefront.cu
-// rows [y0, y1) of the image, or — when d_rows is given — entries [y0, y1) of that row list
+// rows [y0, y1) of the image, or — when d_rows is given — entries [y0, y1) of that row list.  With
+// RG_OPT_SUPERSAMPLE = n > 1, d_rows is the expanded list of sample rows, n per listed row (render_rowlist_device).
 int wavefront_render(rg_scene *sc, uint32_t width, uint32_t height, uint32_t y0, uint32_t y1,
                      const uint32_t *d_rows, OutKind kind, uchar4 *d_out, cudaStream_t stream, rg_stats *st);
+// RG_OPT_SUPERSAMPLE = n > 1: writes `out_rows` output rows of `width` pixels, each the average of its n x n samples,
+// which are f32 RGB at src + stride * i, i in the order of the level-0 queue with strips of `strip` rows over the
+// batch's n out_rows sample rows (strip 1: row-major).  Scatter: output row r goes to image row d_rows[row0 + r n] / n.
+int launch_resolve(OutKind kind, const float *src, uint32_t stride, uint32_t strip, uint32_t n, uint32_t width, uint32_t out_rows,
+                   const uint32_t *d_rows, uint32_t row0, void *out, cudaStream_t stream);
 // rg_api.cu
 // rg_render_rowlist_device (kind Rgba8) and rg_render_rowlist_scatter (Rgba8Scatter) without the one-render-at-a-time
 // guard (for callers that hold it)

@@ -226,6 +226,7 @@ int multi_set_option(rg_scene *sc, int32_t key, int64_t value) {
         const int rc = rg_scene_set_option(c, key, value);
         if (rc) return rc;
     }
+    if (key == RG_OPT_SUPERSAMPLE) sc->supersample = (uint32_t)value;   // the handle's own size checks (check_dims)
     return RG_OK;
 }
 

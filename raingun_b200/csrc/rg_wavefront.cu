@@ -417,6 +417,56 @@ __global__ void __launch_bounds__(256) k_quantise_scatter(const float4 *__restri
     }
 }
 
+// RG_OPT_SUPERSAMPLE = n > 1: the last kernel of a batch, in place of k_quantise / k_quantise_scatter / k_export_f32.
+// One thread per output pixel averages its n x n samples as include/raingun_b200.h specifies: per channel s = 0, then
+// s + sample in sub-row, sub-column order, then s / (n n) rounded to nearest (a sum without products: nothing for
+// FMA contraction to fuse).  `po` spans the batch's sample rows; sample (X, Y) is f32 RGB at src + stride * po.index(X, Y)
+// (the level-0 nodes: stride 4, queue order; the megakernel's f32 output: stride 3, row-major = strip 1).  Scatter:
+// output row r of the batch is image row rows[row0 + r n] / n (the row list holds n sample rows per listed row).
+template <OutKind K>
+__global__ void __launch_bounds__(256) k_resolve_ss(const float *__restrict__ src, uint32_t stride, const PixelOrder po, uint32_t n,
+                                                    uint32_t npix, const uint32_t *__restrict__ rows, uint32_t row0, void *out) {
+    const uint32_t p = blockIdx.x * blockDim.x + threadIdx.x;
+    if (p >= npix) return;
+    const uint32_t w = po.width / n, r = p / w, x = p - r * w;
+    float s[3] = {0.0f, 0.0f, 0.0f};
+    for (uint32_t j = 0; j < n; ++j)
+        for (uint32_t i = 0; i < n; ++i) {
+            const float *c = src + (size_t)stride * po.index(n * x + i, n * r + j);
+            float v[3];
+            if (stride == 4) { const float4 a = *reinterpret_cast<const float4 *>(c); v[0] = a.x; v[1] = a.y; v[2] = a.z; }
+            else { v[0] = c[0]; v[1] = c[1]; v[2] = c[2]; }
+#pragma unroll
+            for (int k = 0; k < 3; ++k) s[k] = __fadd_rn(s[k], v[k]);
+        }
+    const float nn = (float)(n * n);
+    const C3 avg = c3(__fdiv_rn(s[0], nn), __fdiv_rn(s[1], nn), __fdiv_rn(s[2], nn));
+    if constexpr (K == OutKind::F32) {
+        float *o = static_cast<float *>(out) + 3 * (size_t)p;
+        o[0] = avg.r; o[1] = avg.g; o[2] = avg.b;
+    } else if constexpr (K == OutKind::Rgba8Scatter) {
+        static_cast<uchar4 *>(out)[(size_t)(rows[row0 + r * n] / n) * w + x] = quantise(avg);
+    } else {
+        static_cast<uchar4 *>(out)[p] = quantise(avg);
+    }
+}
+
+int launch_resolve(OutKind kind, const float *src, uint32_t stride, uint32_t strip, uint32_t n, uint32_t width, uint32_t out_rows,
+                   const uint32_t *d_rows, uint32_t row0, void *out, cudaStream_t stream) {
+    const uint32_t npix = out_rows * width;
+    if (npix == 0) return RG_OK;
+    PixelOrder po;
+    po.width = n * width;
+    po.rows = n * out_rows;
+    po.strip = strip;
+    const unsigned blocks = (npix + 255) / 256;
+    if (kind == OutKind::F32) k_resolve_ss<OutKind::F32><<<blocks, 256, 0, stream>>>(src, stride, po, n, npix, d_rows, row0, out);
+    else if (kind == OutKind::Rgba8Scatter) k_resolve_ss<OutKind::Rgba8Scatter><<<blocks, 256, 0, stream>>>(src, stride, po, n, npix, d_rows, row0, out);
+    else k_resolve_ss<OutKind::Rgba8><<<blocks, 256, 0, stream>>>(src, stride, po, n, npix, d_rows, row0, out);
+    RG_CUDA(cudaGetLastError());
+    return RG_OK;
+}
+
 // RG_OPT_VERIFY_CULL >= 2: re-trace every ray of a queue with the verbatim reference scan and
 // count results that differ from what the production trace kernel wrote (must be 0).
 template <bool ANY>
@@ -805,7 +855,12 @@ static int enqueue_batch_dev(rg_scene *sc, const DevPlan &plan, uint32_t width, 
         RG_CUDA(cudaGetLastError());
         st->gpu_launches++;
     }
-    if (kind == OutKind::F32)
+    if (sc->supersample > 1) {   // width, height, y0 and npix are in sample space: npix / (n n) output pixels
+        const uint32_t n = sc->supersample;
+        if ((rc = launch_resolve(kind, reinterpret_cast<const float *>(wf.nodes[0].as<float4>()), 4, po.strip, n, width / n,
+                                 po.rows / n, d_rows, y0, d_out, stream)))
+            return rc;
+    } else if (kind == OutKind::F32)
         k_export_f32<<<(npix + 255) / 256, 256, 0, stream>>>(wf.nodes[0].as<float4>(), reinterpret_cast<float *>(d_out), npix, po);
     else if (kind == OutKind::Rgba8Scatter)
         k_quantise_scatter<<<(unsigned)((((uint64_t)npix + 3) / 4 + 255) / 256), 256, 0, stream>>>(wf.nodes[0].as<float4>(), d_out, npix, d_rows, y0, po);
@@ -824,7 +879,8 @@ static std::vector<uint64_t> graph_key(const rg_scene *sc, const DevPlan &plan, 
     std::vector<uint64_t> k = {width, height, y0, npix, (uint64_t)(uintptr_t)d_rows, (uint64_t)(uintptr_t)d_out,
                                (uint64_t)use_grid, (uint64_t)kind, (uint64_t)sc->ds.max_depth, (uint64_t)sc->overlap,
                                (uint64_t)sc->verify_cull, (uint64_t)sc->trace_stats | ((uint64_t)sc->origin_hints << 1), (uint64_t)plan.levels,
-                               (uint64_t)sc->level_growth};   // the capacities are baked into the captured launches
+                               (uint64_t)sc->level_growth,    // the capacities are baked into the captured launches
+                               (uint64_t)sc->supersample};    // the last launch: (n, w, h) and (1, n w, n h) share a sample space
     auto add = [&](const DeviceBuffer &b) { k.push_back((uint64_t)(uintptr_t)b.ptr); };
     add(wf.ray[0]); add(wf.ray[1]); add(wf.hit_t); add(wf.hit_body);
     for (int p = 0; p < 2; ++p) { add(wf.sray[p]); add(wf.s_tmax[p]); add(wf.s_ab[p]); add(wf.s_lit[p]); add(wf.lit_bc[p]); add(wf.lit_node[p]); }
@@ -910,9 +966,12 @@ int wavefront_render(rg_scene *sc, uint32_t width, uint32_t height, uint32_t y0,
     EventPool events(sc->wf.events);
     EventPool sync_events(sc->wf.sync_events, cudaEventDisableTiming);
     std::vector<std::pair<cudaEvent_t, cudaEvent_t>> trace_spans;
+    // RG_OPT_SUPERSAMPLE: the batches trace the (n width x n height) sample image, output row y being sample rows
+    // [n y, n y + n) (or, with a row list, entries [n k, n k + n) of the expanded list); batches are cut in whole output rows.
+    const uint32_t n = sc->supersample, sw = n * width, sh = n * height;
     const uint32_t rows = y1 - y0;
     const uint64_t batch_pixels = sc->batch_pixels ? sc->batch_pixels : (16ull << 20);
-    uint32_t batch_rows = (uint32_t)std::max<uint64_t>(1, std::min<uint64_t>(rows ? rows : 1, batch_pixels / width));
+    uint32_t batch_rows = (uint32_t)std::max<uint64_t>(1, std::min<uint64_t>(rows ? rows : 1, batch_pixels / ((uint64_t)n * sw)));
     const rg_stats st0 = *st;
     for (;;) {   // a ray tree larger than device memory restarts the render with half the rows per batch
         *st = st0;
@@ -930,14 +989,14 @@ int wavefront_render(rg_scene *sc, uint32_t width, uint32_t height, uint32_t y0,
             uchar4 *out = kind == OutKind::Rgba8Scatter ? d_out
                         : reinterpret_cast<uchar4 *>(reinterpret_cast<unsigned char *>(d_out) + (size_t)(y - y0) * width * bytes_per_pixel(kind));
             DevPlan plan;
-            const uint64_t npix64 = (uint64_t)(ye - y) * width;
+            const uint64_t npix64 = (uint64_t)(ye - y) * n * sw;
             if (npix64 > 0x7FFFFFFFull) { set_error("batch of %llu pixels is too large", (unsigned long long)npix64); rc = RG_E_NOMEM; }
             else if (npix64 && (rc = plan_batch_dev(sc, (uint32_t)npix64, plan, use_grid)) == RG_OK) {
                 bool done = false;
                 if (sc->graph != 1 && sc->verify_cull == 0)
-                    rc = graph_batch(sc, plan, width, height, y, (uint32_t)npix64, d_rows, kind, out, stream, st, use_grid, sync_events, &done);
+                    rc = graph_batch(sc, plan, sw, sh, n * y, (uint32_t)npix64, d_rows, kind, out, stream, st, use_grid, sync_events, &done);
                 if (rc == RG_OK && !done)
-                    rc = enqueue_batch_dev(sc, plan, width, height, y, (uint32_t)npix64, d_rows, kind, out, stream, st, use_grid, &events,
+                    rc = enqueue_batch_dev(sc, plan, sw, sh, n * y, (uint32_t)npix64, d_rows, kind, out, stream, st, use_grid, &events,
                                            sync_events, &trace_spans);
             }
             y = ye;
