@@ -206,10 +206,14 @@ k_trace_brute(const DScene s, const TraceArgs a) {
     static_assert(kCullPad % U == 0 && U <= kCullPad, "records are padded to kCullPad");
     __shared__ __align__(128) float4 stage[2][kChunkSpheres + 3 * kCullPad];   // + slack for the prefetch (two groups ahead)
     __shared__ uint64_t mbar[2];
-    __shared__ uint32_t cq[kTraceWarps][64];
+    // The candidate queue keeps the full 32-bit sphere index beside a 16-bit ray slot: a packed
+    // (sph << kSlotBits | slot) word, as the resident kernel uses, would lose the top bits of sphere
+    // indices >= 2^22.  (Static shared memory is at its 48 KB limit at R = 4: the slots take the
+    // place of the per-ray tag array the drain no longer needs.)
+    __shared__ uint32_t cq_sph[kTraceWarps][64];
+    __shared__ uint16_t cq_slot[kTraceWarps][64];
     __shared__ double best_t[R * kTraceThreads];
     __shared__ uint32_t best_b[R * kTraceThreads];   // nearest: body; ANY: 1 = occluded
-    __shared__ uint8_t tag[R * kTraceThreads];
 
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     const uint32_t block_base = blockIdx.x * (uint32_t)(R * kTraceThreads);
@@ -271,18 +275,17 @@ k_trace_brute(const DScene s, const TraceArgs a) {
         best_t[slot] = best.t;
         best_b[slot] = ANY ? (occluded ? 1u : 0u) : best.body;
     }
-    uint32_t qn = 0;   // warp-uniform: candidates waiting in cq[warp]
+    uint32_t qn = 0;   // warp-uniform: candidates waiting in cq_*[warp]
 
-    // Evaluates candidates cq[warp][first .. first+count) — one per lane — exactly.
+    // Evaluates candidates cq_*[warp][first .. first+count) — one per lane — exactly.
     auto drain = [&](uint32_t first, uint32_t count) {
         bool have = (uint32_t)lane < count;
         uint32_t slot = 0, sph = 0;
         bool hit = false;
         double t = 0.0;
         if (have) {
-            uint32_t e = cq[warp][first + lane];
-            slot = e & ((1u << kSlotBits) - 1u);
-            sph = e >> kSlotBits;
+            slot = cq_slot[warp][first + lane];
+            sph = cq_sph[warp][first + lane];
             Ray ray = load_ray(a.q, phys_index(seg_len, a.seg_stride, block_base + slot));
             double4 sp = s.sph[sph];
             hit = sphere_intersect(sp.x, sp.y, sp.z, sp.w, ray, t);
@@ -296,11 +299,13 @@ k_trace_brute(const DScene s, const TraceArgs a) {
             if (hit && t <= a.tmax[phys_index(seg_len, a.seg_stride, block_base + slot)]) best_b[slot] = 1u;   // benign race: all write 1
         } else {
             const uint32_t body = hit ? s.sph_body[sph] : 0u;
+            // serialise hits on the same ray: the k-th of them (in lane order) offers in round k
+            // (slot < 2^16, so a lane without a hit never shares the key of one with a hit)
+            const uint32_t peers = __match_any_sync(0xffffffffu, hit ? slot : 0xFFFFFFFFu);
+            const uint32_t rank = __popc(peers & lanemask_lt);
             bool pend = hit;
-            while (__any_sync(0xffffffffu, pend)) {      // serialise candidates of the same ray
-                if (pend) tag[slot] = (uint8_t)lane;
-                __syncwarp();
-                if (pend && tag[slot] == (uint8_t)lane) {
+            for (uint32_t k = 0; __any_sync(0xffffffffu, pend); ++k) {
+                if (pend && rank == k) {
                     Nearest cur;
                     cur.t = best_t[slot];
                     cur.body = best_b[slot];
@@ -349,7 +354,11 @@ k_trace_brute(const DScene s, const TraceArgs a) {
                     }
                     const uint32_t mask = __ballot_sync(0xffffffffu, pass);
                     if (mask) {
-                        if (pass) cq[warp][qn + __popc(mask & lanemask_lt)] = (sph << kSlotBits) | slot;
+                        if (pass) {
+                            const uint32_t at = qn + __popc(mask & lanemask_lt);
+                            cq_sph[warp][at] = sph;
+                            cq_slot[warp][at] = (uint16_t)slot;
+                        }
                         qn += __popc(mask);
                         __syncwarp();
                         if (qn >= 32u) {
@@ -367,7 +376,11 @@ k_trace_brute(const DScene s, const TraceArgs a) {
         auto enqueue = [&](bool pass, uint32_t sph, uint32_t slot) {
             const uint32_t mask = __ballot_sync(0xffffffffu, pass);
             if (mask) {
-                if (pass) cq[warp][qn + __popc(mask & lanemask_lt)] = (sph << kSlotBits) | slot;
+                if (pass) {
+                    const uint32_t at = qn + __popc(mask & lanemask_lt);
+                    cq_sph[warp][at] = sph;
+                    cq_slot[warp][at] = (uint16_t)slot;
+                }
                 qn += __popc(mask);
                 __syncwarp();
                 if (qn >= 32u) {

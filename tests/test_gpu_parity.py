@@ -20,12 +20,18 @@ MODES = [
 ]
 
 
-def _render(data, w, h, pipeline, accel, verify=False):
+# The brute-force tracer twice: RG_OPT_VERIFY_CULL=1 runs its debug loop, which re-tests every culled pair exactly
+# (cull soundness); =2 runs the shipped FFMA2 loop and then re-traces every queued ray with the verbatim FP64 scan.
+CULL_MODES = MODES[:2] + [("wavefront-brute-shipped", rg.PIPELINE_WAVEFRONT, rg.ACCEL_BRUTE)] + MODES[2:]
+VERIFY = {"wavefront-brute": 1, "wavefront-brute-shipped": 2}
+
+
+def _render(data, w, h, pipeline, accel, verify=0):
     with rg.Scene(data) as sc:
         sc.set_pipeline(pipeline)
         sc.set_accel(accel)
         if verify:
-            sc.set_option(rg._native.OPT_VERIFY_CULL, 1)
+            sc.set_option(rg._native.OPT_VERIFY_CULL, int(verify))
         img = sc.render_image(w, h)
         return img, sc.last_stats
 
@@ -63,7 +69,7 @@ def test_examples_match_reference_png(name):
 SYNTH = [("C3", 300, 4, 320, 180), ("C4", 400, 8, 256, 144), ("C5", 500, 6, 192, 108)]
 
 
-@pytest.mark.parametrize("mode", MODES, ids=[m[0] for m in MODES])
+@pytest.mark.parametrize("mode", CULL_MODES, ids=[m[0] for m in CULL_MODES])
 @pytest.mark.parametrize("cfg", SYNTH, ids=[c[0] for c in SYNTH])
 def test_synthetic_match_oracle(oracle, cfg, mode):
     """configs[2..4] shrunk (same generator stream, fewer spheres / pixels) so the CPU oracle
@@ -71,7 +77,7 @@ def test_synthetic_match_oracle(oracle, cfg, mode):
     name, spheres, depth, w, h = cfg
     data, _ = make_scene(name, spheres=spheres, depth=depth, texture_loader=bundled_texture_loader)
     ref, ost, _ = oracle.render(data, w, h)
-    img, st = _render(data, w, h, mode[1], mode[2], verify=(mode[0] == "wavefront-brute"))
+    img, st = _render(data, w, h, mode[1], mode[2], verify=VERIFY.get(mode[0], 0))
     _assert_same(img, ref, st, ost, f"{name}/{mode[0]}")
     assert st.cull_unsound == 0
 
@@ -327,8 +333,8 @@ def test_non_unit_directions_and_unnormalised_normals(oracle):
     doc["bodies"][0]["Plane"]["material"]["surface"] = {"Reflecting": {"reflectivity": 0.6}}
     data = scene_from_dict(doc)
     ref, ost, _ = oracle.render(data, 240, 135)
-    for mode in MODES:
-        img, st = _render(data, 240, 135, mode[1], mode[2], verify=(mode[0] == "wavefront-brute"))
+    for mode in CULL_MODES:
+        img, st = _render(data, 240, 135, mode[1], mode[2], verify=VERIFY.get(mode[0], 0))
         _assert_same(img, ref, st, ost, mode[0])
         assert st.cull_unsound == 0
 
@@ -457,13 +463,15 @@ def test_origin_hints_change_no_pixel_and_spare_the_exact_tests():
 def test_resident_brute_kernel_cull_is_sound_at_scale():
     """The shared-memory-resident brute-force kernel (queues of >= 300 k rays, scenes of <= ~11,000
     spheres) with RG_OPT_VERIFY_CULL=1: every pair the FP32 cull rejects is re-tested exactly on the
-    device and must miss; the image must equal the grid tracer's."""
+    device and must miss; and with RG_OPT_VERIFY_CULL=2: the shipped loop's result for every ray must
+    equal the verbatim scan's.  Both images must equal the grid tracer's."""
     data, _ = make_scene("C3")
     w, h = 1920, 1080
-    img, st = _render(data, w, h, rg.PIPELINE_WAVEFRONT, rg.ACCEL_BRUTE, verify=True)
-    assert st.cull_unsound == 0 and st.rays_primary == w * h
     ref, rst = _render(data, w, h, rg.PIPELINE_WAVEFRONT, rg.ACCEL_GRID)
-    assert np.array_equal(img, ref) and st.rays == rst.rays
+    for verify in (1, 2):
+        img, st = _render(data, w, h, rg.PIPELINE_WAVEFRONT, rg.ACCEL_BRUTE, verify=verify)
+        assert st.cull_unsound == 0 and st.rays_primary == w * h, verify
+        assert np.array_equal(img, ref) and st.rays == rst.rays, verify
 
 
 def test_full_size_c5_row_matches_oracle(oracle):
@@ -648,8 +656,8 @@ def test_adversarial_geometry_matches_oracle(oracle, case):
     data = scene_from_dict(doc, bundled_texture_loader)
     w, h = 224, 126
     ref, ost, _ = oracle.render(data, w, h)
-    for mode in MODES:
-        img, st = _render(data, w, h, mode[1], mode[2], verify=(mode[0] == "wavefront-brute"))
+    for mode in CULL_MODES:
+        img, st = _render(data, w, h, mode[1], mode[2], verify=VERIFY.get(mode[0], 0))
         _assert_same(img, ref, st, ost, f"{name}/{mode[0]}")
         assert st.cull_unsound == 0
 
