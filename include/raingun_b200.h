@@ -318,6 +318,21 @@ int rg_render_rows_f32(rg_scene *scene, uint32_t width, uint32_t height,
 int rg_render_stream_f32(rg_scene *scene, uint32_t width, uint32_t height,
                          uint32_t band_rows, rg_rows_f32_cb cb, void *user, rg_stats *stats);
 
+/* The f32 twins of rg_render_rows_device, rg_render_rowlist_device, rg_render_rowlist_scatter and
+ * rg_render_rowlist_host: the same rows, destinations, streams, checks, refusals and stats, with 3 floats
+ * (12 bytes) per pixel holding the bits rg_render_rows_f32 delivers for the same pixels.  The scatter and
+ * host forms store row rows[k] at `d_frame` / `frame` + rows[k]*width*3 floats of a full width*height*3
+ * frame; the scatter form needs the wavefront pipeline and writes 128-bit stores when width % 4 == 0 and
+ * the frame is 16-byte aligned.  Single-device scenes. */
+int rg_render_rows_f32_device(rg_scene *scene, uint32_t width, uint32_t height, uint32_t y0, uint32_t y1,
+                              float *d_rgb_out, void *cuda_stream, rg_stats *stats);
+int rg_render_rowlist_f32_device(rg_scene *scene, uint32_t width, uint32_t height, const uint32_t *rows,
+                                 uint32_t n_rows, float *d_rgb_out, void *cuda_stream, rg_stats *stats);
+int rg_render_rowlist_f32_scatter(rg_scene *scene, uint32_t width, uint32_t height, const uint32_t *rows,
+                                  uint32_t n_rows, float *d_frame, void *cuda_stream, rg_stats *stats);
+int rg_render_rowlist_f32_host(rg_scene *scene, uint32_t width, uint32_t height, const uint32_t *rows,
+                               uint32_t n_rows, float *frame, rg_stats *stats);
+
 /* Thread-local description of the last failure in this thread. */
 const char *rg_last_error(void);
 

@@ -158,6 +158,17 @@ extern "C" {
                               rgb_out: *mut f32, stats: *mut rg_stats) -> c_int;
     pub fn rg_render_stream_f32(scene: *mut rg_scene, width: u32, height: u32, band_rows: u32,
                                 cb: rg_rows_f32_cb, user: *mut c_void, stats: *mut rg_stats) -> c_int;
+    pub fn rg_render_rows_f32_device(scene: *mut rg_scene, width: u32, height: u32, y0: u32, y1: u32,
+                                     d_rgb_out: *mut f32, cuda_stream: *mut c_void,
+                                     stats: *mut rg_stats) -> c_int;
+    pub fn rg_render_rowlist_f32_device(scene: *mut rg_scene, width: u32, height: u32, rows: *const u32,
+                                        n_rows: u32, d_rgb_out: *mut f32, cuda_stream: *mut c_void,
+                                        stats: *mut rg_stats) -> c_int;
+    pub fn rg_render_rowlist_f32_scatter(scene: *mut rg_scene, width: u32, height: u32, rows: *const u32,
+                                         n_rows: u32, d_frame: *mut f32, cuda_stream: *mut c_void,
+                                         stats: *mut rg_stats) -> c_int;
+    pub fn rg_render_rowlist_f32_host(scene: *mut rg_scene, width: u32, height: u32, rows: *const u32,
+                                      n_rows: u32, frame: *mut f32, stats: *mut rg_stats) -> c_int;
     pub fn rg_trim() -> c_int;
     pub fn rg_last_error() -> *const c_char;
     pub fn rg_measure_peaks(device: i32, fp32_tflops: *mut f64, fp64_tflops: *mut f64,

@@ -198,6 +198,15 @@ class Scene:
         self.last_stats = st
         return st
 
+    def render_rows_f32_device(self, width: int, height: int, y0: int, y1: int, device_ptr: int,
+                               cuda_stream: int = 0) -> Stats:
+        """``render_rows_device`` with the unquantised f32 colours: (y1-y0)*width*3 floats in HBM at ``device_ptr``."""
+        st = Stats()
+        _native.check(_native.lib().rg_render_rows_f32_device(self._h, width, height, y0, y1, ctypes.c_void_p(device_ptr),
+                                                              ctypes.c_void_p(cuda_stream), ctypes.byref(st)))
+        self.last_stats = st
+        return st
+
     def render_rowlist_device(self, width: int, height: int, rows, device_ptr: int, cuda_stream: int = 0) -> Stats:
         """Row-tile sharding unit: renders the listed image rows, compacted in list order, into
         HBM at ``device_ptr`` (len(rows)*width*4 bytes)."""
@@ -210,6 +219,22 @@ class Scene:
         frame fused into the last kernel."""
         return self._render_rowlist(_native.lib().rg_render_rowlist_scatter, width, height, rows, frame_ptr,
                                     ctypes.c_void_p(cuda_stream))
+
+    def render_rowlist_f32_device(self, width: int, height: int, rows, device_ptr: int, cuda_stream: int = 0) -> Stats:
+        """``render_rowlist_device`` with f32 colours: len(rows)*width*3 floats, compacted in list order."""
+        return self._render_rowlist(_native.lib().rg_render_rowlist_f32_device, width, height, rows, device_ptr,
+                                    ctypes.c_void_p(cuda_stream))
+
+    def render_rowlist_f32_scatter(self, width: int, height: int, rows, frame_ptr: int, cuda_stream: int = 0) -> Stats:
+        """``render_rowlist_scatter`` with f32 colours: row ``rows[k]`` lands at ``frame_ptr + rows[k]*width*12`` bytes
+        of a full width*height*3 float frame (device memory, possibly another GPU's, or pinned host memory)."""
+        return self._render_rowlist(_native.lib().rg_render_rowlist_f32_scatter, width, height, rows, frame_ptr,
+                                    ctypes.c_void_p(cuda_stream))
+
+    def render_rowlist_f32_host(self, width: int, height: int, rows, frame_ptr: int) -> Stats:
+        """``render_rowlist_host`` with f32 colours: row ``rows[k]`` is copied to ``frame_ptr + rows[k]*width*12`` bytes
+        of a full width*height*3 float frame in HOST memory."""
+        return self._render_rowlist(_native.lib().rg_render_rowlist_f32_host, width, height, rows, frame_ptr)
 
     def render_rows_f32(self, width: int, height: int, y0: int = 0, y1: Optional[int] = None) -> np.ndarray:
         """The unquantised f32 colours (``RenderedPixel.color``, rendering.rs:18-22): (rows, width, 3) float32."""

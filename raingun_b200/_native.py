@@ -37,7 +37,8 @@ ROWS_F32_CB = ctypes.CFUNCTYPE(ctypes.c_int, ctypes.c_uint32, ctypes.c_uint32, c
 # every symbol include/raingun_b200.h declares
 EXPORTS = ("rg_scene_create", "rg_scene_create_multi", "rg_scene_device_count", "rg_scene_destroy", "rg_scene_set_option", "rg_render", "rg_render_rows",
            "rg_render_rows_device", "rg_render_rowlist_device", "rg_render_rowlist_scatter", "rg_render_rowlist_host", "rg_host_register", "rg_host_unregister", "rg_device_enable_peer", "rg_shm_barrier_open", "rg_shm_barrier_wait", "rg_shm_barrier_close", "rg_shared_frame_create",
-           "rg_shared_frame_open", "rg_shared_frame_close", "rg_render_stream", "rg_render_rows_f32", "rg_render_stream_f32", "rg_trim", "rg_last_error", "rg_measure_peaks",
+           "rg_shared_frame_open", "rg_shared_frame_close", "rg_render_stream", "rg_render_rows_f32", "rg_render_stream_f32",
+           "rg_render_rows_f32_device", "rg_render_rowlist_f32_device", "rg_render_rowlist_f32_scatter", "rg_render_rowlist_f32_host", "rg_trim", "rg_last_error", "rg_measure_peaks",
            "rg_device_count")
 IPC_HANDLE_BYTES = 64
 
@@ -106,6 +107,14 @@ def lib() -> ctypes.CDLL:
     L.rg_render_rows_f32.argtypes = [vp, u32, u32, u32, u32, vp, ctypes.POINTER(Stats)]
     L.rg_render_stream_f32.restype = ctypes.c_int
     L.rg_render_stream_f32.argtypes = [vp, u32, u32, u32, ROWS_F32_CB, vp, ctypes.POINTER(Stats)]
+    L.rg_render_rows_f32_device.restype = ctypes.c_int
+    L.rg_render_rows_f32_device.argtypes = [vp, u32, u32, u32, u32, vp, vp, ctypes.POINTER(Stats)]
+    L.rg_render_rowlist_f32_device.restype = ctypes.c_int
+    L.rg_render_rowlist_f32_device.argtypes = [vp, u32, u32, vp, u32, vp, vp, ctypes.POINTER(Stats)]
+    L.rg_render_rowlist_f32_scatter.restype = ctypes.c_int
+    L.rg_render_rowlist_f32_scatter.argtypes = [vp, u32, u32, vp, u32, vp, vp, ctypes.POINTER(Stats)]
+    L.rg_render_rowlist_f32_host.restype = ctypes.c_int
+    L.rg_render_rowlist_f32_host.argtypes = [vp, u32, u32, vp, u32, vp, ctypes.POINTER(Stats)]
     L.rg_trim.restype = ctypes.c_int
     L.rg_trim.argtypes = []
     L.rg_last_error.restype = ctypes.c_char_p

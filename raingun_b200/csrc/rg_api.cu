@@ -755,7 +755,7 @@ static int mega_render(rg_scene *sc, uint32_t w, uint32_t h, uint32_t y0, uint32
                 const unsigned blocks = (unsigned)(((uint64_t)(ye - y) * row_samples + 127) / 128);
                 kernel<<<blocks, 128, 0, stream>>>(sc->ds, n * w, n * h, n * y, n * ye, d_rows, nullptr, samples, sc->d_counters);
                 RG_CUDA(cudaGetLastError());
-                uint8_t *out = kind == OutKind::Rgba8Scatter ? reinterpret_cast<uint8_t *>(d_out)
+                uint8_t *out = is_scatter(kind) ? reinterpret_cast<uint8_t *>(d_out)
                                                              : reinterpret_cast<uint8_t *>(d_out) + (size_t)(y - y0) * w * bytes_per_pixel(kind);
                 if ((rc = launch_resolve(kind, samples, 3, 1, n, w, ye - y, d_rows, n * y, out, stream))) return rc;
                 launches += 2;
@@ -798,7 +798,7 @@ static int render_device(rg_scene *sc, uint32_t w, uint32_t h, uint32_t y0, uint
     // the crossover lies near kMegaAutoBodies bodies (RG_MEGA_AUTO_BODIES for tuning runs)
     static const uint32_t mega_auto_bodies = [] { const char *e = getenv("RG_MEGA_AUTO_BODIES"); return e ? (uint32_t)atoi(e) : kMegaAutoBodies; }();
     const bool mega = sc->pipeline == RG_PIPELINE_MEGAKERNEL ||
-                      (sc->pipeline == RG_PIPELINE_AUTO && kind != OutKind::Rgba8Scatter && sc->n_bodies <= mega_auto_bodies && sc->verify_cull == 0);
+                      (sc->pipeline == RG_PIPELINE_AUTO && !is_scatter(kind) && sc->n_bodies <= mega_auto_bodies && sc->verify_cull == 0);
     if (mega) rc = mega_render(sc, w, h, y0, y1, d_rows, kind, (uchar4 *)d_out, stream, &local);
     else rc = wavefront_render(sc, w, h, y0, y1, d_rows, kind, (uchar4 *)d_out, stream, &local);
     local.pipeline_used = mega ? RG_PIPELINE_MEGAKERNEL : RG_PIPELINE_WAVEFRONT;
@@ -987,14 +987,36 @@ struct BusyGuard {
 };
 #define RG_ENTER(sc) BusyGuard _guard(sc); if (!_guard.ok) return RG_E_BUSY
 
-int rg_render_rows_device(rg_scene *sc, uint32_t w, uint32_t h, uint32_t y0, uint32_t y1, void *d_rgba_out, void *cuda_stream, rg_stats *stats) {
-    RG_ENTER(sc);
+// rg_render_rows_device (kind Rgba8) and rg_render_rows_f32_device (F32), inside the one-render-at-a-time guard
+static int render_rows_device(rg_scene *sc, uint32_t w, uint32_t h, uint32_t y0, uint32_t y1, OutKind kind, void *d_out,
+                              void *cuda_stream, rg_stats *stats) {
     int rc = check_dims(sc, w, h, y0, y1);
     if (rc) return rc;
     if ((rc = single_device_only(sc, "rg_render_rows_device"))) return rc;
-    if (!d_rgba_out && y1 > y0) { set_error("output pointer is NULL"); return RG_E_INVALID; }
+    if (!d_out && y1 > y0) { set_error("output pointer is NULL"); return RG_E_INVALID; }
     RG_CUDA(cudaSetDevice(sc->device));
-    return render_device(sc, w, h, y0, y1, nullptr, OutKind::Rgba8, d_rgba_out, reinterpret_cast<cudaStream_t>(cuda_stream), stats);
+    return render_device(sc, w, h, y0, y1, nullptr, kind, d_out, reinterpret_cast<cudaStream_t>(cuda_stream), stats);
+}
+// rg_render_rowlist_scatter (kind Rgba8Scatter) and rg_render_rowlist_f32_scatter (F32Scatter), inside the guard
+static int render_rowlist_scatter(rg_scene *sc, uint32_t w, uint32_t h, const uint32_t *rows, uint32_t n_rows, OutKind kind,
+                                  void *d_frame, void *cuda_stream, rg_stats *stats) {
+    if (sc && sc->pipeline == RG_PIPELINE_MEGAKERNEL) { set_error("rg_render_rowlist_scatter needs the wavefront pipeline"); return RG_E_INVALID; }
+    return render_rowlist_device(sc, w, h, rows, n_rows, kind, d_frame, reinterpret_cast<cudaStream_t>(cuda_stream), stats);
+}
+// rg_render_rowlist_host (kind Rgba8) and rg_render_rowlist_f32_host (F32), inside the guard
+static int render_rowlist_host(rg_scene *sc, uint32_t w, uint32_t h, const uint32_t *rows, uint32_t n_rows, OutKind kind, void *frame,
+                               rg_stats *stats) {
+    int rc = check_dims(sc, w, h, 0, h);
+    if (rc) return rc;
+    if ((rc = single_device_only(sc, "rg_render_rowlist_host"))) return rc;
+    if (n_rows && (!rows || !frame)) { set_error("rows / frame pointer is NULL"); return RG_E_INVALID; }
+    RG_CUDA(cudaSetDevice(sc->device));
+    return render_rowlist_to_host(sc, w, h, rows, n_rows, kind, static_cast<uint8_t *>(frame), stats);
+}
+
+int rg_render_rows_device(rg_scene *sc, uint32_t w, uint32_t h, uint32_t y0, uint32_t y1, void *d_rgba_out, void *cuda_stream, rg_stats *stats) {
+    RG_ENTER(sc);
+    return render_rows_device(sc, w, h, y0, y1, OutKind::Rgba8, d_rgba_out, cuda_stream, stats);
 }
 int rg_render_rowlist_device(rg_scene *sc, uint32_t w, uint32_t h, const uint32_t *rows, uint32_t n_rows, void *d_rgba_out, void *cuda_stream, rg_stats *stats) {
     RG_ENTER(sc);
@@ -1002,8 +1024,7 @@ int rg_render_rowlist_device(rg_scene *sc, uint32_t w, uint32_t h, const uint32_
 }
 int rg_render_rowlist_scatter(rg_scene *sc, uint32_t w, uint32_t h, const uint32_t *rows, uint32_t n_rows, void *d_frame, void *cuda_stream, rg_stats *stats) {
     RG_ENTER(sc);
-    if (sc && sc->pipeline == RG_PIPELINE_MEGAKERNEL) { set_error("rg_render_rowlist_scatter needs the wavefront pipeline"); return RG_E_INVALID; }
-    return render_rowlist_device(sc, w, h, rows, n_rows, OutKind::Rgba8Scatter, d_frame, reinterpret_cast<cudaStream_t>(cuda_stream), stats);
+    return render_rowlist_scatter(sc, w, h, rows, n_rows, OutKind::Rgba8Scatter, d_frame, cuda_stream, stats);
 }
 int rg_render_rows(rg_scene *sc, uint32_t w, uint32_t h, uint32_t y0, uint32_t y1, uint8_t *rgba_out, rg_stats *stats) {
     RG_ENTER(sc);
@@ -1027,15 +1048,30 @@ int rg_render_stream_f32(rg_scene *sc, uint32_t w, uint32_t h, uint32_t band_row
     RG_ENTER(sc);
     return render_bands(sc, w, h, band_rows, cb, user, stats);
 }
+// the f32 twins of the device-memory and row-list entry points: 3 floats per pixel, the bits rg_render_rows_f32 delivers
+int rg_render_rows_f32_device(rg_scene *sc, uint32_t w, uint32_t h, uint32_t y0, uint32_t y1, float *d_rgb_out, void *cuda_stream,
+                              rg_stats *stats) {
+    RG_ENTER(sc);
+    return render_rows_device(sc, w, h, y0, y1, OutKind::F32, d_rgb_out, cuda_stream, stats);
+}
+int rg_render_rowlist_f32_device(rg_scene *sc, uint32_t w, uint32_t h, const uint32_t *rows, uint32_t n_rows, float *d_rgb_out,
+                                 void *cuda_stream, rg_stats *stats) {
+    RG_ENTER(sc);
+    return render_rowlist_device(sc, w, h, rows, n_rows, OutKind::F32, d_rgb_out, reinterpret_cast<cudaStream_t>(cuda_stream), stats);
+}
+int rg_render_rowlist_f32_scatter(rg_scene *sc, uint32_t w, uint32_t h, const uint32_t *rows, uint32_t n_rows, float *d_frame,
+                                  void *cuda_stream, rg_stats *stats) {
+    RG_ENTER(sc);
+    return render_rowlist_scatter(sc, w, h, rows, n_rows, OutKind::F32Scatter, d_frame, cuda_stream, stats);
+}
 
 int rg_render_rowlist_host(rg_scene *sc, uint32_t w, uint32_t h, const uint32_t *rows, uint32_t n_rows, uint8_t *frame, rg_stats *stats) {
     RG_ENTER(sc);
-    int rc = check_dims(sc, w, h, 0, h);
-    if (rc) return rc;
-    if ((rc = single_device_only(sc, "rg_render_rowlist_host"))) return rc;
-    if (n_rows && (!rows || !frame)) { set_error("rows / frame pointer is NULL"); return RG_E_INVALID; }
-    RG_CUDA(cudaSetDevice(sc->device));
-    return render_rowlist_to_host(sc, w, h, rows, n_rows, frame, stats);
+    return render_rowlist_host(sc, w, h, rows, n_rows, OutKind::Rgba8, frame, stats);
+}
+int rg_render_rowlist_f32_host(rg_scene *sc, uint32_t w, uint32_t h, const uint32_t *rows, uint32_t n_rows, float *frame, rg_stats *stats) {
+    RG_ENTER(sc);
+    return render_rowlist_host(sc, w, h, rows, n_rows, OutKind::F32, frame, stats);
 }
 
 int rg_trim(void) { return (int)trim_parked(-1); }

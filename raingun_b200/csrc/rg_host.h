@@ -102,9 +102,12 @@ struct DeviceContext {
 };
 
 // What a render call delivers: RGBA8 rows in order, RGBA8 rows stored at their place in a full frame
-// (rg_render_rowlist_scatter), or unquantised f32 RGB (rg_render_rows_f32).
-enum class OutKind { Rgba8, Rgba8Scatter, F32 };
-constexpr size_t bytes_per_pixel(OutKind k) { return k == OutKind::F32 ? 12 : 4; }
+// (rg_render_rowlist_scatter), unquantised f32 RGB rows in order (rg_render_rows_f32), or f32 RGB rows stored at
+// their place in a full frame (rg_render_rowlist_f32_scatter).
+enum class OutKind { Rgba8, Rgba8Scatter, F32, F32Scatter };
+constexpr size_t bytes_per_pixel(OutKind k) { return k == OutKind::F32 || k == OutKind::F32Scatter ? 12 : 4; }
+// the output pointer is a full frame (address of image row 0), not the batch's first row
+constexpr bool is_scatter(OutKind k) { return k == OutKind::Rgba8Scatter || k == OutKind::F32Scatter; }
 
 }  // namespace rg
 
@@ -156,15 +159,17 @@ int wavefront_render(rg_scene *sc, uint32_t width, uint32_t height, uint32_t y0,
 int launch_resolve(OutKind kind, const float *src, uint32_t stride, uint32_t strip, uint32_t n, uint32_t width, uint32_t out_rows,
                    const uint32_t *d_rows, uint32_t row0, void *out, cudaStream_t stream);
 // rg_api.cu
-// rg_render_rowlist_device (kind Rgba8) and rg_render_rowlist_scatter (Rgba8Scatter) without the one-render-at-a-time
-// guard (for callers that hold it)
+// rg_render_rowlist_device / rg_render_rowlist_f32_device (kind Rgba8 / F32) and rg_render_rowlist_scatter /
+// rg_render_rowlist_f32_scatter (Rgba8Scatter / F32Scatter) without the one-render-at-a-time guard (for callers that hold it)
 int render_rowlist_device(rg_scene *sc, uint32_t w, uint32_t h, const uint32_t *rows, uint32_t n_rows, OutKind kind, void *d_out,
                           cudaStream_t stream, rg_stats *stats);
 // adds the stats of one part of a call to `total`; device times add up for parts that ran one after another and
 // overlap for `concurrent` ones (the slowest counts)
 void merge_stats(rg_stats &total, const rg_stats &part, bool concurrent);
 // rg_multi.cu
-int render_rowlist_to_host(rg_scene *sc, uint32_t w, uint32_t h, const uint32_t *rows, uint32_t n_rows, uint8_t *frame, rg_stats *st);
+// kind Rgba8 or F32: row rows[k] goes to frame + rows[k] * w * bytes_per_pixel(kind)
+int render_rowlist_to_host(rg_scene *sc, uint32_t w, uint32_t h, const uint32_t *rows, uint32_t n_rows, OutKind kind, uint8_t *frame,
+                           rg_stats *st);
 int multi_create(const rg_scene_desc *desc, const int32_t *devices, uint32_t n_devices, rg_scene **out);
 void multi_destroy(rg_scene *sc);
 int multi_set_option(rg_scene *sc, int32_t key, int64_t value);

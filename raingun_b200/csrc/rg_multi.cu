@@ -97,14 +97,15 @@ static int copy_rows_to_host(const uint8_t *d_src, const uint32_t *rows, size_t 
 }
 
 // Renders the listed image rows on the scene's device and delivers each at its place in a HOST frame.
-int render_rowlist_to_host(rg_scene *sc, uint32_t w, uint32_t h, const uint32_t *rows, uint32_t n_rows, uint8_t *frame, rg_stats *st) {
+int render_rowlist_to_host(rg_scene *sc, uint32_t w, uint32_t h, const uint32_t *rows, uint32_t n_rows, OutKind kind, uint8_t *frame,
+                           rg_stats *st) {
     if (n_rows == 0) { if (st) std::memset(st, 0, sizeof *st); return RG_OK; }
-    const size_t row_bytes = (size_t)w * 4;
+    const size_t row_bytes = (size_t)w * bytes_per_pixel(kind);
     int rc = sc->frame.reserve((size_t)n_rows * row_bytes);
     if (rc) return rc;
     rg_stats local;
     std::memset(&local, 0, sizeof local);
-    rc = render_rowlist_device(sc, w, h, rows, n_rows, OutKind::Rgba8, sc->frame.ptr, sc->stream, &local);
+    rc = render_rowlist_device(sc, w, h, rows, n_rows, kind, sc->frame.ptr, sc->stream, &local);
     if (rc) return rc;
     if ((rc = copy_rows_to_host(static_cast<const uint8_t *>(sc->frame.ptr), rows, n_rows, frame, row_bytes, sc->stream))) return rc;
     RG_CUDA(cudaStreamSynchronize(sc->stream));
@@ -119,7 +120,8 @@ static int render_tiles_to_host(rg_scene *sc, const MultiJob &j, const std::vect
     if (rows.empty()) return RG_OK;
     rg_stats local;
     // j.out holds rows [y0, y1): address of image row 0 = out - y0 rows
-    const int rc = render_rowlist_to_host(sc, j.w, j.h, rows.data(), (uint32_t)rows.size(), j.out - (size_t)j.y0 * j.w * 4, &local);
+    const int rc = render_rowlist_to_host(sc, j.w, j.h, rows.data(), (uint32_t)rows.size(), OutKind::Rgba8, j.out - (size_t)j.y0 * j.w * 4,
+                                          &local);
     if (rc) return rc;
     merge_stats(*st, local, false);
     return RG_OK;

@@ -417,7 +417,45 @@ __global__ void __launch_bounds__(256) k_quantise_scatter(const float4 *__restri
     }
 }
 
-// RG_OPT_SUPERSAMPLE = n > 1: the last kernel of a batch, in place of k_quantise / k_quantise_scatter / k_export_f32.
+// The f32 counterpart of k_quantise_scatter: RenderedPixel.color of batch row r stored at its place in a FULL frame of
+// 3 floats per pixel, frame + rows[row0 + r] * width * 3.  4 pixels per thread: their 48 bytes go out as three 128-bit
+// stores when the destination is 16-byte aligned (every group of 4 whenever width % 4 == 0 and the frame is 16-byte
+// aligned), as scalar stores otherwise; a group that crosses the end of a row stores pixel by pixel.
+__global__ void __launch_bounds__(256) k_export_f32_scatter(const float4 *__restrict__ node_a, float *frame, uint32_t npix,
+                                                            const uint32_t *__restrict__ rows, uint32_t row0, const PixelOrder po) {
+    const uint32_t p4 = (blockIdx.x * blockDim.x + threadIdx.x) * 4u;
+    if (p4 >= npix) return;
+    const uint32_t width = po.width;
+    const uint32_t r = p4 / width, x = p4 - r * width;
+    if (x + 4u <= width) {
+        float *dst = frame + ((size_t)rows[row0 + r] * width + x) * 3;
+        float v[12];
+#pragma unroll
+        for (uint32_t k = 0; k < 4; ++k) {
+            const float4 a = node_a[po.index(x + k, r)];
+            v[3 * k] = a.x; v[3 * k + 1] = a.y; v[3 * k + 2] = a.z;
+        }
+        if ((reinterpret_cast<uintptr_t>(dst) & 15u) == 0) {
+            float4 *d4 = reinterpret_cast<float4 *>(dst);
+            d4[0] = make_float4(v[0], v[1], v[2], v[3]);
+            d4[1] = make_float4(v[4], v[5], v[6], v[7]);
+            d4[2] = make_float4(v[8], v[9], v[10], v[11]);
+        } else {
+#pragma unroll
+            for (int k = 0; k < 12; ++k) dst[k] = v[k];
+        }
+    } else {
+        for (uint32_t k = p4; k < npix && k < p4 + 4u; ++k) {
+            const uint32_t rk = k / width, xk = k - rk * width;
+            const float4 a = node_a[po.index(xk, rk)];
+            float *d = frame + ((size_t)rows[row0 + rk] * width + xk) * 3;
+            d[0] = a.x; d[1] = a.y; d[2] = a.z;
+        }
+    }
+}
+
+// RG_OPT_SUPERSAMPLE = n > 1: the last kernel of a batch, in place of k_quantise / k_quantise_scatter / k_export_f32 /
+// k_export_f32_scatter.
 // One thread per output pixel averages its n x n samples as include/raingun_b200.h specifies: per channel s = 0, then
 // s + sample in sub-row, sub-column order, then s / (n n) rounded to nearest (a sum without products: nothing for
 // FMA contraction to fuse).  `po` spans the batch's sample rows; sample (X, Y) is f32 RGB at src + stride * po.index(X, Y)
@@ -444,6 +482,9 @@ __global__ void __launch_bounds__(256) k_resolve_ss(const float *__restrict__ sr
     if constexpr (K == OutKind::F32) {
         float *o = static_cast<float *>(out) + 3 * (size_t)p;
         o[0] = avg.r; o[1] = avg.g; o[2] = avg.b;
+    } else if constexpr (K == OutKind::F32Scatter) {
+        float *o = static_cast<float *>(out) + ((size_t)(rows[row0 + r * n] / n) * w + x) * 3;
+        o[0] = avg.r; o[1] = avg.g; o[2] = avg.b;
     } else if constexpr (K == OutKind::Rgba8Scatter) {
         static_cast<uchar4 *>(out)[(size_t)(rows[row0 + r * n] / n) * w + x] = quantise(avg);
     } else {
@@ -460,9 +501,12 @@ int launch_resolve(OutKind kind, const float *src, uint32_t stride, uint32_t str
     po.rows = n * out_rows;
     po.strip = strip;
     const unsigned blocks = (npix + 255) / 256;
-    if (kind == OutKind::F32) k_resolve_ss<OutKind::F32><<<blocks, 256, 0, stream>>>(src, stride, po, n, npix, d_rows, row0, out);
-    else if (kind == OutKind::Rgba8Scatter) k_resolve_ss<OutKind::Rgba8Scatter><<<blocks, 256, 0, stream>>>(src, stride, po, n, npix, d_rows, row0, out);
-    else k_resolve_ss<OutKind::Rgba8><<<blocks, 256, 0, stream>>>(src, stride, po, n, npix, d_rows, row0, out);
+    switch (kind) {
+        case OutKind::Rgba8: k_resolve_ss<OutKind::Rgba8><<<blocks, 256, 0, stream>>>(src, stride, po, n, npix, d_rows, row0, out); break;
+        case OutKind::Rgba8Scatter: k_resolve_ss<OutKind::Rgba8Scatter><<<blocks, 256, 0, stream>>>(src, stride, po, n, npix, d_rows, row0, out); break;
+        case OutKind::F32: k_resolve_ss<OutKind::F32><<<blocks, 256, 0, stream>>>(src, stride, po, n, npix, d_rows, row0, out); break;
+        case OutKind::F32Scatter: k_resolve_ss<OutKind::F32Scatter><<<blocks, 256, 0, stream>>>(src, stride, po, n, npix, d_rows, row0, out); break;
+    }
     RG_CUDA(cudaGetLastError());
     return RG_OK;
 }
@@ -860,12 +904,18 @@ static int enqueue_batch_dev(rg_scene *sc, const DevPlan &plan, uint32_t width, 
         if ((rc = launch_resolve(kind, reinterpret_cast<const float *>(wf.nodes[0].as<float4>()), 4, po.strip, n, width / n,
                                  po.rows / n, d_rows, y0, d_out, stream)))
             return rc;
-    } else if (kind == OutKind::F32)
-        k_export_f32<<<(npix + 255) / 256, 256, 0, stream>>>(wf.nodes[0].as<float4>(), reinterpret_cast<float *>(d_out), npix, po);
-    else if (kind == OutKind::Rgba8Scatter)
-        k_quantise_scatter<<<(unsigned)((((uint64_t)npix + 3) / 4 + 255) / 256), 256, 0, stream>>>(wf.nodes[0].as<float4>(), d_out, npix, d_rows, y0, po);
-    else
-        k_quantise<<<(unsigned)((((uint64_t)npix + 3) / 4 + 255) / 256), 256, 0, stream>>>(wf.nodes[0].as<float4>(), d_out, npix, po);
+    } else {
+        const unsigned blocks4 = (unsigned)((((uint64_t)npix + 3) / 4 + 255) / 256);   // 4 pixels per thread
+        const float4 *a = wf.nodes[0].as<float4>();
+        switch (kind) {
+            case OutKind::Rgba8: k_quantise<<<blocks4, 256, 0, stream>>>(a, d_out, npix, po); break;
+            case OutKind::Rgba8Scatter: k_quantise_scatter<<<blocks4, 256, 0, stream>>>(a, d_out, npix, d_rows, y0, po); break;
+            case OutKind::F32: k_export_f32<<<(npix + 255) / 256, 256, 0, stream>>>(a, reinterpret_cast<float *>(d_out), npix, po); break;
+            case OutKind::F32Scatter:
+                k_export_f32_scatter<<<blocks4, 256, 0, stream>>>(a, reinterpret_cast<float *>(d_out), npix, d_rows, y0, po);
+                break;
+        }
+    }
     RG_CUDA(cudaGetLastError());
     st->gpu_launches++;
     st->batches++;
@@ -986,7 +1036,7 @@ int wavefront_render(rg_scene *sc, uint32_t width, uint32_t height, uint32_t y0,
         }
         for (uint32_t y = y0; y < y1 && rc == RG_OK;) {
             const uint32_t ye = (uint32_t)std::min<uint64_t>((uint64_t)y + batch_rows, y1);
-            uchar4 *out = kind == OutKind::Rgba8Scatter ? d_out
+            uchar4 *out = is_scatter(kind) ? d_out
                         : reinterpret_cast<uchar4 *>(reinterpret_cast<unsigned char *>(d_out) + (size_t)(y - y0) * width * bytes_per_pixel(kind));
             DevPlan plan;
             const uint64_t npix64 = (uint64_t)(ye - y) * n * sw;

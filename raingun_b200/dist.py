@@ -6,7 +6,7 @@ replicated, the image is cut into tiles of ``tile_rows`` rows, and every rank re
 tiles it claims.  Cost per row is very uneven (sky vs sphere field), so tiles are handed out
 by a work-stealing counter — an atomic fetch-add on the c10d store all ranks already share —
 in guided chunks (large first, small last).  The only exchange is the final gather of the
-RGBA8 tiles into rank 0's frame: point-to-point sends over NVLink (NCCL send/recv), i.e.
+finished tiles into rank 0's frame: point-to-point sends over NVLink (NCCL send/recv), i.e.
 rayon's ``collect`` (rendering.rs:34-35).
 
 A batch of few rows cannot fill a B200 (its 8 bounce levels are ~40 short, latency-bound launches
@@ -19,6 +19,11 @@ Gather.  ``peer`` (GPUs): rank 0 owns the frame (two, alternating per frame), ev
 maps it through CUDA IPC and its last kernel stores each finished row at its place in rank 0's
 memory over NVLink (``rg_render_rowlist_scatter``) — compute and "collective" are one kernel, and a
 barrier is all that is left.  ``reduce`` / ``p2p``: NCCL (or gloo) collectives on packed rows.
+
+Pixel formats.  ``pixel_format="rgba8"`` (the default) gathers the reference's RGBA8 bytes, 4 per pixel;
+``"f32"`` the unquantised f32 colours (``RenderedPixel.color``), 3 floats per pixel.  Rows travel as bytes
+either way: ``row_bytes = width * bytes_per_pixel`` is the only place the format enters, and only the
+finished frame is viewed as (H, W, 4) uint8 or (H, W, 3) float32.
 
 One process per GPU (torchrun); works unchanged on the gloo backend with CPU tensors, which
 is how the host logic is tested without GPUs (tests/test_dist_gloo.py).
@@ -41,6 +46,25 @@ DEFAULT_TILE_ROWS = 8
 # while every stolen tail batch costs ~1 ms of latency-bound launches (measured: +0.5..0.9 ms per
 # 4K frame at 4-8 GPUs); below it, cost per tile is too uneven to trust static ownership.
 AUTO_STATIC_MIN_TILES_PER_RANK = 16
+
+# pixel_format -> (bytes per pixel, channels, numpy dtype, torch dtype) of a finished frame
+PIXEL_FORMATS = {"rgba8": (4, 4, np.uint8, torch.uint8), "f32": (12, 3, np.float32, torch.float32)}
+
+
+def _format(pixel_format: str):
+    if pixel_format not in PIXEL_FORMATS:
+        raise ValueError(f"pixel_format must be one of {sorted(PIXEL_FORMATS)}, not {pixel_format!r}")
+    return PIXEL_FORMATS[pixel_format]
+
+
+def bytes_per_pixel(pixel_format: str) -> int:
+    return _format(pixel_format)[0]
+
+
+def frame_view(buf: torch.Tensor, height: int, width: int, pixel_format: str) -> torch.Tensor:
+    """The finished frame over the bytes of a contiguous uint8 buffer: (H, W, 4) uint8 or (H, W, 3) float32."""
+    _, channels, _, dtype = _format(pixel_format)
+    return buf.view(dtype).view(height, width, channels)
 
 
 def n_tiles(height: int, tile_rows: int) -> int:
@@ -213,11 +237,14 @@ class SharedHostFrame:
     (``Scene.render_rowlist_host``) and nothing is gathered on one GPU first.  Two frames alternate like
     ``PeerFrames``.  Rank 0 reads the finished frame after the end-of-frame barrier."""
 
-    def __init__(self, width: int, height: int, rank: int, world: int, store=None, tag: str = "0", pin: bool = True) -> None:
+    def __init__(self, width: int, height: int, rank: int, world: int, store=None, tag: str = "0", pin: bool = True,
+                 pixel_format: str = "rgba8") -> None:
         import os
 
         self.width, self.height, self.rank, self.world = width, height, rank, world
-        self.nbytes = width * height * 4
+        bpp, channels, np_dtype, _ = _format(pixel_format)
+        self.pixel_format = pixel_format
+        self.nbytes = width * height * bpp
         self.maps, self.paths, self.pinned = [], [], []
         for k in range(2):
             key = f"raingun/host_frame/{tag}/{k}"
@@ -229,7 +256,7 @@ class SharedHostFrame:
                     (store or default_store()).set(key, path)
             else:
                 path = bytes((store or default_store()).get(key)).decode()
-            mm = np.memmap(path, dtype=np.uint8, mode="r+", shape=(height, width, 4))
+            mm = np.memmap(path, dtype=np_dtype, mode="r+", shape=(height, width, channels))
             self.maps.append(mm)
             self.paths.append(path)
             if pin:
@@ -269,11 +296,12 @@ class PeerFrames:
     frame of each other."""
 
     def __init__(self, width: int, height: int, rank: int, world: int, device_index: int, store=None,
-                 tag: str = "0") -> None:
+                 tag: str = "0", pixel_format: str = "rgba8") -> None:
         from . import SharedFrame
 
         self.width, self.height, self.rank, self.world, self.device_index = width, height, rank, world, device_index
-        nbytes = width * height * 4
+        self.pixel_format = pixel_format
+        nbytes = width * height * bytes_per_pixel(pixel_format)
         self.frames = []
         for k in range(2):
             key = f"raingun/peer_frame/{tag}/{k}"
@@ -297,9 +325,10 @@ class PeerFrames:
         return self.frames[frame_id & 1].ptr
 
     def tensor(self, frame_id: int) -> torch.Tensor:
-        """Zero-copy (H, W, 4) uint8 view of the frame (meaningful on rank 0, which owns the memory)."""
+        """Zero-copy (H, W, 4) uint8 or (H, W, 3) float32 view of the frame (meaningful on rank 0, which owns the
+        memory)."""
         t = torch.as_tensor(self.frames[frame_id & 1], device=torch.device("cuda", self.device_index))
-        return t.view(self.height, self.width, 4)
+        return frame_view(t, self.height, self.width, self.pixel_format)
 
     def close(self, sync: bool = True) -> None:
         """``sync=False`` only when no peer can be using the frames (e.g. set-up failed on some rank)."""
@@ -319,7 +348,7 @@ class PeerFrames:
 
 @dataclass
 class ShardResult:
-    frame: Optional[torch.Tensor]          # (H, W, 4) uint8 on rank 0, None elsewhere
+    frame: Optional[torch.Tensor]          # (H, W, 4) uint8 or (H, W, 3) float32 on rank 0, None elsewhere
     my_tiles: List[int] = field(default_factory=list)
     claims: int = 0
     schedule: str = ""                     # the schedule actually used ("auto" resolved)
@@ -339,12 +368,13 @@ def render_frame_sharded(render_rowlist: Union[Callable[[np.ndarray, torch.Tenso
                          gather: bool = True, staging: Optional[torch.Tensor] = None,
                          gather_mode: str = "reduce", frame_buf: Optional[torch.Tensor] = None,
                          lead: float = 0.6, peer_frames: Optional[PeerFrames] = None,
-                         host_barrier: Optional["HostBarrier"] = None) -> ShardResult:
+                         host_barrier: Optional["HostBarrier"] = None, pixel_format: str = "rgba8") -> ShardResult:
     """Renders one frame across ``world`` ranks.
 
-    ``render_rowlist(rows, out)`` must fill ``out`` (a uint8 tensor of ``len(rows)*width*4``
-    bytes on ``device``) with the listed image rows, compacted in list order, and return once they
-    are there — on a GPU that is ``Scene.render_rowlist_device``.  A LIST of such callables keeps
+    ``render_rowlist(rows, out)`` must fill ``out`` (a uint8 tensor of ``len(rows)*row_bytes``
+    bytes on ``device``, ``row_bytes = width * bytes_per_pixel(pixel_format)``) with the listed image rows,
+    compacted in list order, and return once they are there — on a GPU that is ``Scene.render_rowlist_device``
+    (``"rgba8"``) or ``Scene.render_rowlist_f32_device`` (``"f32"``).  A LIST of such callables keeps
     that many batches in flight on this rank (one host thread each; see the module docstring).
     ``schedule`` is ``"steal"`` (static interleaved share first, then the
     work-stealing counter for the tail — see ``hybrid_plan``), ``"static"`` (interleaved
@@ -352,20 +382,26 @@ def render_frame_sharded(render_rowlist: Union[Callable[[np.ndarray, torch.Tenso
     ``AUTO_STATIC_MIN_TILES_PER_RANK`` tiles, else steal).
 
     ``gather_mode``: ``"peer"`` — needs ``peer_frames``; the renderers are then called as
-    ``render_rowlist(rows, frame_ptr)`` and must store row ``rows[k]`` at ``frame_ptr + rows[k]*width*4``
-    (``Scene.render_rowlist_scatter``); the frame is complete on rank 0 after one barrier.
+    ``render_rowlist(rows, frame_ptr)`` and must store row ``rows[k]`` at ``frame_ptr + rows[k]*row_bytes``
+    (``Scene.render_rowlist_scatter`` / ``render_rowlist_f32_scatter``); the frame is complete on rank 0 after one
+    barrier.
     ``"host"`` — as ``"peer"`` with ``peer_frames`` a ``SharedHostFrame``: the renderers
-    (``Scene.render_rowlist_host``) copy every row to its place in ONE pinned host frame all ranks map, each GPU
+    (``Scene.render_rowlist_host`` / ``render_rowlist_f32_host``) copy every row to its place in ONE pinned host frame all ranks map, each GPU
     over its own PCIe link; the frame is complete in rank 0's host memory after one barrier.
     ``"reduce"`` — every rank scatters its rows into a zeroed full frame and ONE
     NCCL reduce (MAX over disjoint rows, i.e. a gather that needs no ownership exchange) lands the
     frame on rank 0 over NVLink; ``"p2p"`` — the row lists travel through the store and rank 0
-    receives each rank's packed rows point to point.
+    receives each rank's packed rows point to point.  ``"peer"``, ``"host"`` and ``"p2p"`` move bytes and serve
+    either ``pixel_format``; ``"reduce"`` is RGBA8 only (a MAX over zero-filled rows does not carry the f32 NaN
+    bits the reference's colours can hold) and raises ``ValueError`` for ``"f32"`` before any collective.
     """
+    row_bytes = width * bytes_per_pixel(pixel_format)
+    if gather and gather_mode == "reduce" and pixel_format != "rgba8":
+        raise ValueError(f"gather_mode='reduce' cannot gather pixel_format={pixel_format!r}: a MAX reduction does not "
+                         "carry NaN bits; use 'p2p', 'peer' or 'host'")
     nt = n_tiles(height, tile_rows)
     schedule = resolve_schedule(schedule, nt, world)
     res = ShardResult(frame=None, schedule=schedule)
-    row_bytes = width * 4
     renderers = list(render_rowlist) if isinstance(render_rowlist, (list, tuple)) else [render_rowlist]
     workers = len(renderers)
     host = gather_mode == "host"     # like "peer", but the shared frame lives in pinned host memory (SharedHostFrame)
@@ -465,8 +501,9 @@ def render_frame_sharded(render_rowlist: Union[Callable[[np.ndarray, torch.Tenso
     # ---- gather: ownership is dynamic, so the row lists travel first (tiny), then the pixels
     packed = staging[: filled_rows * row_bytes]
     if world == 1:
-        res.frame = packed.view(height, width, 4) if np.array_equal(rows_all, np.arange(height)) else \
-            _scatter_rows(torch.empty((height, width, 4), dtype=torch.uint8, device=device), rows_all, packed, width)
+        frame = packed if np.array_equal(rows_all, np.arange(height)) else \
+            _scatter_rows(torch.empty((height, row_bytes), dtype=torch.uint8, device=device), rows_all, packed, width)
+        res.frame = frame_view(frame, height, width, pixel_format)
         return res
     if gather_mode == "reduce":
         frame = frame_buf if frame_buf is not None else torch.empty((height, width, 4), dtype=torch.uint8, device=device)
@@ -481,7 +518,7 @@ def render_frame_sharded(render_rowlist: Union[Callable[[np.ndarray, torch.Tenso
         store = default_store()
     store.set(f"raingun/rows/{frame_id}/{rank}", pickle.dumps(rows_all))
     if rank == 0:
-        frame = torch.empty((height, width, 4), dtype=torch.uint8, device=device)
+        frame = torch.empty((height, row_bytes), dtype=torch.uint8, device=device)
         _scatter_rows(frame, rows_all, packed, width)
         lists = {r: pickle.loads(store.get(f"raingun/rows/{frame_id}/{r}")) for r in range(1, world)}
         recv_bufs, ops = {}, []
@@ -494,7 +531,7 @@ def render_frame_sharded(render_rowlist: Union[Callable[[np.ndarray, torch.Tenso
                 req.wait()
         for r, buf in recv_bufs.items():
             _scatter_rows(frame, lists[r], buf, width)
-        res.frame = frame
+        res.frame = frame_view(frame, height, width, pixel_format)
         check_all_rows_rendered()
     elif filled_rows:
         for req in dist.batch_isend_irecv([dist.P2POp(dist.isend, packed, 0)]):
@@ -506,6 +543,8 @@ _IDX_CACHE: dict = {}
 
 
 def _scatter_rows(frame: torch.Tensor, rows: np.ndarray, packed: torch.Tensor, width: int) -> torch.Tensor:
+    """Copies packed row ``k`` to row ``rows[k]`` of ``frame`` (contiguous, one image row per index of dim 0; rows
+    are moved as bytes, whatever the pixel format)."""
     if rows.size:
         key = (str(frame.device), rows.tobytes())   # static ownership repeats every frame: keep the index on the device
         idx = _IDX_CACHE.get(key)
@@ -513,5 +552,5 @@ def _scatter_rows(frame: torch.Tensor, rows: np.ndarray, packed: torch.Tensor, w
             if len(_IDX_CACHE) > 64:
                 _IDX_CACHE.clear()
             idx = _IDX_CACHE[key] = torch.from_numpy(rows.astype(np.int64)).to(frame.device)
-        frame.index_copy_(0, idx, packed.view(int(rows.size), width, 4))
+        frame.view(frame.shape[0], -1).index_copy_(0, idx, packed.view(int(rows.size), -1))
     return frame
