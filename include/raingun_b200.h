@@ -146,20 +146,24 @@ enum {
                                 rendering.rs:24-38).  Values 0-2 are accepted and ignored */
     RG_OPT_GRAPH = 8,        /* replay the host-free frame as one CUDA graph: 0 = automatic, 1 = off, 2 = on */
     RG_OPT_TRACE_STATS = 9,  /* 1 = the grid tracer counts cells / fetches / cull tests / lane use
-                                (rg_stats.grid_*); an instrumented kernel, slower; results unchanged */
+                                (rg_stats.grid_*); an instrumented kernel, slower; results unchanged.
+                                2 = count the any-hit (shadow) launches only, 3 = the nearest-hit ones only */
     RG_OPT_SCHEDULE = 11,    /* multi-GPU scenes: 0 = automatic, 1 = static (tile t on device t mod N),
                                 2 = static share + a stealable tail handed out by an atomic tile counter */
     RG_OPT_TILE_ROWS = 12,   /* multi-GPU scenes: rows per tile (default 8) */
     RG_OPT_ORIGIN_HINTS = 13, /* 1 (default) = every secondary ray carries the outcome of the reference's test against the
                                 sphere it starts on, and the grid tracer skips that test; 0 = off.  Results unchanged
                                 (Scene::trace is a minimum: a body proven to return None may be left out, scene.rs:34-39) */
-    RG_OPT_SUPERSAMPLE = 14  /* n x n primary rays per pixel, box-filtered on the device; 1 (default) ... 8, anything else
+    RG_OPT_SUPERSAMPLE = 14, /* n x n primary rays per pixel, box-filtered on the device; 1 (default) ... 8, anything else
                                 is RG_E_INVALID.  A (w x h) frame is the reference's render at (n*w x n*h) reduced n x n:
                                 sample (X, Y) is the f32 Color of create_prime(X, Y, n*w, n*h) (ray.rs:37-54), and per
                                 channel, in f32, s = 0; for j in 0..n, for i in 0..n: s = s + sample(n*x + i, n*y + j);
                                 avg = s / (n*n), rounded to nearest.  The RGBA8 entry points store Color::rgba(avg)
                                 (color.rs:32-37), the f32 ones avg.  Output buffers keep their sizes; the ray and error
                                 counters count every sample's rays.  (n*w)*(n*h) must fit in u32, else RG_E_TOO_LARGE. */
+    RG_OPT_LIGHT_GRIDS = 15  /* 1 (default) = the grid tracer traces the shadow rays of a scene's first 8 lights through
+                                per-light 2-D grids (one short list per ray instead of a 3-D walk); 0 = the 3-D walk for
+                                every ray.  Results unchanged (DESIGN.md section 4.2) */
 };
 
 /* Counters and timings of one render call.  A "ray" is one `Scene::trace`

@@ -500,6 +500,8 @@ static int build_scene(rg_scene *sc, const rg_scene_desc *d) {
     lap("textures");
     if ((rc = grid_build(sc, sph, nsp))) return rc;   // (synchronises the stream: the staging buffer is free again)
     lap("grid");
+    if ((rc = light_grid_build(sc, sph, nsp))) return rc;
+    lap("light grids");
     RG_CUDA(cudaStreamSynchronize(sc->stream));
     return RG_OK;
 }
@@ -690,10 +692,15 @@ int rg_scene_set_option(rg_scene *sc, int32_t key, int64_t value) {
             sc->graph = (int)value;
             return RG_OK;
         case RG_OPT_TRACE_STATS:
-            sc->trace_stats = value != 0;
+            if (value < 0 || value > 3) break;
+            sc->trace_stats = (int)value;
             return RG_OK;
         case RG_OPT_ORIGIN_HINTS:
             sc->origin_hints = value != 0;
+            return RG_OK;
+        case RG_OPT_LIGHT_GRIDS:
+            if (value < 0 || value > 1) break;
+            sc->light_grids = value != 0;
             return RG_OK;
         case RG_OPT_SUPERSAMPLE:
             if (value < 1 || value > 8) break;

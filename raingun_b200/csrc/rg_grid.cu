@@ -461,5 +461,135 @@ int grid_build(rg_scene *sc, const double *sph, uint32_t n) {
     return on_host ? grid_build_host(sc, sph, n) : grid_build_device(sc, sph, n);
 }
 
+// ---- light grids (rg_light_grid.h) -------------------------------------------------------------
+// Built like the 3-D grid on the device: count -> scan -> fill -> per-cell sort -> records, over the items of
+// every light at once (one thread per (light, item)).  Lists are sorted by (FP32 depth rounded down, item index),
+// so the build is deterministic; a record's 4th word holds the depth of its first item.
+static double light_grid_density() {   // key cells per item (RG_LIGHT_GRID_DENSITY overrides, for tuning runs)
+    static const double d = [] { const char *e = getenv("RG_LIGHT_GRID_DENSITY"); double v = e ? atof(e) : 0.0; return v > 0.0 ? v : 2.0; }();
+    return d;
+}
+
+__device__ __forceinline__ uint64_t lg_sort_key(const LightGridInfo &g, const double4 sp, uint32_t i) {
+    const double c[3] = {sp.x, sp.y, sp.z};
+    return ((uint64_t)lg_float_order(lg_float_down(lg_item_depth(g, c, sp.w))) << 32) | i;
+}
+
+// FILL = false: count the entries of every cell; true: write them (sort keys) at start[c] + cursor[c]
+template <bool FILL>
+__global__ void __launch_bounds__(256) k_lg_bin(const LightGridInfo *__restrict__ info, uint32_t n_lights, const double4 *__restrict__ sph,
+                                                uint32_t n, uint32_t *count, const uint32_t *__restrict__ start, uint64_t *keys,
+                                                const uint32_t *__restrict__ ctr, uint32_t items_cap) {
+    const uint64_t t = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (t >= (uint64_t)n * n_lights) return;
+    if (FILL && ctr[GB_TOTAL] > items_cap) return;
+    const uint32_t l = (uint32_t)(t / n), i = (uint32_t)(t % n);
+    const LightGridInfo g = info[l];
+    const double4 sp = sph[i];
+    const double c[3] = {sp.x, sp.y, sp.z};
+    int rng[6][4];
+    const int k = lg_item_ranges(g, c, sp.w, rng);
+    const uint64_t key = FILL ? lg_sort_key(g, sp, i) : 0ull;
+    auto put = [&](uint32_t cell) {
+        if (FILL) keys[start[cell] + atomicAdd(&count[cell], 1u)] = key;
+        else atomicAdd(&count[cell], 1u);
+    };
+    if (k < 0) { put(g.always); return; }
+    for (int f = 0; f < 6; ++f)
+        for (int y = rng[f][2]; y <= rng[f][3]; ++y)
+            for (int x = rng[f][0]; x <= rng[f][1]; ++x) put(g.base + lg_cell_index(g, f, x, y));
+}
+
+// per cell: sort the keys, then the item list and the chain of 48-byte records (as k_gb_finish)
+__global__ void __launch_bounds__(256) k_lg_finish(uint32_t ncells, const uint32_t *__restrict__ start, uint64_t *keys, uint32_t *items,
+                                                   const float4 *__restrict__ cull4, float4 *recs, const uint32_t *__restrict__ ctr,
+                                                   uint32_t items_cap) {
+    const uint32_t c = blockIdx.x * blockDim.x + threadIdx.x;
+    if (c >= ncells || ctr[GB_TOTAL] > items_cap) return;
+    const uint32_t b0 = start[c], b1 = start[c + 1];
+    lg_sort_u64(keys + b0, b1 - b0);
+    for (uint32_t i = b0; i < b1; ++i) items[i] = (uint32_t)keys[i];
+    const float kInf = __int_as_float(0x7f800000);
+    for (uint32_t pos = b0, r = c;; pos += 2) {
+        const uint32_t m = b1 - pos > 2 ? 2 : b1 - pos;
+        const uint32_t next = pos + 2 < b1 ? grid_chain_record(ncells, pos + 2) : 0u;
+        recs[3 * (size_t)r] = m > 0 ? cull4[items[pos]] : make_float4(0.f, 0.f, 0.f, kInf);
+        recs[3 * (size_t)r + 1] = m > 1 ? cull4[items[pos + 1]] : make_float4(0.f, 0.f, 0.f, kInf);
+        const float depth = m > 0 ? lg_order_float((uint32_t)(keys[pos] >> 32)) : kInf;
+        *reinterpret_cast<uint4 *>(&recs[3 * (size_t)r + 2]) =
+            make_uint4(m > 0 ? items[pos] : 0xFFFFFFFFu, m > 1 ? items[pos + 1] : 0xFFFFFFFFu, next, __float_as_uint(depth));
+        if (!next) break;
+        r = next;
+    }
+}
+
+int light_grid_build(rg_scene *sc, const double *sph, uint32_t n) {
+    sc->lg = LightGrids{};
+    const uint32_t nl = std::min<uint32_t>((uint32_t)sc->lights.size(), kLightGrids);
+    if (!sc->ds.grid.enabled || nl == 0 || n == 0) return RG_OK;   // only the grid tracer reads light grids
+    double scale = 1.0;
+    for (uint32_t i = 0; i < n; ++i) {
+        const double *c = sph + 4 * (size_t)i;
+        const double m = std::max(std::max(std::fabs(c[0]), std::fabs(c[1])), std::fabs(c[2])) + std::fabs(c[3]);
+        if (m < 1e6) scale = std::max(scale, 1.0 + m);   // (false on NaN: such items go on the always lists)
+    }
+    std::vector<LightGridInfo> info;
+    uint32_t ncells = 1;   // cell 0: the empty placeholder (rg_light_grid.h)
+    for (uint32_t l = 0; l < nl; ++l) {
+        const DLight &L = sc->lights[l];
+        double sl = scale;
+        if (L.kind != RG_LIGHT_DIRECTIONAL) {
+            const double m = std::max(std::max(std::fabs(L.v[0]), std::fabs(L.v[1])), std::fabs(L.v[2]));
+            if (!(m < 1e6)) break;
+            sl = std::max(sl, 1.0 + m);
+        }
+        LightGridInfo g;
+        if (!lg_setup(g, L.kind == RG_LIGHT_DIRECTIONAL ? 0u : 1u, L.v, sph, n, sl, light_grid_density())) break;   // lights [0, l) keep theirs
+        g.base = ncells;
+        g.always = ncells + lg_key_cells(g);
+        ncells = g.always + 1;
+        info.push_back(g);
+    }
+    if (info.empty()) return RG_OK;
+    const uint32_t nlg = (uint32_t)info.size();
+    const LightGridInfo *d_info = nullptr;
+    int rc;
+    if ((rc = upload_vec(sc, info, &d_info))) return rc;
+    uint32_t items_cap = (uint32_t)std::min<uint64_t>(std::max<uint64_t>(4ull * n * nlg, 4096), 0x7FFFFFFFull);
+    cudaStream_t st = sc->stream;
+    uint32_t h_ctr[4] = {0, 0, 0, 0};
+    uint32_t *start = nullptr, *cursor = nullptr, *ctr = nullptr, *items = nullptr;
+    uint64_t *keys = nullptr;
+    float4 *recs = nullptr;
+    const unsigned bblocks = (unsigned)(((uint64_t)n * nlg + 255) / 256);
+    for (int pass = 0; pass < 2; ++pass) {
+        start = static_cast<uint32_t *>(sc->arena.alloc(((size_t)ncells + 1) * sizeof(uint32_t)));
+        cursor = static_cast<uint32_t *>(sc->arena.alloc((size_t)ncells * sizeof(uint32_t)));
+        ctr = static_cast<uint32_t *>(sc->arena.alloc(4 * sizeof(uint32_t)));
+        keys = static_cast<uint64_t *>(sc->arena.alloc((size_t)items_cap * sizeof(uint64_t)));
+        items = static_cast<uint32_t *>(sc->arena.alloc((size_t)items_cap * sizeof(uint32_t)));
+        recs = static_cast<float4 *>(sc->arena.alloc(grid_record_count(ncells, items_cap) * 3 * sizeof(float4)));
+        if (!start || !cursor || !ctr || !keys || !items || !recs) return RG_E_NOMEM;
+        RG_CUDA(cudaMemsetAsync(start, 0, ((size_t)ncells + 1) * sizeof(uint32_t), st));
+        RG_CUDA(cudaMemsetAsync(cursor, 0, (size_t)ncells * sizeof(uint32_t), st));
+        RG_CUDA(cudaMemsetAsync(ctr, 0, 4 * sizeof(uint32_t), st));
+        k_lg_bin<false><<<bblocks, 256, 0, st>>>(d_info, nlg, sc->ds.sph, n, start, nullptr, nullptr, ctr, items_cap);
+        k_gb_scan<<<1, 1024, 0, st>>>(start, ncells, ctr);
+        k_lg_bin<true><<<bblocks, 256, 0, st>>>(d_info, nlg, sc->ds.sph, n, cursor, start, keys, ctr, items_cap);
+        k_lg_finish<<<(ncells + 255) / 256, 256, 0, st>>>(ncells, start, keys, items, sc->ds.cull4, recs, ctr, items_cap);
+        RG_CUDA(cudaGetLastError());
+        RG_CUDA(cudaMemcpyAsync(h_ctr, ctr, sizeof h_ctr, cudaMemcpyDeviceToHost, st));
+        RG_CUDA(cudaStreamSynchronize(st));
+        if (h_ctr[GB_TOTAL] <= items_cap) break;
+        items_cap = h_ctr[GB_TOTAL];   // lists longer than the guess: once more, exactly sized
+    }
+    LightGrids &lg = sc->lg;
+    lg.n_lights = nlg;
+    lg.info = d_info;
+    lg.cell_rec = recs;
+    lg.cell_start = start;
+    lg.cell_items = items;
+    return RG_OK;
+}
 
 }  // namespace rg

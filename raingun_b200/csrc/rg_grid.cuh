@@ -39,6 +39,7 @@
 //   * a lane that finds a cull survivor parks it ("pending"); the warp evaluates pending
 //     candidates together, so the expensive exact test runs with many lanes active instead of one.
 #pragma once
+#include "rg_light_grid.h"
 #include "rg_trace.cuh"
 
 namespace rg {
@@ -112,9 +113,12 @@ __device__ __forceinline__ void exact_sphere(const DScene &s, const Ray &ray, ui
 // STATS = true: the instrumented build of the same kernel (RG_OPT_TRACE_STATS) that counts cells visited,
 // records fetched, cull tests, refills and lane use into DCounters::grid_*; results are unchanged.
 // PROXY = true: the grid also holds boxes and disks (`gp`, rg_scene.cuh); false: spheres only, `gp` is not read.
-template <bool ANY, bool STATS = false, bool PROXY = false>
+// LIGHT = true (any-hit launches of a light-major shadow queue): a ray whose light has a light grid (`lg`,
+// rg_light_grid.h) and whose key it covers scans that cell's list ("flat" walk) instead of walking the 3-D grid.
+template <bool ANY, bool STATS = false, bool PROXY = false, bool LIGHT = false>
 __global__ void __launch_bounds__(kGridTraceThreads, RG_GRID_MINB) k_trace_grid(const DScene s, const TraceArgs a,
-                                                                                const GridProxies gp) {
+                                                                                const GridProxies gp, const LightGrids lg) {
+    static_assert(ANY || !LIGHT, "light grids serve shadow rays only");
     const GridDev &g = s.grid;
     const uint32_t lane = threadIdx.x & 31u;
     const uint32_t lanemask_lt = (1u << lane) - 1u;
@@ -144,7 +148,8 @@ __global__ void __launch_bounds__(kGridTraceThreads, RG_GRID_MINB) k_trace_grid(
     float kx = 0, ky = 0, kz = 0;
     float dtx = 0, dty = 0, dtz = 0;
     float tex = 0, tey = 0, tez = 0;
-    float tcur = 0;                                            // parameter at which the walk enters `cell` (+inf: it has left the grid)
+    float tcur = 0;                                            // parameter at which the walk enters `cell` (+inf: it has left the grid);
+                                                               // flat walk: the ray's own light-space depth (rounded up)
     float boundf = 0;                                          // distances worth looking at, in walk parameter units (FP32, rounded up)
     float t0f = 0;                                             // the walk is parameterised from o + t0*d (far origins)
     int cell = 0, scx = 0, scy = 0, scz = 0;                   // linear index of the next cell to examine, per-axis stride (signed)
@@ -153,6 +158,7 @@ __global__ void __launch_bounds__(kGridTraceThreads, RG_GRID_MINB) k_trace_grid(
     uint32_t skip = kNoSphere;                                 // a sphere whose exact result for this ray is already known: the origin hint
                                                                // (rg_trace.cuh), then the sphere tested last (it is listed in the next cells too)
     bool exhausted = false;                                    // warp-uniform: the queue has no more rays
+    bool flat = false;                                         // LIGHT: the ray scans one light-grid list; chain == 0 ends it
     h.best.init();
     h.occluded = false;
     h.tmax = 0.0;
@@ -190,6 +196,7 @@ __global__ void __launch_bounds__(kGridTraceThreads, RG_GRID_MINB) k_trace_grid(
                 walking = false;
                 pend0 = pend1 = kNoSphere;
                 chain = 0;
+                if (LIGHT) flat = false;
                 pi = phys_index(seg_len, a.seg_stride, ri);
                 const Ray ray = load_ray(a.q, pi);
                 skip = a.q.hint[pi];
@@ -243,6 +250,28 @@ __global__ void __launch_bounds__(kGridTraceThreads, RG_GRID_MINB) k_trace_grid(
                 if (ANY && skip == kHintOccluded) h.occluded = true;   // the sphere the ray starts on is in the way
                 if (!(ANY && h.occluded)) {
                 cr = make_cull_ray(s, ray, true);
+                if (LIGHT) {
+                    // light-major segments: ray ri belongs to light first_light + ri / seg_len
+                    const uint32_t li = seg_len ? lg.first_light + ri / seg_len : 0xFFFFFFFFu;
+                    if (li < lg.n_lights) {
+                        const LightGridInfo &gi = lg.info[li];
+                        const double o3[3] = {ray.o.x, ray.o.y, ray.o.z}, d3_[3] = {ray.d.x, ray.d.y, ray.d.z};
+                        double depth = 0.0;
+                        const long long key = lg_ray_key(gi, o3, d3_, h.tmax, depth);
+                        if (key != -2) {   // inside the argument of DESIGN.md 4.2: the light grid replaces the 3-D walk
+                            flat = true;
+                            for (uint32_t q = lg.cell_start[gi.always]; q < lg.cell_start[gi.always + 1]; ++q) {
+                                const uint32_t sp = lg.cell_items[q];
+                                if (sp != skip && !cull_reject(cr, s.cull4[sp])) exact_sphere<ANY, PROXY>(s, ray, sp, h, n_exact, nan_count);
+                            }
+                            chain = key >= 0 ? gi.base + (uint32_t)key : 0u;   // the cell's first record
+                            tcur = __double2float_ru(depth);
+                            walking = chain != 0u && !h.occluded;
+                            if (STATS) st_cells += walking ? 1u : 0u;
+                        }
+                    }
+                }
+                if (!(LIGHT && flat)) {
                 D3 op = ray.o - d3(s.cull_ref[0], s.cull_ref[1], s.cull_ref[2]);
                 const double D2 = dot(ray.d, ray.d);
                 // Far-away origins (e.g. hits on an infinite plane near the horizon) would lose FP32
@@ -344,6 +373,7 @@ __global__ void __launch_bounds__(kGridTraceThreads, RG_GRID_MINB) k_trace_grid(
                         }
                     }
                 }
+                }   // not a flat walk
                 }   // not occluded by a body tested above / by the origin hint
             }
         }
@@ -359,9 +389,13 @@ __global__ void __launch_bounds__(kGridTraceThreads, RG_GRID_MINB) k_trace_grid(
 #pragma unroll 1
         for (int burst = 0; burst < a.g_burst; ++burst) {
             bool go = active && walking && pend0 == kNoSphere && pend1 == kNoSphere;
-            const bool enter = chain == 0u;   // the next record is a new cell's first
-            if (go && enter && ((ANY && h.occluded) || boundf < fmaf(tcur, 0.99999f, -1e-5f))) {
+            const bool enter = chain == 0u;   // the next record is a new cell's first (flat walk: the list has ended)
+            if (go && enter && ((ANY && h.occluded) || (LIGHT && flat) || boundf < fmaf(tcur, 0.99999f, -1e-5f))) {
                 walking = false;   // nothing nearer can lie in or beyond this cell (or the walk has left the grid)
+                go = false;
+            }
+            if (LIGHT && go && flat && h.occluded) {   // a flat list is one long cell: stop inside it
+                walking = false;
                 go = false;
             }
             if (STATS) {
@@ -369,7 +403,7 @@ __global__ void __launch_bounds__(kGridTraceThreads, RG_GRID_MINB) k_trace_grid(
                 if (lane == 0) st_lane_slots += 32u;
             }
             if (go) {
-                const float4 *rec = g.cell_rec + 3 * (size_t)(enter ? (uint32_t)cell : chain);
+                const float4 *rec = (LIGHT && flat ? lg.cell_rec : g.cell_rec) + 3 * (size_t)(enter ? (uint32_t)cell : chain);
                 const float4 c0 = rec[0], c1 = rec[1];
                 const uint4 cm = *reinterpret_cast<const uint4 *>(rec + 2);
                 if (enter) {
@@ -390,10 +424,14 @@ __global__ void __launch_bounds__(kGridTraceThreads, RG_GRID_MINB) k_trace_grid(
                     tcur = fmaxf(kx, fmaxf(ky, kz)) > 0.0f ? kFltInf : tnext;
                 }
                 if (STATS) { st_cells += enter ? 1u : 0u; st_fetch += (cm.x != kNoSphere) ? 1u : 0u; st_culls += (cm.x != kNoSphere) + (cm.y != kNoSphere); }
+                if (LIGHT && flat && __uint_as_float(cm.w) > tcur) {
+                    chain = 0u;   // this record and every later one lie farther from the light than the ray's origin
+                } else {
                 // (an empty slot holds kNoSphere: "parking" it parks nothing, so it needs no test of its own)
                 if (cm.x != skip && !cull_reject(cr, c0)) pend0 = cm.x;
                 if (cm.y != skip && !cull_reject(cr, c1)) pend1 = cm.y;
                 chain = cm.z;
+                }
             }
         }
 

@@ -121,6 +121,7 @@ struct rg_scene : rg::DeviceContext {
     std::atomic<bool> busy{false};         // a render call is running on this handle (second callers get RG_E_BUSY)
     rg::DScene ds{};                    // device pointers inside
     rg::GridProxies gp{};               // boxes and disks binned into the grid (rg_scene.cuh)
+    rg::LightGrids lg{};                // per-light grids of the shadow rays (rg_light_grid.h)
     std::vector<rg::DLight> lights;        // every light, as uploaded (light_all): the host builds each light chunk's
                                            // DScene from these without reading the device
     std::vector<cudaTextureObject_t> tex_objs;
@@ -135,8 +136,9 @@ struct rg_scene : rg::DeviceContext {
     int verify_cull = 0;
     int overlap = 0;                       // RG_OPT_OVERLAP: 0 auto (on with the grid tracer), 1 off, 2 on
     int graph = 0;                         // RG_OPT_GRAPH: 0 auto, 1 off, 2 on
-    bool trace_stats = false;              // RG_OPT_TRACE_STATS
+    int trace_stats = 0;                   // RG_OPT_TRACE_STATS: 0 off, 1 every grid trace launch, 2 any-hit only, 3 nearest-hit only
     bool origin_hints = true;              // RG_OPT_ORIGIN_HINTS
+    bool light_grids = true;               // RG_OPT_LIGHT_GRIDS
     uint32_t supersample = 1;              // RG_OPT_SUPERSAMPLE: n x n samples per pixel (a multi-GPU handle keeps a copy
                                            // for its size checks)
     uint32_t depth_hint = 0;               // levels the ray tree of this scene has been seen to use (0 = unknown)
@@ -177,4 +179,6 @@ uint32_t multi_device_count(const rg_scene *sc);
 int multi_render_rows(rg_scene *sc, uint32_t w, uint32_t h, uint32_t y0, uint32_t y1, uint8_t *rgba_out, rg_stats *stats);
 // rg_grid.cu
 int grid_build(rg_scene *sc, const double *sph /* n x 4, host */, uint32_t n);
+// after grid_build: the light grids of the scene's first kLightGrids lights (none without the 3-D grid)
+int light_grid_build(rg_scene *sc, const double *sph /* n x 4, host */, uint32_t n);
 }  // namespace rg

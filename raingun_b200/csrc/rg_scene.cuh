@@ -107,6 +107,18 @@ struct GridProxies {
     const FaceRef *faces;         // [3][n_faces]: per axis k, (lo_k, box) and (hi_k, box) of every binned box, sorted by c
 };
 
+// Per-light grids for shadow rays (rg_light_grid.h, DESIGN.md section 4.2).  Only the any-hit k_trace_grid of a
+// light-major shadow queue reads this struct; like GridProxies it is a kernel argument of its own.
+struct LightGridInfo;
+struct LightGrids {
+    uint32_t n_lights;            // lights [0, n_lights) of the scene have a grid (0: none)
+    uint32_t first_light;         // scene index of the launch's first light (a light chunk's first)
+    const LightGridInfo *info;    // [n_lights]
+    const float4 *cell_rec;       // records in the grid's 48-byte format; record c is cell c's first, chained ones follow
+    const uint32_t *cell_start;   // [cells + 1]: the cells' lists in cell_items
+    const uint32_t *cell_items;   // item indices (into the sphere list), cell by cell
+};
+
 // Per recursion level of the wavefront loop (rg_wavefront.cu): every launch of a level reads its
 // size from here instead of from the host.  Zeroed at the start of a batch.
 struct DLevelCtr {

@@ -588,8 +588,10 @@ static bool brute_resident_fits(const rg_scene *sc) {
     return resident_smem_bytes(n_records, 4, 20) <= (size_t)kResidentSmemMax;
 }
 
+// first_light >= 0: `ta` is a light-major shadow queue whose first segment is that light of the scene (light grids
+// may serve it); -1: any other queue.
 template <bool ANY>
-static int launch_trace(rg_scene *sc, const TraceArgs &ta, bool use_grid, cudaStream_t stream) {
+static int launch_trace(rg_scene *sc, const TraceArgs &ta, bool use_grid, cudaStream_t stream, int first_light = -1) {
     if (ta.n == 0) return RG_OK;
     if (use_grid) {
         // persistent warps: enough blocks to fill the chip, each pulling rays from ta.fetch
@@ -601,13 +603,22 @@ static int launch_trace(rg_scene *sc, const TraceArgs &ta, bool use_grid, cudaSt
         const unsigned blocks = std::min<unsigned>(want, (unsigned)(sc->sm_count * bps));
         TraceArgs tuned = ta;
         tuned.g_refill = t_refill; tuned.g_quorum = t_quorum; tuned.g_burst = t_burst;
-        if (sc->gp.n_proxies) {   // boxes / disks in the grid
-            if (sc->trace_stats) k_trace_grid<ANY, true, true><<<blocks, kGridTraceThreads, 0, stream>>>(sc->ds, tuned, sc->gp);
-            else k_trace_grid<ANY, false, true><<<blocks, kGridTraceThreads, 0, stream>>>(sc->ds, tuned, sc->gp);
+        const bool stats = sc->trace_stats == 1 || sc->trace_stats == (ANY ? 2 : 3);
+        LightGrids lg = sc->lg;
+        lg.first_light = first_light >= 0 ? (uint32_t)first_light : 0u;
+        const bool light = ANY && sc->light_grids && first_light >= 0 && (uint32_t)first_light < lg.n_lights;
+#define RG_LAUNCH_GRID(S_, P_, L_) k_trace_grid<ANY, S_, P_, L_><<<blocks, kGridTraceThreads, 0, stream>>>(sc->ds, tuned, sc->gp, lg)
+        if (ANY && light) {   // (any-hit only: the nearest-hit kernels are never built with light grids)
+            if (sc->gp.n_proxies) { if (stats) RG_LAUNCH_GRID(true, true, ANY); else RG_LAUNCH_GRID(false, true, ANY); }
+            else { if (stats) RG_LAUNCH_GRID(true, false, ANY); else RG_LAUNCH_GRID(false, false, ANY); }
+        } else if (sc->gp.n_proxies) {   // boxes / disks in the grid
+            if (stats) RG_LAUNCH_GRID(true, true, false);
+            else RG_LAUNCH_GRID(false, true, false);
         } else {
-            if (sc->trace_stats) k_trace_grid<ANY, true><<<blocks, kGridTraceThreads, 0, stream>>>(sc->ds, tuned, sc->gp);
-            else k_trace_grid<ANY, false><<<blocks, kGridTraceThreads, 0, stream>>>(sc->ds, tuned, sc->gp);
+            if (stats) RG_LAUNCH_GRID(true, false, false);
+            else RG_LAUNCH_GRID(false, false, false);
         }
+#undef RG_LAUNCH_GRID
     } else if (brute_resident_fits(sc) && ta.n >= (uint32_t)sc->sm_count * 64u * 32u) {
         // the whole cull array fits in one SM's shared memory: one persistent CTA per SM, warps
         // pull ray tiles from a counter and never meet at a barrier again (rg_trace.cuh)
@@ -872,7 +883,7 @@ static int enqueue_batch_dev(rg_scene *sc, const DevPlan &plan, uint32_t width, 
                 sa.ctr = dc;
                 sa.verify = sc->verify_cull == 1;
                 if (events) { e0 = events->get(); e1 = events->get(); RG_CUDA(cudaEventRecord(e0, aux)); }
-                if ((rc = launch_trace<true>(sc, sa, use_grid, aux))) return rc;
+                if ((rc = launch_trace<true>(sc, sa, use_grid, aux, light_major ? (int)(c * kLightChunk) : -1))) return rc;
                 if (events) { RG_CUDA(cudaEventRecord(e1, aux)); trace_spans->emplace_back(e0, e1); }
                 st->gpu_launches++;
                 if (sc->verify_cull >= 2) k_verify_trace<true><<<(sa.n + 127) / 128, 128, 0, aux>>>(cs, sa, (int)d);
@@ -928,7 +939,7 @@ static std::vector<uint64_t> graph_key(const rg_scene *sc, const DevPlan &plan, 
     const WavefrontScratch &wf = sc->wf;
     std::vector<uint64_t> k = {width, height, y0, npix, (uint64_t)(uintptr_t)d_rows, (uint64_t)(uintptr_t)d_out,
                                (uint64_t)use_grid, (uint64_t)kind, (uint64_t)sc->ds.max_depth, (uint64_t)sc->overlap,
-                               (uint64_t)sc->verify_cull, (uint64_t)sc->trace_stats | ((uint64_t)sc->origin_hints << 1), (uint64_t)plan.levels,
+                               (uint64_t)sc->verify_cull, (uint64_t)sc->trace_stats | ((uint64_t)sc->origin_hints << 2) | ((uint64_t)sc->light_grids << 3), (uint64_t)plan.levels,
                                (uint64_t)sc->level_growth,    // the capacities are baked into the captured launches
                                (uint64_t)sc->supersample};    // the last launch: (n, w, h) and (1, n w, n h) share a sample space
     auto add = [&](const DeviceBuffer &b) { k.push_back((uint64_t)(uintptr_t)b.ptr); };
