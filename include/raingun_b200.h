@@ -161,9 +161,24 @@ enum {
                                 avg = s / (n*n), rounded to nearest.  The RGBA8 entry points store Color::rgba(avg)
                                 (color.rs:32-37), the f32 ones avg.  Output buffers keep their sizes; the ray and error
                                 counters count every sample's rays.  (n*w)*(n*h) must fit in u32, else RG_E_TOO_LARGE. */
-    RG_OPT_LIGHT_GRIDS = 15  /* 1 (default) = the grid tracer traces the shadow rays of a scene's first 8 lights through
+    RG_OPT_LIGHT_GRIDS = 15, /* 1 (default) = the grid tracer traces the shadow rays of a scene's first 8 lights through
                                 per-light 2-D grids (one short list per ray instead of a 3-D walk); 0 = the 3-D walk for
                                 every ray.  Results unchanged (DESIGN.md section 4.2) */
+    RG_OPT_SUPERSAMPLE_EDGES = 16 /* edge-adaptive RG_OPT_SUPERSAMPLE: -1 (default) = off, every pixel gets n x n samples;
+                                T = 0 ... 255 = only pixels on an edge of the reference frame do; anything else is
+                                RG_E_INVALID.  No effect with n = 1.  With n > 1 and T >= 0, for a (w x h) image:
+                                R is the reference's own RGBA8 frame of the WHOLE image (Color::rgba of
+                                create_prime(x, y, w, h), the n = 1 frame).  Pixel (x, y) is refined iff some
+                                8-neighbour (x + dx, y + dy) inside the image has |R(x,y)_c - R(x+dx,y+dy)_c| > T, in
+                                integer bytes, for some c in r, g, b (alpha is ignored; a NaN colour is 0 in R).  A
+                                refined pixel is what RG_OPT_SUPERSAMPLE = n delivers for it; any other pixel is the
+                                n = 1 pixel (R's bytes, or its f32 colour).  The mask is a function of the whole frame:
+                                every entry point (row ranges, row lists in any order with duplicates, scatter, host,
+                                device, f32, streaming, multi-GPU at any tile height) gives the pixels of a full-frame
+                                render.  Counters count every ray traced: with R' = the requested rows and their
+                                in-image neighbours y +- 1, once each, rays_primary = |R'| w + n*n (refined requested
+                                pixels), the other counters those rays' trees.  Output sizes, refusals and size checks
+                                are those of RG_OPT_SUPERSAMPLE (DESIGN.md section 4.6) */
 };
 
 /* Counters and timings of one render call.  A "ray" is one `Scene::trace`

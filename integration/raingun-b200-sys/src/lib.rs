@@ -47,6 +47,7 @@ pub const RG_OPT_TILE_ROWS: i32 = 12;
 pub const RG_OPT_ORIGIN_HINTS: i32 = 13;
 pub const RG_OPT_SUPERSAMPLE: i32 = 14; // n x n primary rays per pixel (1-8), box-filtered on the device
 pub const RG_OPT_LIGHT_GRIDS: i32 = 15; // shadow rays through per-light 2-D grids (default 1)
+pub const RG_OPT_SUPERSAMPLE_EDGES: i32 = 16; // -1 (default) off, T in 0..=255: supersample only edge pixels
 
 #[repr(C)]
 pub struct rg_texture_desc {

@@ -158,6 +158,13 @@ class Scene:
         default) is the reference's own frame."""
         self.set_option(_native.OPT_SUPERSAMPLE, n)
 
+    def set_supersample_edges(self, t: Optional[int]) -> None:
+        """Edge-adaptive anti-aliasing (RG_OPT_SUPERSAMPLE_EDGES): with ``set_supersample(n)``, n > 1, only pixels on an
+        edge of the reference's own frame get their n x n samples: a pixel whose r, g or b byte differs by more than
+        ``t`` (0 <= t <= 255) from one of its 8 neighbours in that frame.  Every other pixel is the reference's pixel.
+        ``None`` (the default) supersamples every pixel."""
+        self.set_option(_native.OPT_SUPERSAMPLE_EDGES, -1 if t is None else t)
+
     # -- Scene::render_image (scene.rs:41-43)
     def render_image(self, width: int, height: int, out: Optional[np.ndarray] = None) -> np.ndarray:
         return self.render_rows(width, height, 0, height, out)

@@ -26,7 +26,7 @@ PIPELINE_WAVEFRONT, PIPELINE_MEGAKERNEL, PIPELINE_AUTO = 0, 1, 2
 ACCEL_AUTO, ACCEL_BRUTE, ACCEL_GRID = 0, 1, 2
 OPT_PIPELINE, OPT_ACCEL, OPT_MAX_DEPTH, OPT_BATCH_PIXELS, OPT_VERIFY_CULL, OPT_OVERLAP = 1, 2, 3, 4, 5, 6
 OPT_HOST_FREE, OPT_GRAPH, OPT_TRACE_STATS, OPT_SCHEDULE, OPT_TILE_ROWS, OPT_ORIGIN_HINTS = 7, 8, 9, 11, 12, 13
-OPT_SUPERSAMPLE, OPT_LIGHT_GRIDS = 14, 15
+OPT_SUPERSAMPLE, OPT_LIGHT_GRIDS, OPT_SUPERSAMPLE_EDGES = 14, 15, 16
 
 ROWS_CB = ctypes.CFUNCTYPE(ctypes.c_int, ctypes.c_uint32, ctypes.c_uint32, ctypes.c_uint32,
                            ctypes.POINTER(ctypes.c_uint8), ctypes.c_void_p)

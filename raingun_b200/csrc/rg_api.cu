@@ -94,6 +94,7 @@ void DeviceContext::release() {
     frame.release();
     rowlist.release();
     samples.release();
+    edge_ref.release(); edge_rows.release(); edge_flag.release(); edge_list.release();
     arena.release();
     if (d_counters) cudaFree(d_counters);
     if (h_counters) cudaFreeHost(h_counters);
@@ -706,6 +707,10 @@ int rg_scene_set_option(rg_scene *sc, int32_t key, int64_t value) {
             if (value < 1 || value > 8) break;
             sc->supersample = (uint32_t)value;
             return RG_OK;
+        case RG_OPT_SUPERSAMPLE_EDGES:
+            if (value < -1 || value > 255) break;
+            sc->supersample_edges = (int)value;
+            return RG_OK;
         default: break;
     }
     set_error("bad option key %d / value %lld", key, (long long)value);
@@ -731,10 +736,10 @@ static int check_dims(rg_scene *sc, uint32_t w, uint32_t h, uint32_t y0, uint32_
     return RG_OK;
 }
 
+// n x n samples per pixel; with `list` (RG_OPT_SUPERSAMPLE_EDGES), the listed refined pixels instead of rows [y0, y1).
 static int mega_render(rg_scene *sc, uint32_t w, uint32_t h, uint32_t y0, uint32_t y1, const uint32_t *d_rows,
-                       OutKind kind, uchar4 *d_out, cudaStream_t stream, rg_stats *st) {
-    const uint64_t npix = (uint64_t)(y1 - y0) * w;
-    const uint32_t n = sc->supersample;
+                       OutKind kind, uchar4 *d_out, cudaStream_t stream, rg_stats *st, uint32_t n, const EdgeList *list) {
+    const uint64_t npix = list ? list->count : (uint64_t)(y1 - y0) * w;
     uint32_t launches = 0;
     int rc;
     RG_CUDA(cudaMemsetAsync(sc->d_counters, 0, sizeof(DCounters), stream));
@@ -742,7 +747,25 @@ static int mega_render(rg_scene *sc, uint32_t w, uint32_t h, uint32_t y0, uint32
     if (npix) {
         auto kernel = sc->ds.max_depth <= 12 ? k_render_mega<12, false> : k_render_mega<RG_MAX_DEPTH, false>;
         if (sc->ds.n_lights > RG_MAX_LIGHTS) kernel = sc->ds.max_depth <= 12 ? k_render_mega<12, true> : k_render_mega<RG_MAX_DEPTH, true>;
-        if (n == 1) {
+        if (list) {
+            // the samples of bands of whole refined pixels, pixel-major into sc->samples (at most RG_OPT_BATCH_PIXELS
+            // samples, default 16M), each band averaged by k_resolve_list
+            auto lkernel = sc->ds.max_depth <= 12 ? k_render_mega_list<12, false> : k_render_mega_list<RG_MAX_DEPTH, false>;
+            if (sc->ds.n_lights > RG_MAX_LIGHTS)
+                lkernel = sc->ds.max_depth <= 12 ? k_render_mega_list<12, true> : k_render_mega_list<RG_MAX_DEPTH, true>;
+            const uint64_t band_samples = sc->batch_pixels ? sc->batch_pixels : (16ull << 20), nn = (uint64_t)n * n;
+            const uint32_t band = (uint32_t)std::max<uint64_t>(1, std::min<uint64_t>(list->count, band_samples / nn));
+            if ((rc = sc->samples.reserve((size_t)band * nn * 12))) return rc;
+            float *samples = sc->samples.as<float>();
+            for (uint32_t e = 0; e < list->count; e += band) {
+                const uint32_t cnt = std::min(band, list->count - e);
+                lkernel<<<(unsigned)((cnt * nn + 127) / 128), 128, 0, stream>>>(sc->ds, w, h, n, list->entries + e, cnt, list->req_rows,
+                                                                               samples, sc->d_counters);
+                RG_CUDA(cudaGetLastError());
+                if ((rc = launch_resolve_list(kind, samples, 3, n, w, list->entries + e, cnt, list->req_rows, d_out, stream))) return rc;
+                launches += 2;
+            }
+        } else if (n == 1) {
             const unsigned blocks = (unsigned)((npix + 127) / 128);
             float *f32 = kind == OutKind::F32 ? reinterpret_cast<float *>(d_out) : nullptr;
             kernel<<<blocks, 128, 0, stream>>>(sc->ds, w, h, y0, y1, d_rows, d_out, f32, sc->d_counters);
@@ -793,26 +816,127 @@ static int mega_render(rg_scene *sc, uint32_t w, uint32_t h, uint32_t y0, uint32
     return RG_OK;
 }
 
-// Common tail of the device-output entry points: rows [y0, y1), or entries [0, n) of a row list.
-static int render_device(rg_scene *sc, uint32_t w, uint32_t h, uint32_t y0, uint32_t y1, const uint32_t *d_rows,
-                         OutKind kind, void *d_out, cudaStream_t stream, rg_stats *stats) {
+// RG_PIPELINE_AUTO: with a handful of bodies the per-pixel recursion (every body tested in FP64, no queues)
+// beats the wavefront at every image size (measured on the shipped examples, 800x600 .. 4K: 2-3x);
+// the crossover lies near kMegaAutoBodies bodies (RG_MEGA_AUTO_BODIES for tuning runs)
+static bool use_mega(const rg_scene *sc, OutKind kind) {
+    static const uint32_t mega_auto_bodies = [] { const char *e = getenv("RG_MEGA_AUTO_BODIES"); return e ? (uint32_t)atoi(e) : kMegaAutoBodies; }();
+    return sc->pipeline == RG_PIPELINE_MEGAKERNEL ||
+           (sc->pipeline == RG_PIPELINE_AUTO && !is_scatter(kind) && sc->n_bodies <= mega_auto_bodies && sc->verify_cull == 0);
+}
+
+// Rows [y0, y1), entries [y0, y1) of a row list, or the pixels of `list`, at n x n samples per pixel, on the megakernel
+// or the wavefront pipeline.
+static int render_pass(rg_scene *sc, uint32_t w, uint32_t h, uint32_t y0, uint32_t y1, const uint32_t *d_rows, OutKind kind,
+                       void *d_out, cudaStream_t stream, rg_stats *stats, uint32_t n, bool mega, const EdgeList *list = nullptr) {
     auto t0 = std::chrono::steady_clock::now();
     rg_stats local;
     std::memset(&local, 0, sizeof(local));
     int rc;
-    // RG_PIPELINE_AUTO: with a handful of bodies the per-pixel recursion (every body tested in FP64, no queues)
-    // beats the wavefront at every image size (measured on the shipped examples, 800x600 .. 4K: 2-3x);
-    // the crossover lies near kMegaAutoBodies bodies (RG_MEGA_AUTO_BODIES for tuning runs)
-    static const uint32_t mega_auto_bodies = [] { const char *e = getenv("RG_MEGA_AUTO_BODIES"); return e ? (uint32_t)atoi(e) : kMegaAutoBodies; }();
-    const bool mega = sc->pipeline == RG_PIPELINE_MEGAKERNEL ||
-                      (sc->pipeline == RG_PIPELINE_AUTO && !is_scatter(kind) && sc->n_bodies <= mega_auto_bodies && sc->verify_cull == 0);
-    if (mega) rc = mega_render(sc, w, h, y0, y1, d_rows, kind, (uchar4 *)d_out, stream, &local);
-    else rc = wavefront_render(sc, w, h, y0, y1, d_rows, kind, (uchar4 *)d_out, stream, &local);
+    if (mega) rc = mega_render(sc, w, h, y0, y1, d_rows, kind, (uchar4 *)d_out, stream, &local, n, list);
+    else rc = wavefront_render(sc, w, h, y0, y1, d_rows, kind, (uchar4 *)d_out, stream, &local, n, list);
     local.pipeline_used = mega ? RG_PIPELINE_MEGAKERNEL : RG_PIPELINE_WAVEFRONT;
     local.devices_used = 1;
     local.ms_wall = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count();
     if (stats) *stats = local;
     return rc;
+}
+
+// Common tail of the device-output entry points: rows [y0, y1), or entries [0, n) of a row list.
+static int render_device(rg_scene *sc, uint32_t w, uint32_t h, uint32_t y0, uint32_t y1, const uint32_t *d_rows,
+                         OutKind kind, void *d_out, cudaStream_t stream, rg_stats *stats) {
+    return render_pass(sc, w, h, y0, y1, d_rows, kind, d_out, stream, stats, sc->supersample, use_mega(sc, kind));
+}
+
+static bool adaptive(const rg_scene *sc) { return sc->supersample > 1 && sc->supersample_edges >= 0; }
+
+// RG_OPT_SUPERSAMPLE_EDGES (include/raingun_b200.h, DESIGN.md section 4.6): the requested rows — rows [y0, y1), or, when
+// `rows` (host memory) is given, the n_rows listed rows — with n x n samples only where the reference frame has an edge.
+// 1. the reference pass: R' = the requested rows and their neighbours in the image, once each, at n = 1 as f32 into
+//    sc->edge_ref (a row range stays a range; a list becomes the sorted list of the rows of R');
+// 2. k_edge_emit / k_edge_scan / k_edge_compact: the mask; unrefined pixels get their reference value, refined ones go
+//    to a list in row-major order; one read-back of their count;
+// 3. the refined pixels' samples, in batches of whole pixels, each batch ending in k_resolve_list.
+// Every output pixel is written by exactly one of k_edge_emit and k_resolve_list.  A phase whose frame is repeated
+// (queue overflow, depth hint) repeats inside its own wavefront_render, resolve included.
+static int adaptive_render(rg_scene *sc, uint32_t w, uint32_t h, uint32_t y0, uint32_t y1, const uint32_t *rows, uint32_t n_rows,
+                           OutKind kind, void *d_out, cudaStream_t stream, rg_stats *stats) {
+    auto t0 = std::chrono::steady_clock::now();
+    const uint32_t K = rows ? n_rows : y1 - y0;
+    const uint32_t n = sc->supersample;
+    const bool mega = use_mega(sc, kind);
+    int rc;
+    // host side of R': the sorted image rows, each requested row's neighbours as rows of R' (-1 outside the image)
+    std::vector<uint32_t> meta;   // [req_rows: K][nb: 3 K][R' rows]
+    std::vector<int32_t> pos(h, -1);
+    uint32_t ra = 0, rb = 0;      // a row range: R' = [ra, rb)
+    if (rows) {
+        std::vector<char> in(h, 0);
+        for (uint32_t k = 0; k < K; ++k)
+            for (int d = -1; d <= 1; ++d) {
+                const int64_t y = (int64_t)rows[k] + d;
+                if (y >= 0 && y < (int64_t)h) in[(size_t)y] = 1;
+            }
+        meta.resize((size_t)4 * K);
+        for (uint32_t y = 0; y < h; ++y)
+            if (in[y]) { pos[y] = (int32_t)(meta.size() - (size_t)4 * K); meta.push_back(y); }
+    } else {
+        ra = y0 > 0 ? y0 - 1 : 0;
+        rb = y1 < h ? y1 + 1 : h;
+        for (uint32_t y = ra; y < rb; ++y) pos[y] = (int32_t)(y - ra);
+        meta.resize((size_t)4 * K);
+    }
+    const uint32_t n_ref = rows ? (uint32_t)(meta.size() - (size_t)4 * K) : rb - ra;
+    for (uint32_t k = 0; k < K; ++k) {
+        const uint32_t y = rows ? rows[k] : y0 + k;
+        meta[k] = y;
+        for (int d = -1; d <= 1; ++d) {
+            const int64_t yy = (int64_t)y + d;
+            meta[(size_t)K + 3 * k + (d + 1)] = (uint32_t)(yy >= 0 && yy < (int64_t)h ? pos[(size_t)yy] : -1);
+        }
+    }
+    const uint64_t npix = (uint64_t)K * w;
+    if (npix > 0xFFFFFFFFull) { set_error("%u rows of %u pixels are too many for one call", K, w); return RG_E_TOO_LARGE; }
+    const uint32_t blocks = (uint32_t)((npix + 255) / 256);
+    if ((rc = sc->edge_ref.reserve((size_t)n_ref * w * 12))) return rc;
+    if ((rc = sc->edge_rows.reserve(meta.size() * 4))) return rc;
+    if ((rc = sc->edge_flag.reserve(npix + 16 + ((size_t)blocks + 1) * 4))) return rc;
+    if ((rc = sc->edge_list.reserve(npix * 8))) return rc;
+    uint32_t *d_meta = sc->edge_rows.as<uint32_t>();
+    RG_CUDA(cudaMemcpyAsync(d_meta, meta.data(), meta.size() * 4, cudaMemcpyHostToDevice, stream));
+    RG_CUDA(cudaStreamSynchronize(stream));   // `meta` goes away; `rows` may be pageable and reused by the caller
+    const uint32_t *req_rows = d_meta;
+    const int32_t *nb = reinterpret_cast<const int32_t *>(d_meta + K);
+    uint8_t *flag = sc->edge_flag.as<uint8_t>();
+    uint32_t *block_count = reinterpret_cast<uint32_t *>(flag + ((npix + 15) & ~(uint64_t)15));
+    uint2 *list = sc->edge_list.as<uint2>();
+
+    rg_stats total, part;
+    std::memset(&total, 0, sizeof total);
+    // 1. the reference pass: the ordinary n = 1 render of R' (its batches replay the n = 1 graphs of that shape)
+    float *ref = sc->edge_ref.as<float>();
+    if (rows) rc = render_pass(sc, w, h, 0, n_ref, d_meta + 4 * (size_t)K, OutKind::F32, ref, stream, &part, 1, mega);
+    else rc = render_pass(sc, w, h, ra, rb, nullptr, OutKind::F32, ref, stream, &part, 1, mega);
+    if (rc) return rc;
+    merge_stats(total, part, false);
+    // 2. mask, emit, compact
+    if ((rc = launch_edge_mask(kind, ref, nb, w, (uint32_t)npix, (uint32_t)sc->supersample_edges, req_rows, d_out, flag, block_count,
+                               list, stream)))
+        return rc;
+    uint32_t refined = 0;
+    RG_CUDA(cudaMemcpyAsync(&refined, block_count + blocks, 4, cudaMemcpyDeviceToHost, stream));
+    RG_CUDA(cudaStreamSynchronize(stream));
+    total.gpu_launches += 3;
+    // 3. the refined pixels
+    if (refined) {
+        const EdgeList el{list, refined, req_rows};
+        if ((rc = render_pass(sc, w, h, 0, 0, nullptr, kind, d_out, stream, &part, n, mega, &el))) return rc;
+        merge_stats(total, part, false);
+    }
+    total.devices_used = 1;
+    total.ms_wall = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count();
+    if (stats) *stats = total;
+    return RG_OK;
 }
 
 static int single_device_only(const rg_scene *sc, const char *what) {
@@ -829,6 +953,7 @@ int render_rowlist_device(rg_scene *sc, uint32_t w, uint32_t h, const uint32_t *
     for (uint32_t k = 0; k < n_rows; ++k)
         if (rows[k] >= h) { set_error("rows[%u] = %u is outside the image (height %u)", k, rows[k], h); return RG_E_INVALID; }
     RG_CUDA(cudaSetDevice(sc->device));
+    if (adaptive(sc) && n_rows) return adaptive_render(sc, w, h, 0, 0, rows, n_rows, kind, d_out, stream, stats);
     std::vector<uint32_t> sample_rows;   // RG_OPT_SUPERSAMPLE = n > 1: listed row r is sample rows n r, ..., n r + n - 1
     const uint32_t n = sc->supersample;
     if (n > 1) {
@@ -889,7 +1014,9 @@ static int render_rows_host(rg_scene *sc, uint32_t w, uint32_t h, uint32_t y0, u
     const size_t bytes = (size_t)(y1 - y0) * w * bytes_per_pixel(kind);
     if ((rc = sc->frame.reserve(bytes ? bytes : 4))) return rc;
     rg_stats local;
-    if ((rc = render_device(sc, w, h, y0, y1, nullptr, kind, sc->frame.ptr, sc->stream, &local))) return rc;
+    if (adaptive(sc) && y1 > y0) rc = adaptive_render(sc, w, h, y0, y1, nullptr, 0, kind, sc->frame.ptr, sc->stream, &local);
+    else rc = render_device(sc, w, h, y0, y1, nullptr, kind, sc->frame.ptr, sc->stream, &local);
+    if (rc) return rc;
     if (bytes) {
         RG_CUDA(cudaMemcpyAsync(host, sc->frame.ptr, bytes, cudaMemcpyDeviceToHost, sc->stream));
         RG_CUDA(cudaStreamSynchronize(sc->stream));
@@ -1002,6 +1129,8 @@ static int render_rows_device(rg_scene *sc, uint32_t w, uint32_t h, uint32_t y0,
     if ((rc = single_device_only(sc, "rg_render_rows_device"))) return rc;
     if (!d_out && y1 > y0) { set_error("output pointer is NULL"); return RG_E_INVALID; }
     RG_CUDA(cudaSetDevice(sc->device));
+    if (adaptive(sc) && y1 > y0)
+        return adaptive_render(sc, w, h, y0, y1, nullptr, 0, kind, d_out, reinterpret_cast<cudaStream_t>(cuda_stream), stats);
     return render_device(sc, w, h, y0, y1, nullptr, kind, d_out, reinterpret_cast<cudaStream_t>(cuda_stream), stats);
 }
 // rg_render_rowlist_scatter (kind Rgba8Scatter) and rg_render_rowlist_f32_scatter (F32Scatter), inside the guard

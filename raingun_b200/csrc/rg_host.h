@@ -89,6 +89,11 @@ struct DeviceContext {
     DeviceBuffer frame;                // staging of host-buffer renders
     DeviceBuffer rowlist;              // device copy of a caller's row list
     DeviceBuffer samples;              // megakernel with RG_OPT_SUPERSAMPLE > 1: f32 RGB of a band of samples
+    // RG_OPT_SUPERSAMPLE_EDGES (rg_api.cu adaptive_render)
+    DeviceBuffer edge_ref;             // the reference frame of the requested rows and their neighbours: f32 RGB
+    DeviceBuffer edge_rows;            // requested rows, their neighbours' rows in edge_ref, and those rows' image rows
+    DeviceBuffer edge_flag;            // per requested pixel: refined; then per emit block: refined count / offset
+    DeviceBuffer edge_list;            // the refined pixels (EdgeList)
     SceneArena arena;                  // scene arrays
     DCounters *d_counters = nullptr;
     DCounters *h_counters = nullptr;   // pinned
@@ -99,6 +104,14 @@ struct DeviceContext {
     // every handle exists: a create() that failed half-way must not hand its holes to the next scene
     bool complete() const { return stream && d_counters && h_counters && ev[0] && ev[1] && ev[2] && ev[3]; }
     void release();                    // frees everything; the context's device must be current
+};
+
+// RG_OPT_SUPERSAMPLE_EDGES: the refined pixels of an adaptive frame (rg_api.cu adaptive_render), in device memory.
+// Entry (k, x) is column x of the call's k-th requested row, which is image row req_rows[k].
+struct EdgeList {
+    const uint2 *entries;
+    uint32_t count;
+    const uint32_t *req_rows;
 };
 
 // What a render call delivers: RGBA8 rows in order, RGBA8 rows stored at their place in a full frame
@@ -141,6 +154,7 @@ struct rg_scene : rg::DeviceContext {
     bool light_grids = true;               // RG_OPT_LIGHT_GRIDS
     uint32_t supersample = 1;              // RG_OPT_SUPERSAMPLE: n x n samples per pixel (a multi-GPU handle keeps a copy
                                            // for its size checks)
+    int supersample_edges = -1;            // RG_OPT_SUPERSAMPLE_EDGES: -1 off, else the mask's threshold T (0 ... 255)
     uint32_t depth_hint = 0;               // levels the ray tree of this scene has been seen to use (0 = unknown)
     uint32_t level_growth = 2;             // wavefront queue of level d holds min(2^d, level_growth) x the batch's pixels;
                                            // doubled when a level outgrows its queue (the frame is then repeated)
@@ -151,15 +165,25 @@ struct rg_scene : rg::DeviceContext {
 
 namespace rg {
 // rg_wavefront.cu
-// rows [y0, y1) of the image, or — when d_rows is given — entries [y0, y1) of that row list.  With
-// RG_OPT_SUPERSAMPLE = n > 1, d_rows is the expanded list of sample rows, n per listed row (render_rowlist_device).
+// rows [y0, y1) of the image, or — when d_rows is given — entries [y0, y1) of that row list, at n x n samples per
+// pixel (n > 1: d_rows is the expanded list of sample rows, n per listed row, render_rowlist_device).  With `list`, the
+// refined pixels of an adaptive frame instead (y0, y1 and d_rows unused), each stored at its place (EdgeList).
 int wavefront_render(rg_scene *sc, uint32_t width, uint32_t height, uint32_t y0, uint32_t y1,
-                     const uint32_t *d_rows, OutKind kind, uchar4 *d_out, cudaStream_t stream, rg_stats *st);
+                     const uint32_t *d_rows, OutKind kind, uchar4 *d_out, cudaStream_t stream, rg_stats *st, uint32_t n,
+                     const EdgeList *list = nullptr);
 // RG_OPT_SUPERSAMPLE = n > 1: writes `out_rows` output rows of `width` pixels, each the average of its n x n samples,
 // which are f32 RGB at src + stride * i, i in the order of the level-0 queue with strips of `strip` rows over the
 // batch's n out_rows sample rows (strip 1: row-major).  Scatter: output row r goes to image row d_rows[row0 + r n] / n.
 int launch_resolve(OutKind kind, const float *src, uint32_t stride, uint32_t strip, uint32_t n, uint32_t width, uint32_t out_rows,
                    const uint32_t *d_rows, uint32_t row0, void *out, cudaStream_t stream);
+// RG_OPT_SUPERSAMPLE_EDGES: stores the average of each listed pixel's n x n samples (f32 RGB at src + stride * i, pixel-
+// major, sub-row-major) at the pixel's place: row k of `out`, or image row req_rows[k] of a full frame (scatter kinds)
+int launch_resolve_list(OutKind kind, const float *src, uint32_t stride, uint32_t n, uint32_t width, const uint2 *list, uint32_t count,
+                        const uint32_t *req_rows, void *out, cudaStream_t stream);
+// RG_OPT_SUPERSAMPLE_EDGES: mask, emit and compact over the npix = K width requested pixels (k_edge_emit): the unrefined
+// pixels get their reference value in `out`, the refined ones go to `list`, their count to block_count[(npix + 255) / 256]
+int launch_edge_mask(OutKind kind, const float *ref, const int32_t *nb, uint32_t width, uint32_t npix, uint32_t t,
+                     const uint32_t *req_rows, void *out, uint8_t *flag, uint32_t *block_count, uint2 *list, cudaStream_t stream);
 // rg_api.cu
 // rg_render_rowlist_device / rg_render_rowlist_f32_device (kind Rgba8 / F32) and rg_render_rowlist_scatter /
 // rg_render_rowlist_f32_scatter (Rgba8Scatter / F32Scatter) without the one-render-at-a-time guard (for callers that hold it)

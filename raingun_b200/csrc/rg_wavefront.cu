@@ -511,6 +511,184 @@ int launch_resolve(OutKind kind, const float *src, uint32_t stride, uint32_t str
     return RG_OK;
 }
 
+// ---- RG_OPT_SUPERSAMPLE_EDGES (include/raingun_b200.h, DESIGN.md section 4.6) --------------------------------------
+// The level-0 queue of a batch of refined pixels: n x n rays per listed pixel (entry (k, x): column x of image row
+// req_rows[k]), pixel-major and sub-row-major, as create_prime(n x + i, n y + j, n w, n h) of the sample image.
+__global__ void __launch_bounds__(256) k_generate_list(const DScene s, RayQueue q, uint32_t width, uint32_t height, uint32_t n,
+                                                       const uint2 *__restrict__ list, uint32_t npix,
+                                                       const uint32_t *__restrict__ req_rows, unsigned int *n_level0) {
+    const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i == 0) *n_level0 = npix;
+    if (i >= npix) return;
+    const uint32_t nn = n * n, e = i / nn, sub = i - e * nn, j = sub / n, si = sub - j * n;
+    const uint2 p = list[e];
+    store_ray(q, i, create_prime(s, n * p.y + si, n * req_rows[p.x] + j, n * width, n * height));
+    q.hint[i] = kHintNone;   // camera rays start on no body
+}
+
+// The place of requested pixel (k, x) in the output: row k of the batch, or image row req_rows[k] of a full frame.
+template <OutKind K>
+__device__ __forceinline__ size_t edge_place(uint32_t k, uint32_t x, uint32_t width, const uint32_t *req_rows) {
+    return (size_t)(is_scatter(K) ? req_rows[k] : k) * width + x;
+}
+template <OutKind K>
+__device__ __forceinline__ void edge_store(void *out, size_t o, C3 c) {
+    if constexpr (K == OutKind::F32 || K == OutKind::F32Scatter) {
+        float *d = static_cast<float *>(out) + 3 * o;
+        d[0] = c.r; d[1] = c.g; d[2] = c.b;
+    } else {
+        static_cast<uchar4 *>(out)[o] = quantise(c);
+    }
+}
+
+// The last kernel of a batch of refined pixels: one thread per pixel sums its n x n samples (f32 RGB at
+// src + stride * (e n n + j n + i), the order k_generate_list / k_render_mega_list made them) in the contract's order,
+// exactly as k_resolve_ss, and stores the average at the pixel's place.
+template <OutKind K>
+__global__ void __launch_bounds__(256) k_resolve_list(const float *__restrict__ src, uint32_t stride, uint32_t n, uint32_t width,
+                                                      const uint2 *__restrict__ list, uint32_t count,
+                                                      const uint32_t *__restrict__ req_rows, void *out) {
+    const uint32_t e = blockIdx.x * blockDim.x + threadIdx.x;
+    if (e >= count) return;
+    const size_t first = (size_t)e * n * n;
+    float s[3] = {0.0f, 0.0f, 0.0f};
+    for (uint32_t j = 0; j < n; ++j)
+        for (uint32_t i = 0; i < n; ++i) {
+            const float *c = src + (size_t)stride * (first + j * n + i);
+            float v[3];
+            if (stride == 4) { const float4 a = *reinterpret_cast<const float4 *>(c); v[0] = a.x; v[1] = a.y; v[2] = a.z; }
+            else { v[0] = c[0]; v[1] = c[1]; v[2] = c[2]; }
+#pragma unroll
+            for (int k = 0; k < 3; ++k) s[k] = __fadd_rn(s[k], v[k]);
+        }
+    const float nn = (float)(n * n);
+    const uint2 p = list[e];
+    edge_store<K>(out, edge_place<K>(p.x, p.y, width, req_rows), c3(__fdiv_rn(s[0], nn), __fdiv_rn(s[1], nn), __fdiv_rn(s[2], nn)));
+}
+
+int launch_resolve_list(OutKind kind, const float *src, uint32_t stride, uint32_t n, uint32_t width, const uint2 *list, uint32_t count,
+                        const uint32_t *req_rows, void *out, cudaStream_t stream) {
+    if (count == 0) return RG_OK;
+    const unsigned blocks = (count + 255) / 256;
+    switch (kind) {
+        case OutKind::Rgba8: k_resolve_list<OutKind::Rgba8><<<blocks, 256, 0, stream>>>(src, stride, n, width, list, count, req_rows, out); break;
+        case OutKind::Rgba8Scatter: k_resolve_list<OutKind::Rgba8Scatter><<<blocks, 256, 0, stream>>>(src, stride, n, width, list, count, req_rows, out); break;
+        case OutKind::F32: k_resolve_list<OutKind::F32><<<blocks, 256, 0, stream>>>(src, stride, n, width, list, count, req_rows, out); break;
+        case OutKind::F32Scatter: k_resolve_list<OutKind::F32Scatter><<<blocks, 256, 0, stream>>>(src, stride, n, width, list, count, req_rows, out); break;
+    }
+    RG_CUDA(cudaGetLastError());
+    return RG_OK;
+}
+
+// The mask.  One thread per requested pixel (k, x): its 3 x 3 neighbourhood in the reference frame `ref` (f32 RGB,
+// row r of R' at ref + 3 r width), whose rows y - 1, y, y + 1 are rows nb[3 k], nb[3 k + 1], nb[3 k + 2] of R'
+// (-1: outside the image), quantised with Color::rgba.  The pixel is refined iff a neighbour differs from it by more
+// than `t` in r, g or b.  An unrefined pixel gets its reference value here; a refined one is left to k_resolve_list.
+// flag[p] = refined, block_count[b] = refined pixels of block b (k_edge_scan turns them into offsets).
+template <OutKind K>
+__global__ void __launch_bounds__(256) k_edge_emit(const float *__restrict__ ref, const int32_t *__restrict__ nb, uint32_t width,
+                                                   uint32_t npix, uint32_t t, const uint32_t *__restrict__ req_rows, void *out,
+                                                   uint8_t *flag, uint32_t *block_count) {
+    const uint32_t p = blockIdx.x * blockDim.x + threadIdx.x;
+    bool refined = false;
+    if (p < npix) {
+        const uint32_t k = p / width, x = p - k * width;
+        const int32_t r[3] = {nb[3 * (size_t)k], nb[3 * (size_t)k + 1], nb[3 * (size_t)k + 2]};
+        const float *c = ref + 3 * ((size_t)r[1] * width + x);
+        const C3 centre = c3(c[0], c[1], c[2]);
+        const uchar4 q = quantise(centre);
+        for (int dy = 0; dy < 3; ++dy) {
+            if (r[dy] < 0) continue;
+            for (int dx = -1; dx <= 1; ++dx) {
+                if ((dx < 0 && x == 0) || (dx > 0 && x + 1 == width) || (dy == 1 && dx == 0)) continue;
+                const float *o = ref + 3 * ((size_t)r[dy] * width + (x + dx));
+                const uchar4 v = quantise(c3(o[0], o[1], o[2]));
+                refined = refined || abs((int)v.x - (int)q.x) > (int)t || abs((int)v.y - (int)q.y) > (int)t ||
+                          abs((int)v.z - (int)q.z) > (int)t;
+            }
+        }
+        if (!refined) edge_store<K>(out, edge_place<K>(k, x, width, req_rows), centre);
+        flag[p] = refined ? 1 : 0;
+    }
+    const int n_b = __syncthreads_count(refined);
+    if (threadIdx.x == 0) block_count[blockIdx.x] = (uint32_t)n_b;
+}
+
+// Exclusive prefix sum of count[0, n) in place, count[n] = total: one 1024-thread block, as the grid builder's k_gb_scan
+// (which reports its total into the grid builder's counters, and whose SASS stays as it is).
+__global__ void __launch_bounds__(1024) k_edge_scan(uint32_t *count, uint32_t n) {
+    __shared__ uint32_t warp_sum[32];
+    __shared__ uint32_t carry;
+    const uint32_t t = threadIdx.x, lane = t & 31u, warp = t >> 5;
+    if (t == 0) carry = 0;
+    __syncthreads();
+    for (uint32_t base = 0; base < n; base += 1024u) {
+        const uint32_t i = base + t;
+        const uint32_t mine = i < n ? count[i] : 0u;
+        uint32_t incl = mine;
+#pragma unroll
+        for (int o = 1; o < 32; o <<= 1) {
+            const uint32_t up = __shfl_up_sync(0xffffffffu, incl, o);
+            if ((int)lane >= o) incl += up;
+        }
+        if (lane == 31u) warp_sum[warp] = incl;
+        __syncthreads();
+        if (warp == 0) {
+            uint32_t w = warp_sum[lane];
+#pragma unroll
+            for (int o = 1; o < 32; o <<= 1) {
+                const uint32_t up = __shfl_up_sync(0xffffffffu, w, o);
+                if ((int)lane >= o) w += up;
+            }
+            warp_sum[lane] = w;   // inclusive over warps
+        }
+        __syncthreads();
+        if (i < n) count[i] = carry + (warp ? warp_sum[warp - 1] : 0u) + (incl - mine);
+        __syncthreads();
+        if (t == 1023u) carry += warp_sum[31];
+        __syncthreads();
+    }
+    if (t == 0) count[n] = carry;
+}
+
+// The refined pixels as entries (k, x), in row-major order of the requested pixels: block b of k_edge_emit's grid
+// writes its pixels from offset[b] on, ranked by warp ballots.
+__global__ void __launch_bounds__(256) k_edge_compact(const uint8_t *__restrict__ flag, const uint32_t *__restrict__ offset,
+                                                      uint32_t width, uint32_t npix, uint2 *list) {
+    __shared__ uint32_t warp_base[8];
+    const uint32_t p = blockIdx.x * blockDim.x + threadIdx.x, lane = threadIdx.x & 31u, warp = threadIdx.x >> 5;
+    const bool refined = p < npix && flag[p] != 0;
+    const uint32_t m = __ballot_sync(0xffffffffu, refined);
+    if (lane == 0) warp_base[warp] = (uint32_t)__popc(m);
+    __syncthreads();
+    if (threadIdx.x == 0) {
+        uint32_t s = offset[blockIdx.x];
+        for (int w = 0; w < 8; ++w) { const uint32_t c = warp_base[w]; warp_base[w] = s; s += c; }
+    }
+    __syncthreads();
+    if (refined) {
+        const uint32_t k = p / width;
+        list[warp_base[warp] + (uint32_t)__popc(m & ((1u << lane) - 1u))] = make_uint2(k, p - k * width);
+    }
+}
+
+int launch_edge_mask(OutKind kind, const float *ref, const int32_t *nb, uint32_t width, uint32_t npix, uint32_t t,
+                     const uint32_t *req_rows, void *out, uint8_t *flag, uint32_t *block_count, uint2 *list, cudaStream_t stream) {
+    const unsigned blocks = (npix + 255) / 256;
+    switch (kind) {
+        case OutKind::Rgba8: k_edge_emit<OutKind::Rgba8><<<blocks, 256, 0, stream>>>(ref, nb, width, npix, t, req_rows, out, flag, block_count); break;
+        case OutKind::Rgba8Scatter: k_edge_emit<OutKind::Rgba8Scatter><<<blocks, 256, 0, stream>>>(ref, nb, width, npix, t, req_rows, out, flag, block_count); break;
+        case OutKind::F32: k_edge_emit<OutKind::F32><<<blocks, 256, 0, stream>>>(ref, nb, width, npix, t, req_rows, out, flag, block_count); break;
+        case OutKind::F32Scatter: k_edge_emit<OutKind::F32Scatter><<<blocks, 256, 0, stream>>>(ref, nb, width, npix, t, req_rows, out, flag, block_count); break;
+    }
+    RG_CUDA(cudaGetLastError());
+    k_edge_scan<<<1, 1024, 0, stream>>>(block_count, blocks);
+    RG_CUDA(cudaGetLastError());
+    k_edge_compact<<<blocks, 256, 0, stream>>>(flag, block_count, width, npix, list);
+    RG_CUDA(cudaGetLastError());
+    return RG_OK;
+}
+
 // RG_OPT_VERIFY_CULL >= 2: re-trace every ray of a queue with the verbatim reference scan and
 // count results that differ from what the production trace kernel wrote (must be 0).
 template <bool ANY>
@@ -756,10 +934,12 @@ static DScene chunk_scene(const rg_scene *sc, uint32_t c) {
 
 // Enqueues one batch.  No allocation, no synchronisation, no host read: legal inside a stream capture.
 // `timed` = record CUDA events around the trace launches (not possible while capturing).
+// `n` is the batch's sample factor (width, height, y0 and npix are in sample space).  `list` (RG_OPT_SUPERSAMPLE_EDGES):
+// the batch is list->count refined pixels of a (width / n x height / n) image, n x n rays each; y0 and d_rows are unused.
 static int enqueue_batch_dev(rg_scene *sc, const DevPlan &plan, uint32_t width, uint32_t height, uint32_t y0, uint32_t npix,
                              const uint32_t *d_rows, OutKind kind, uchar4 *d_out, cudaStream_t stream, rg_stats *st, bool use_grid,
                              EventPool *events, EventPool &sync_events,
-                             std::vector<std::pair<cudaEvent_t, cudaEvent_t>> *trace_spans) {
+                             std::vector<std::pair<cudaEvent_t, cudaEvent_t>> *trace_spans, uint32_t n, const EdgeList *list) {
     const DScene &ds = sc->ds;
     const uint32_t L = ds.n_lights;
     WavefrontScratch &wf = sc->wf;
@@ -793,7 +973,11 @@ static int enqueue_batch_dev(rg_scene *sc, const DevPlan &plan, uint32_t width, 
     RG_CUDA(cudaMemsetAsync(dc->lvl, 0, sizeof(dc->lvl), stream));
     RayQueue cur = make_queue(wf.ray[0], plan.cap[0]);
     const PixelOrder po = pixel_order(width, npix / width);
-    k_generate<<<(npix + 255) / 256, 256, 0, stream>>>(ds, cur, width, height, y0, npix, d_rows, &dc->lvl[0].n, po);
+    if (list)
+        k_generate_list<<<(npix + 255) / 256, 256, 0, stream>>>(ds, cur, width / n, height / n, n, list->entries, npix, list->req_rows,
+                                                                &dc->lvl[0].n);
+    else
+        k_generate<<<(npix + 255) / 256, 256, 0, stream>>>(ds, cur, width, height, y0, npix, d_rows, &dc->lvl[0].n, po);
     RG_CUDA(cudaGetLastError());
     st->gpu_launches++;
     st->rays_primary += npix;
@@ -910,8 +1094,11 @@ static int enqueue_batch_dev(rg_scene *sc, const DevPlan &plan, uint32_t width, 
         RG_CUDA(cudaGetLastError());
         st->gpu_launches++;
     }
-    if (sc->supersample > 1) {   // width, height, y0 and npix are in sample space: npix / (n n) output pixels
-        const uint32_t n = sc->supersample;
+    if (list) {
+        if ((rc = launch_resolve_list(kind, reinterpret_cast<const float *>(wf.nodes[0].as<float4>()), 4, n, width / n, list->entries,
+                                      list->count, list->req_rows, d_out, stream)))
+            return rc;
+    } else if (n > 1) {   // width, height, y0 and npix are in sample space: npix / (n n) output pixels
         if ((rc = launch_resolve(kind, reinterpret_cast<const float *>(wf.nodes[0].as<float4>()), 4, po.strip, n, width / n,
                                  po.rows / n, d_rows, y0, d_out, stream)))
             return rc;
@@ -935,13 +1122,14 @@ static int enqueue_batch_dev(rg_scene *sc, const DevPlan &plan, uint32_t width, 
 
 // ---- one CUDA graph per batch shape --------------------------------------------------------------
 static std::vector<uint64_t> graph_key(const rg_scene *sc, const DevPlan &plan, uint32_t width, uint32_t height, uint32_t y0,
-                                       uint32_t npix, const uint32_t *d_rows, OutKind kind, const uchar4 *d_out, bool use_grid) {
+                                       uint32_t npix, const uint32_t *d_rows, OutKind kind, const uchar4 *d_out, bool use_grid,
+                                       uint32_t n, const EdgeList *list) {
     const WavefrontScratch &wf = sc->wf;
     std::vector<uint64_t> k = {width, height, y0, npix, (uint64_t)(uintptr_t)d_rows, (uint64_t)(uintptr_t)d_out,
                                (uint64_t)use_grid, (uint64_t)kind, (uint64_t)sc->ds.max_depth, (uint64_t)sc->overlap,
                                (uint64_t)sc->verify_cull, (uint64_t)sc->trace_stats | ((uint64_t)sc->origin_hints << 2) | ((uint64_t)sc->light_grids << 3), (uint64_t)plan.levels,
                                (uint64_t)sc->level_growth,    // the capacities are baked into the captured launches
-                               (uint64_t)sc->supersample};    // the last launch: (n, w, h) and (1, n w, n h) share a sample space
+                               (uint64_t)n};                  // the last launch: (n, w, h) and (1, n w, n h) share a sample space
     auto add = [&](const DeviceBuffer &b) { k.push_back((uint64_t)(uintptr_t)b.ptr); };
     add(wf.ray[0]); add(wf.ray[1]); add(wf.hit_t); add(wf.hit_body);
     for (int p = 0; p < 2; ++p) { add(wf.sray[p]); add(wf.s_tmax[p]); add(wf.s_ab[p]); add(wf.s_lit[p]); add(wf.lit_bc[p]); add(wf.lit_node[p]); }
@@ -949,6 +1137,11 @@ static std::vector<uint64_t> graph_key(const rg_scene *sc, const DevPlan &plan, 
     // The light-chunk count needs no entry: it is fixed by the handle's scene, and a graph dies with its scene.
     if (sc->ds.n_lights > kLightChunk)
         for (int p = 0; p < 2; ++p) { add(wf.lit_geo[p]); add(wf.lit_acc[p]); }
+    if (list) {   // a batch of refined pixels (its pixel count is npix / (n n)); row batches have no such entries
+        k.push_back((uint64_t)(uintptr_t)list->entries);
+        k.push_back((uint64_t)(uintptr_t)list->req_rows);
+        k.push_back((uint64_t)list->count);
+    }
     return k;
 }
 
@@ -956,10 +1149,10 @@ static std::vector<uint64_t> graph_key(const rg_scene *sc, const DevPlan &plan, 
 // Returns RG_OK with *done = false when the batch should be enqueued the ordinary way.
 static int graph_batch(rg_scene *sc, const DevPlan &plan, uint32_t width, uint32_t height, uint32_t y0, uint32_t npix,
                        const uint32_t *d_rows, OutKind kind, uchar4 *d_out, cudaStream_t stream, rg_stats *st, bool use_grid,
-                       EventPool &sync_events, bool *done) {
+                       EventPool &sync_events, bool *done, uint32_t n, const EdgeList *list) {
     *done = false;
     GraphCache &gc = sc->graphs;
-    const std::vector<uint64_t> key = graph_key(sc, plan, width, height, y0, npix, d_rows, kind, d_out, use_grid);
+    const std::vector<uint64_t> key = graph_key(sc, plan, width, height, y0, npix, d_rows, kind, d_out, use_grid, n, list);
     GraphEntry *hit = nullptr;
     for (auto &e : gc.entries)
         if (e.key == key) { hit = &e; break; }
@@ -977,7 +1170,8 @@ static int graph_batch(rg_scene *sc, const DevPlan &plan, uint32_t width, uint32
         rg_stats tmp{};
         const size_t sync_used = sync_events.used;
         RG_CUDA(cudaStreamBeginCapture(cs, cudaStreamCaptureModeThreadLocal));
-        const int rc = enqueue_batch_dev(sc, plan, width, height, y0, npix, d_rows, kind, d_out, cs, &tmp, use_grid, nullptr, sync_events, nullptr);
+        const int rc = enqueue_batch_dev(sc, plan, width, height, y0, npix, d_rows, kind, d_out, cs, &tmp, use_grid, nullptr, sync_events, nullptr,
+                                     n, list);
         cudaGraph_t graph = nullptr;
         const cudaError_t ce = cudaStreamEndCapture(cs, &graph);
         sync_events.used = sync_used;
@@ -1017,7 +1211,8 @@ static int graph_batch(rg_scene *sc, const DevPlan &plan, uint32_t width, uint32
 }
 
 int wavefront_render(rg_scene *sc, uint32_t width, uint32_t height, uint32_t y0, uint32_t y1,
-                     const uint32_t *d_rows, OutKind kind, uchar4 *d_out, cudaStream_t stream, rg_stats *st) {
+                     const uint32_t *d_rows, OutKind kind, uchar4 *d_out, cudaStream_t stream, rg_stats *st, uint32_t n,
+                     const EdgeList *list) {
     const DScene &ds = sc->ds;
     bool use_grid = false;
     if (sc->accel == RG_ACCEL_GRID) use_grid = ds.grid.enabled != 0;
@@ -1029,10 +1224,13 @@ int wavefront_render(rg_scene *sc, uint32_t width, uint32_t height, uint32_t y0,
     std::vector<std::pair<cudaEvent_t, cudaEvent_t>> trace_spans;
     // RG_OPT_SUPERSAMPLE: the batches trace the (n width x n height) sample image, output row y being sample rows
     // [n y, n y + n) (or, with a row list, entries [n k, n k + n) of the expanded list); batches are cut in whole output rows.
-    const uint32_t n = sc->supersample, sw = n * width, sh = n * height;
-    const uint32_t rows = y1 - y0;
+    // A list of refined pixels (RG_OPT_SUPERSAMPLE_EDGES) is cut in whole pixels instead: its "rows" are list entries.
+    const uint32_t sw = n * width, sh = n * height;
+    const uint32_t rows = list ? list->count : y1 - y0;
+    const uint64_t unit = list ? (uint64_t)n * n : (uint64_t)n * sw;   // samples per row (per listed pixel)
+    if (list) y0 = 0;
     const uint64_t batch_pixels = sc->batch_pixels ? sc->batch_pixels : (16ull << 20);
-    uint32_t batch_rows = (uint32_t)std::max<uint64_t>(1, std::min<uint64_t>(rows ? rows : 1, batch_pixels / ((uint64_t)n * sw)));
+    uint32_t batch_rows = (uint32_t)std::max<uint64_t>(1, std::min<uint64_t>(rows ? rows : 1, batch_pixels / unit));
     const rg_stats st0 = *st;
     for (;;) {   // a ray tree larger than device memory restarts the render with half the rows per batch
         *st = st0;
@@ -1045,20 +1243,25 @@ int wavefront_render(rg_scene *sc, uint32_t width, uint32_t height, uint32_t y0,
         if (sc->ds.n_lights > 0 && (sc->overlap == 2 || (sc->overlap == 0 && use_grid))) {
             if (!sc->wf.aux) RG_CUDA(cudaStreamCreateWithFlags(&sc->wf.aux, cudaStreamNonBlocking));
         }
-        for (uint32_t y = y0; y < y1 && rc == RG_OK;) {
-            const uint32_t ye = (uint32_t)std::min<uint64_t>((uint64_t)y + batch_rows, y1);
-            uchar4 *out = is_scatter(kind) ? d_out
+        const uint32_t y1_ = y0 + rows;
+        for (uint32_t y = y0; y < y1_ && rc == RG_OK;) {
+            const uint32_t ye = (uint32_t)std::min<uint64_t>((uint64_t)y + batch_rows, y1_);
+            uchar4 *out = is_scatter(kind) || list ? d_out
                         : reinterpret_cast<uchar4 *>(reinterpret_cast<unsigned char *>(d_out) + (size_t)(y - y0) * width * bytes_per_pixel(kind));
+            EdgeList part;
+            if (list) part = EdgeList{list->entries + y, ye - y, list->req_rows};
             DevPlan plan;
-            const uint64_t npix64 = (uint64_t)(ye - y) * n * sw;
+            const uint64_t npix64 = (uint64_t)(ye - y) * unit;
             if (npix64 > 0x7FFFFFFFull) { set_error("batch of %llu pixels is too large", (unsigned long long)npix64); rc = RG_E_NOMEM; }
             else if (npix64 && (rc = plan_batch_dev(sc, (uint32_t)npix64, plan, use_grid)) == RG_OK) {
                 bool done = false;
+                const uint32_t ys = list ? 0u : n * y;
                 if (sc->graph != 1 && sc->verify_cull == 0)
-                    rc = graph_batch(sc, plan, sw, sh, n * y, (uint32_t)npix64, d_rows, kind, out, stream, st, use_grid, sync_events, &done);
+                    rc = graph_batch(sc, plan, sw, sh, ys, (uint32_t)npix64, d_rows, kind, out, stream, st, use_grid, sync_events, &done,
+                                     n, list ? &part : nullptr);
                 if (rc == RG_OK && !done)
-                    rc = enqueue_batch_dev(sc, plan, sw, sh, n * y, (uint32_t)npix64, d_rows, kind, out, stream, st, use_grid, &events,
-                                           sync_events, &trace_spans);
+                    rc = enqueue_batch_dev(sc, plan, sw, sh, ys, (uint32_t)npix64, d_rows, kind, out, stream, st, use_grid, &events,
+                                           sync_events, &trace_spans, n, list ? &part : nullptr);
             }
             y = ye;
         }
